@@ -2,6 +2,7 @@
 """bench.py -- samples/sec of the GAT simulation hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config ns|c2|c3|c4|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -45,6 +46,7 @@ import numpy as np  # noqa: E402
 
 UNIT = "samples/s"
 SEED = 20260101
+DUMP_BYTES = 32 << 20          # --dump-outputs: rows of the count matrix kept
 
 # BASELINE.json configs: (segments, annotation tracks, isochores, counter, metric label)
 CONFIGS = {
@@ -85,7 +87,12 @@ def parse_args():
                     help="N > 1: how the per-step count slabs reach every rank -- peer: output routes into every rank's "
                          "matrix over NVLink, served by copy engines behind the next batch; peer-kernel: the same routes "
                          "served by the counting kernel's own stores; nccl: all_gather_into_tensor")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed, seeded sample of rows of the last timed step's count "
+                         "matrix (DIR/counts.npy, float64) and their global sample indices (DIR/sample_index.npy)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     cfg = CONFIGS[args.config]
     for k in ("segments", "annotations", "counter", "isochores"):
         if getattr(args, k) is None:
@@ -133,6 +140,24 @@ def config_of(args, wl, world):
                   "sample indices advance every step"
                   % (wl["n_a_total"] * 2.33 * 8 / 1e6 + 12, args.batch * wl["n_segments"] * 8 / 1e6),
             "data_seed": SEED}
+
+
+def dump_outputs(directory, matrix, sample_index):
+    """the count matrix of a step as a caller of the path receives it ([samples][annotation tracks] on the device),
+    reduced to whole rows picked by a generator with a fixed seed, so that two builds run with the same arguments
+    can be compared output for output; at most DUMP_BYTES of float64 (exact for uint32 counts)"""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    rows, cols = matrix.shape
+    n = min(rows, max(1, DUMP_BYTES // (8 * cols)))
+    pick = np.sort(np.random.default_rng(SEED).choice(rows, n, replace=False))
+    if matrix.dtype == torch.uint32:
+        matrix = matrix.view(torch.int32)
+    sample = matrix.index_select(0, torch.from_numpy(pick).to(matrix.device)).cpu().numpy()
+    if sample.dtype == np.int32:
+        sample = sample.view(np.uint32)
+    np.save(os.path.join(directory, "counts.npy"), sample.astype(np.float64))
+    np.save(os.path.join(directory, "sample_index.npy"), np.asarray(sample_index)[pick].astype(np.float64))
 
 
 # --------------------------------------------------------------------------------------------- clocks
@@ -510,6 +535,12 @@ def run_ours(args):
     clock_info = clocks.stop(t_begin, t_end) if rank == 0 else None
     value = world * S * args.steps / (ms / 1000.0)
     last = args.warmup + args.steps - 1
+    if args.dump_outputs:                          # (before the checks and profiled steps below reuse the slabs)
+        if rank == 0:
+            matrix = gathers[last % nbuf] if world > 1 else outs[last % nbuf]
+            index = np.concatenate([step_begin(last, r) + np.arange(S) for r in range(world)])
+            dump_outputs(args.dump_outputs, matrix, index)
+        barrier()
 
     # ---- checks, outside the timed region: the slab of the last timed step against the CPU oracle, and (N > 1)
     # the gathered matrix of that step against a single-rank recomputation of every rank's global indices

@@ -2,8 +2,8 @@
 UNMODIFIED reference through libgat_b200.so (INTEGRATION.md section 2).
 
 It uses nothing but ctypes, numpy and the reference's own containers -- no import of the gat_b200 package -- and is
-exercised by tests/test_gpu_dropin.py, which installs it into the reference as compiled under oracle/_ref and runs
-the reference's own gat.run() on top of it.
+exercised by tests/test_gpu_dropin.py, which installs it, hands it containers shaped like the reference's and calls
+it the way the reference's gat.run() does.
 
     import gat, _b200
     _b200.install(gat)            # UnconditionalSampler.sample and Engine.computeCounts now call the library

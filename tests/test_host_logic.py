@@ -230,19 +230,30 @@ def test_bed_reader_tracks(tmp_path):
     assert list(r.keys()) == ["merged"] and r["merged"]["chr1"].counts() == 4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/test/data"), reason="reference data only in the build container")
-def test_input_preparation_matches_reference_io():
+def test_input_preparation_matches_reference_io(tmp_path, monkeypatch):
     """our buildSegments + applyIsochores on the reference's test data == the arrays the reference's own
-    IO produced (stored in tests/golden/observed_testdata.npz)"""
+    IO produced (stored in tests/golden/observed_testdata.npz).  The BED files are written from those arrays
+    (segment and annotation tracks in the name column, gzip-compressed like the reference's test/data): reading
+    and preparing what the reference prepared must give it back unchanged.  Host preparation (GATB_HOST_PREP=1)."""
+    import gzip
     import gat_b200
     from gat_b200 import io as IO
-    d = "/root/reference/test/data"
+    monkeypatch.setenv("GATB_HOST_PREP", "1")
+    z, meta = G.load_npz("observed_testdata")
+    d = str(tmp_path)
+    for fn, name, keys in (("segments_single.bed.gz", "segments", meta["segments"]),
+                           ("annotations.bed.gz", "annotations", meta["annotations"]),
+                           ("workspace.bed.gz", "workspace", [(None, k) for k in meta["workspace"]])):
+        with gzip.open(os.path.join(d, fn), "wt") as f:
+            for track, key in keys:
+                arr = z["%s/%s" % (name, key)] if track is None else z["%s/%s/%s" % (name, track, key)]
+                for start, end in G.undelta(arr):
+                    f.write("%s\t%i\t%i%s\n" % (key, start, end, "" if track is None else "\t" + track))
     options, _ = gat_b200.buildParser().parse_args([
         "--segments=%s/segments_single.bed.gz" % d, "--annotations=%s/annotations.bed.gz" % d,
         "--workspace=%s/workspace.bed.gz" % d, "--with-segment-tracks"])
     segments, annotations, workspaces, isochores = IO.buildSegments(options)
     workspace = IO.applyIsochores(segments, annotations, workspaces, options, isochores)
-    z, meta = G.load_npz("observed_testdata")
     assert sorted(workspace.keys()) == sorted(meta["workspace"])
     for key in meta["workspace"]:
         assert np.array_equal(workspace[key].asarray(), G.undelta(z["workspace/%s" % key]))
