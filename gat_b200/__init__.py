@@ -14,6 +14,7 @@ import numpy as np
 
 from . import device
 from . import engine as Engine
+from . import matrixfree
 from . import stats as Stats
 from .engine import (IntervalCollection, IntervalDictionary, SamplerAnnotator, SamplerSegments, SamplerShift, UnconditionalWorkspace,
                      AnnotatorResult, AnnotatorResultExtended, getContext, seed)
@@ -60,19 +61,13 @@ def buildContigAnnotations(annotations, workspace, contigs):
     return atracks, lists, nseg
 
 
-def sampleTrack(track_index, segs, annotations, workspace, sampler, counters, num_samples,
-                sample_range=None, annos_cache=None, return_device=False, routes=None):
-    """all samples of one track: counts[counter_id] = ndarray [num_samples][n_annot]
-    (replaces UnconditionalSampler.sample, gat/__init__.py:704-778).
-    routes: output routes (device.Context.set_output_routes) -- the counting kernels deliver the rows straight to
-    their consumers (other ranks' matrices included) instead of a local slab."""
-    import torch
+def trackSampler(segs, annotations, workspace, sampler, annos_cache=None):
+    """the GPU objects that sample one track: -> (smp, annos), device.Sampler and device.Annotations, or
+    (None, None) for a track without any unit (every sample counts zero)"""
     ctx = getContext()
     problem = TrackProblem(segs, workspace)
-    counter_names = [c.name for c in counters]
-    atracks = list(annotations.tracks)
     if not problem.unit_keys:
-        return atracks, [np.zeros((num_samples, len(atracks))) for _ in counters], np.zeros(3, dtype=np.uint64)
+        return None, None
     try:
         smp = device.Sampler(ctx, problem.unit_contig, len(problem.contigs), problem.has_isochores,
                              problem.unit_segments, problem.unit_workspace,
@@ -111,6 +106,22 @@ def sampleTrack(track_index, segs, annotations, workspace, sampler, counters, nu
         annos = device.Annotations(ctx, lists, key_ws_nseg=nseg, lazy=True)
         if annos_cache is not None:
             annos_cache[key] = annos
+    return smp, annos
+
+
+def sampleTrack(track_index, segs, annotations, workspace, sampler, counters, num_samples,
+                sample_range=None, annos_cache=None, return_device=False, routes=None):
+    """all samples of one track: counts[counter_id] = ndarray [num_samples][n_annot]
+    (replaces UnconditionalSampler.sample, gat/__init__.py:704-778).
+    routes: output routes (device.Context.set_output_routes) -- the counting kernels deliver the rows straight to
+    their consumers (other ranks' matrices included) instead of a local slab."""
+    import torch
+    ctx = getContext()
+    counter_names = [c.name for c in counters]
+    atracks = list(annotations.tracks)
+    smp, annos = trackSampler(segs, annotations, workspace, sampler, annos_cache)
+    if smp is None:
+        return atracks, [np.zeros((num_samples, len(atracks))) for _ in counters], np.zeros(3, dtype=np.uint64)
     begin, end = sample_range if sample_range is not None else (0, num_samples)
     n_local = end - begin
     dev = torch.device("cuda", ctx.device)
@@ -146,7 +157,11 @@ def run(segments, annotations, workspace, sampler, counters, workspace_generator
     kwargs: num_samples (10000), pseudo_count (1.0), reference, output_counts_pattern,
     output_samples_pattern, outfiles, cache / sample_files / num_threads (accepted, unused: the
     reference's sample cache is dead code and its multiprocessing is replaced by the GPU);
-    exchange ("auto" | "allgather" | "columns": how a multi-GPU run combines its slabs, see below).
+    exchange ("auto" | "allgather" | "columns": how a multi-GPU run combines its slabs, see below);
+    keep_samples (None | True | False): False computes the statistics without the sample matrix
+    (gat_b200/matrixfree.py), so that the number of samples is not bounded by GPU memory -- the results are the
+    same, but their samples cannot be asked for; None (default) does so only when the matrices would not fit in
+    the free GPU memory and no counts table is written.
     """
     import torch
     # ONE CUDA stream for the whole run: the library's kernels, torch's tensor operations and the NCCL
@@ -223,6 +238,16 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
         raise ValueError("output_counts_pattern needs every column on rank 0: use exchange='allgather'")
     col_begin, col_end = parallel.column_range(n_atracks, rank, world) if exchange == "columns" else (0, n_atracks)
 
+    # keep the S x A matrices, or stream the samples through column accumulators (the exchange and the transport
+    # below do not apply then: every rank counts its own samples of all columns, the integers are summed)
+    density = any(c.name == "nucleotide-density" for c in counters)
+    keep_samples = kwargs.get("keep_samples", None)
+    matrix_bytes = 4 * len(counters) * num_samples * (col_end - col_begin) * len(segments.tracks)
+    free_bytes = torch.cuda.mem_get_info(ctx.device)[0] if keep_samples is None else 0
+    matrix_free = matrixfree.use_matrix_free(keep_samples, bool(output_counts_pattern), density, matrix_bytes, free_bytes)
+    if keep_samples is None and world > 1:          # (the free memory differs between GPUs: every rank takes one mode)
+        matrix_free = any(matrixfree.allgather(matrix_free, world))
+
     # Transport of a multi-GPU exchange:
     #   "peer"  the counting kernels store every finished row straight into the destination ranks' matrices (CUDA IPC
     #           memory over NVLink, output routes of the C ABI): the exchange happens inside the kernels' epilogue,
@@ -236,7 +261,16 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
 
     sampled = {}
     begin, end = parallel.shard_range(num_samples, rank, world)
-    for ntrack, track in enumerate(segments.tracks):
+    streamed = None
+    if matrix_free:
+        streamed = _sampleStreamed(segments, annotations, workspace, sampler, counters, observed_counts, reference,
+                                   num_samples, pseudo_count, annos_cache, rank, world)
+        sampled = dict((track, (list(annotations.tracks), None, None, None)) for track in streamed)
+        if output_samples_pattern and rank == 0:
+            for ntrack, track in enumerate(segments.tracks):
+                if track in streamed:
+                    _dumpSamples(track, ntrack, segments[track], workspace, sampler, num_samples, output_samples_pattern)
+    for ntrack, track in enumerate(segments.tracks if streamed is None else ()):
         segs = segments[track]
         if workspace.sum() == 0:
             continue
@@ -322,7 +356,10 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
             matrix = None
             lo, hi = col_begin, col_end
             ref_l = None if ref is None else ref[lo:hi]
-            if out_u is None:
+            if streamed is not None:
+                st = streamed[track][counter_id]
+                matrix = Engine.SamplesNotKept(num_samples, len(atracks))
+            elif out_u is None:
                 host = np.zeros((num_samples, len(atracks)))
                 st = ctx.column_stats(host.astype(np.uint32), obs, pseudo_count=pseudo_count, ref_fold=ref)
             elif hi == lo:              # more ranks than columns: nothing to do here
@@ -390,6 +427,51 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
         sys.stderr.write("# gat_b200.run phases: " + ", ".join(
             "%s %.3fs" % (timing[i][0], timing[i][1] - timing[i - 1][1]) for i in range(1, len(timing))) + "\n")
     return annotator_results
+
+
+def _sampleStreamed(segments, annotations, workspace, sampler, counters, observed_counts, reference, num_samples,
+                    pseudo_count, annos_cache, rank, world):
+    """the matrix-free mode of run(): per track, this rank's samples in slabs of one reused device buffer, counted
+    into column accumulators and overwritten; the statistics of the track are complete (summed over the ranks)
+    before the next track starts.  -> {track: [statistics dict per counter]}"""
+    import torch
+    from . import parallel
+    ctx = getContext()
+    dev = torch.device("cuda", ctx.device)
+    names = [c.name for c in counters]
+    atracks = list(annotations.tracks)
+    A = len(atracks)
+    begin, end = parallel.shard_range(num_samples, rank, world)
+    n_local = end - begin
+    matrixfree.info.update(reruns=0, arena_bytes=0, chunk_rows=0)
+    chunk = max(1, min(max(n_local, 1), matrixfree.SLAB_BYTES // (4 * len(names) * max(A, 1))))
+    slab = torch.zeros(len(names) * chunk * max(A, 1), dtype=torch.int32, device=dev)
+    ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or 1)
+    out = {}
+    for ntrack, track in enumerate(segments.tracks):
+        if workspace.sum() == 0:
+            continue
+        smp, annos = trackSampler(segments[track], annotations, workspace, sampler, annos_cache)
+
+        def produce(r0, n):
+            if smp is None:                     # a track without any unit: every sample counts zero
+                slab[:len(names) * n * A].zero_()
+            else:
+                smp.run(annos, names, Engine.getSeed(), ntrack, begin + r0, n, out_counts_ptr=slab.data_ptr())
+            return slab.data_ptr()
+
+        planes = []
+        for counter_id in range(len(counters)):
+            r = observed_counts[counter_id][track]
+            planes.append((np.array([r[a] for a in atracks], dtype=np.float64),
+                           np.array([reference[track][a].fold for a in atracks], dtype=np.float64) if reference else None))
+        try:
+            out[track] = matrixfree.stream_statistics(ctx, produce, planes, num_samples, n_local, A, chunk,
+                                                      pseudo_count=pseudo_count, rank=rank, world=world)
+        finally:
+            if smp is not None:
+                smp.close()
+    return out
 
 
 def _open(filename, mode):

@@ -28,7 +28,11 @@ SYMBOLS = [
     "gatb_lists_info", "gatb_lists_sizes", "gatb_lists_download", "gatb_lists_destroy",
     "gatb_annotations_create_from_lists",
     "gatb_set_output_routes", "gatb_set_route_mode", "gatb_peer_alloc", "gatb_peer_free", "gatb_peer_open", "gatb_peer_close",
+    "gatb_colacc_create", "gatb_colacc_set_windows", "gatb_colacc_add", "gatb_colacc_state", "gatb_colacc_merge",
+    "gatb_colacc_finish", "gatb_colacc_destroy",
 ]
+
+COLACC_SUMS, COLACC_HIST = 1, 2
 
 
 class Route(ctypes.Structure):
@@ -161,4 +165,18 @@ def bind(L):
     L.gatb_peer_open.argtypes = [vp, vp, ctypes.POINTER(vp)]
     L.gatb_peer_close.restype = i32
     L.gatb_peer_close.argtypes = [vp, vp]
+    L.gatb_colacc_create.restype = i32
+    L.gatb_colacc_create.argtypes = [vp, i32, u64, vp, vp, ctypes.POINTER(vp)]
+    L.gatb_colacc_set_windows.restype = i32
+    L.gatb_colacc_set_windows.argtypes = [vp, vp, vp]
+    L.gatb_colacc_add.restype = i32
+    L.gatb_colacc_add.argtypes = [vp, vp, u64, u64, i32]
+    L.gatb_colacc_state.restype = i32
+    L.gatb_colacc_state.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.gatb_colacc_merge.restype = i32
+    L.gatb_colacc_merge.argtypes = [vp, u64, vp, vp, vp, vp]
+    L.gatb_colacc_finish.restype = i32
+    L.gatb_colacc_finish.argtypes = [vp, dbl, vp, vp, vp, vp, vp, vp, vp]
+    L.gatb_colacc_destroy.restype = None
+    L.gatb_colacc_destroy.argtypes = [vp]
     return L

@@ -1530,6 +1530,62 @@ static double exact_sumsq_dev(uint64_t n, unsigned long long sum, unsigned long 
     return (double)num / (double)n;
 }
 
+// The per-column doubles of makeEnrichmentStatistics (gat/Engine.pyx:1635-1718) from a column's reduced integers /
+// order statistics: ONE function for the matrix (gatb_column_stats) and the matrix-free path (gatb_colacc_finish),
+// so that both produce their doubles from the same numbers by the same operations.  mean = sum / l, sumsq = sum
+// (x - mean)^2, qlo / qhi the order statistics at the CI ranks, n_lt / n_eq the counts of pass 1 against obs_eff
+// (= observed / ref_fold).  Any output may be NULL.
+static void finish_columns(uint64_t l, uint32_t A, const double *observed, const double *obs_eff, const double *ref_fold,
+                           double pseudo_count, const double *mean, const double *sumsq, const double *qlo,
+                           const double *qhi, const unsigned long long *n_lt, const unsigned long long *n_eq,
+                           double *expected, double *stddev, double *lower95, double *upper95, double *fold, double *pvalue)
+{
+    for (uint32_t a = 0; a < A; a++) {
+        double exp_ = mean[a];
+        if (ref_fold) exp_ *= ref_fold[a];                                    // :1673-1676
+        const double fo = (exp_ != 0) ? (observed[a] + pseudo_count) / (exp_ + pseudo_count) : 1.0;   // :1679-1682
+        double lo = qlo[a], hi = qhi[a];
+        if (ref_fold) { lo *= ref_fold[a]; hi *= ref_fold[a]; }              // :1713-1714
+        // getTwoSidedPValue (:1543-1576) from counts instead of a sorted copy
+        const uint64_t idx0 = n_lt[a];                                        // lower_bound of val in the sorted samples
+        const bool first_is_eq = n_eq[a] > 0;                                 // sorted[idx0] == val
+        uint64_t idx = idx0;
+        if (idx0 == l) idx = 1;
+        else if (obs_eff[a] > exp_) {
+            if (first_is_eq && idx0 > 0) idx = idx0 - 1;
+            idx = l - (idx + 1);
+        } else {
+            if (first_is_eq) idx = idx0 + n_eq[a];
+        }
+        const double pv = std::max(1.0 / (double)l, (double)idx / (double)l);
+        if (expected) expected[a] = exp_;
+        if (stddev) stddev[a] = std::sqrt(sumsq[a] / (double)l);             // numpy.std ddof 0 (:1684)
+        if (lower95) lower95[a] = lo;
+        if (upper95) upper95[a] = hi;
+        if (fold) fold[a] = fo;
+        if (pvalue) pvalue[a] = pv;
+    }
+}
+
+// observed / ref_fold (the value the samples are compared with) and the CI ranks (gat/Engine.pyx:1689-1696)
+static int effective_observed(gatb_ctx *ctx, uint32_t A, const double *observed, const double *ref_fold, std::vector<double> &obs_eff)
+{
+    obs_eff.resize(A);
+    for (uint32_t a = 0; a < A; a++) {
+        if (ref_fold) {
+            if (!(ref_fold[a] > 0)) return fail(ctx, GATB_ERR_INVALID, "0 fold change not applicable");
+            obs_eff[a] = observed[a] / ref_fold[a];
+        } else obs_eff[a] = observed[a];
+    }
+    return GATB_OK;
+}
+static void ci_ranks(uint64_t l, uint64_t &rank_lo, uint64_t &rank_hi)
+{
+    const uint64_t off = (uint64_t)(0.05 * (double)l);
+    if (off > 0) { rank_lo = std::min<uint64_t>(off, l - 1); rank_hi = (l > off) ? l - off : 0; }
+    else { rank_lo = 0; rank_hi = l - 1; }
+}
+
 struct StreamStatsOut {
     std::vector<double> sum, sumsq, qlo, qhi;       // sumsq = sum (x - mean)^2
     std::vector<unsigned long long> n_lt, n_eq;
@@ -1620,18 +1676,10 @@ extern "C" int gatb_column_stats(gatb_ctx *ctx, const void *counts, int is_float
         CU(ctx, d_counts.upload((const uint8_t *)counts, l * A * esz, st));
         dc = d_counts.p;
     }
-    std::vector<double> obs_eff(A);
-    for (uint32_t a = 0; a < A; a++) {
-        if (ref_fold) {
-            if (!(ref_fold[a] > 0)) return fail(ctx, GATB_ERR_INVALID, "0 fold change not applicable");
-            obs_eff[a] = observed[a] / ref_fold[a];
-        } else obs_eff[a] = observed[a];
-    }
-    // CI ranks (gat/Engine.pyx:1689-1696)
+    std::vector<double> obs_eff;
+    if (const int rc = effective_observed(ctx, A, observed, ref_fold, obs_eff)) return rc;
     uint64_t rank_lo, rank_hi;
-    const uint64_t off = (uint64_t)(0.05 * (double)l);
-    if (off > 0) { rank_lo = std::min<uint64_t>(off, l - 1); rank_hi = (l > off) ? l - off : 0; }
-    else { rank_lo = 0; rank_hi = l - 1; }
+    ci_ranks(l, rank_lo, rank_hi);
     std::vector<double> h_sum(A), h_sq(A), h_qlo(A), h_qhi(A), h_mean(A);
     std::vector<unsigned long long> h_cnt(2 * (size_t)A);
     if (!is_float && ctx->stats_stream && stats_stream_fits(dc, l, A, ctx->smem_optin)) {
@@ -1684,32 +1732,8 @@ extern "C" int gatb_column_stats(gatb_ctx *ctx, const void *counts, int is_float
             for (uint32_t a = 0; a < A; a++) h_sq[a] = exact_sumsq_dev(l, h_sqi[2 * (size_t)A + a], h_sqi[a], h_sqi[A + a]);
     }
 
-    for (uint32_t a = 0; a < A; a++) {
-        double exp_ = h_mean[a];
-        if (ref_fold) exp_ *= ref_fold[a];                                    // :1673-1676
-        const double fo = (exp_ != 0) ? (observed[a] + pseudo_count) / (exp_ + pseudo_count) : 1.0;   // :1679-1682
-        double lo = h_qlo[a], hi = h_qhi[a];
-        if (ref_fold) { lo *= ref_fold[a]; hi *= ref_fold[a]; }              // :1713-1714
-        // getTwoSidedPValue (:1543-1576) from counts instead of a sorted copy
-        const uint64_t n_lt = h_cnt[a], n_eq = h_cnt[A + a];
-        const uint64_t idx0 = n_lt;                                           // lower_bound of val in the sorted samples
-        const bool first_is_eq = n_eq > 0;                                    // sorted[idx0] == val
-        uint64_t idx = idx0;
-        if (idx0 == l) idx = 1;
-        else if (obs_eff[a] > exp_) {
-            if (first_is_eq && idx0 > 0) idx = idx0 - 1;
-            idx = l - (idx + 1);
-        } else {
-            if (first_is_eq) idx = idx0 + n_eq;
-        }
-        const double pv = std::max(1.0 / (double)l, (double)idx / (double)l);
-        if (expected) expected[a] = exp_;
-        if (stddev) stddev[a] = std::sqrt(h_sq[a] / (double)l);              // numpy.std ddof 0 (:1684)
-        if (lower95) lower95[a] = lo;
-        if (upper95) upper95[a] = hi;
-        if (fold) fold[a] = fo;
-        if (pvalue) pvalue[a] = pv;
-    }
+    finish_columns(l, A, observed, obs_eff.data(), ref_fold, pseudo_count, h_mean.data(), h_sq.data(), h_qlo.data(),
+                   h_qhi.data(), h_cnt.data(), h_cnt.data() + A, expected, stddev, lower95, upper95, fold, pvalue);
     return GATB_OK;
 }
 
@@ -1767,6 +1791,271 @@ extern "C" int gatb_column_pvalue(gatb_ctx *ctx, const void *counts, int is_floa
         pvalue[a] = std::max(1.0 / (double)l, (double)idx / (double)l);
     }
     return GATB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// column statistics without the sample matrix: an accumulator of one uint32 counter plane, fed slab by slab.
+// Pass 1 of the streamed statistics ADDS its exact integers (sum, 128-bit sum of squares, #{x < obs}, #{x == obs},
+// extremes) into the accumulator's own arrays, so any split of the rows into slabs gives the integers of one pass
+// over the whole matrix; the two order statistics come from per-column windows of unit-width bins (exact values,
+// so exact ranks).  gatb_colacc_finish turns the integers into doubles with the same finish_columns() as
+// gatb_column_stats: same integers, same doubles.
+struct gatb_colacc {
+    gatb_ctx *ctx = nullptr;
+    uint32_t A = 0;
+    uint64_t l = 0, rows = 0;                       // samples of the whole column / rows counted into the sums so far
+    uint64_t rank_lo = 0, rank_hi = 0;
+    std::vector<double> observed, ref, obs_eff;
+    std::vector<uint32_t> lo, width;
+    uint64_t n_bins = 0;
+    DevBuf<uint32_t> thr;                           // lt_thr | eq_val | flags (stream pass 1)
+    DevBuf<double> d_obs;                           // obs_eff (column-tiled pass 1)
+    DevBuf<unsigned long long> acc;                 // isum | n_lt | n_eq | sq_lo | sq_hi | below | above   [7][A]
+    DevBuf<uint32_t> mm;                            // min | max [2][A], then vmax, error
+    DevBuf<uint32_t> win;                           // lo | width [2][A]
+    DevBuf<unsigned long long> bin_off;             // [A]
+    DevBuf<uint32_t> bins;                          // [n_bins]
+};
+
+static int colacc_error_check(gatb_colacc *c)
+{
+    gatb_ctx *ctx = c->ctx;
+    uint32_t err = 0;
+    CU(ctx, cudaMemcpyAsync(&err, c->mm.p + 2 * (size_t)c->A + 1, sizeof(err), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    if (err) return fail(ctx, GATB_ERR_CUDA, "column accumulator: a TMA copy did not complete");
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_create(gatb_ctx *ctx, int n_cols, uint64_t n_samples_total, const double *observed,
+                                  const double *ref_fold, gatb_colacc **out)
+{
+    if (!ctx || !observed || !out || n_cols <= 0) return GATB_ERR_INVALID;
+    *out = nullptr;
+    if (n_samples_total < 1 || n_samples_total >= (1ull << 32))
+        return fail(ctx, GATB_ERR_INVALID, "colacc_create: n_samples_total must be in [1, 2^32)");
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    gatb_colacc *c = new gatb_colacc();
+    c->ctx = ctx; c->A = (uint32_t)n_cols; c->l = n_samples_total;
+    const uint32_t A = c->A;
+    c->observed.assign(observed, observed + A);
+    if (ref_fold) c->ref.assign(ref_fold, ref_fold + A);
+    int rc = effective_observed(ctx, A, observed, ref_fold, c->obs_eff);
+    if (rc) { delete c; return rc; }
+    ci_ranks(c->l, c->rank_lo, c->rank_hi);
+    std::vector<uint32_t> h_thr(3 * (size_t)A);
+    stats_stream_thresholds(c->obs_eff.data(), A, h_thr.data(), h_thr.data() + A, h_thr.data() + 2 * (size_t)A);
+    std::vector<uint32_t> h_mm(2 * (size_t)A + 2, 0u);
+    std::fill(h_mm.begin(), h_mm.begin() + A, 0xffffffffu);
+    c->lo.assign(A, 0u); c->width.assign(A, 0u);
+    std::vector<uint32_t> h_win(2 * (size_t)A, 0u);
+    std::vector<unsigned long long> h_off(A, 0ull);
+    cudaError_t e = c->thr.upload(h_thr.data(), h_thr.size(), st);
+    if (e == cudaSuccess) e = c->d_obs.upload(c->obs_eff.data(), A, st);
+    if (e == cudaSuccess) e = c->acc.alloc(7 * (size_t)A);
+    if (e == cudaSuccess) e = cudaMemsetAsync(c->acc.p, 0, 7 * (size_t)A * sizeof(unsigned long long), st);
+    if (e == cudaSuccess) e = c->mm.upload(h_mm.data(), h_mm.size(), st);
+    if (e == cudaSuccess) e = c->win.upload(h_win.data(), h_win.size(), st);
+    if (e == cudaSuccess) e = c->bin_off.upload(h_off.data(), A, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);          // (the host vectors above go out of scope)
+    if (e != cudaSuccess) { delete c; return fail(ctx, GATB_ERR_CUDA, std::string("colacc_create: ") + cudaGetErrorString(e)); }
+    *out = c;
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_set_windows(gatb_colacc *c, const uint32_t *lo, const uint32_t *width)
+{
+    if (!c || !lo || !width) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    const uint32_t A = c->A;
+    std::vector<unsigned long long> h_off(A);
+    uint64_t n = 0;
+    for (uint32_t a = 0; a < A; a++) {
+        if ((uint64_t)lo[a] + width[a] > (1ull << 32)) return fail(ctx, GATB_ERR_INVALID, "colacc_set_windows: window past 2^32");
+        h_off[a] = n;
+        n += width[a];
+    }
+    c->lo.assign(lo, lo + A); c->width.assign(width, width + A);
+    std::vector<uint32_t> h_win(2 * (size_t)A);
+    std::copy(lo, lo + A, h_win.begin());
+    std::copy(width, width + A, h_win.begin() + A);
+    CU(ctx, c->bins.alloc(std::max<uint64_t>(n, 1)));
+    c->n_bins = n;
+    CU(ctx, cudaMemsetAsync(c->bins.p, 0, std::max<uint64_t>(n, 1) * sizeof(uint32_t), st));
+    CU(ctx, cudaMemsetAsync(c->acc.p + 5 * (size_t)A, 0, 2 * (size_t)A * sizeof(unsigned long long), st));
+    CU(ctx, cudaMemcpyAsync(c->win.p, h_win.data(), h_win.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(ctx, cudaMemcpyAsync(c->bin_off.p, h_off.data(), A * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_add(gatb_colacc *c, const uint32_t *counts, uint64_t n_rows, uint64_t row_stride, int what)
+{
+    if (!c) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const uint32_t A = c->A;
+    if (what & ~(GATB_COLACC_SUMS | GATB_COLACC_HIST)) return fail(ctx, GATB_ERR_INVALID, "colacc_add: unknown flags");
+    if (n_rows == 0) return GATB_OK;
+    if (!counts || row_stride < A) return fail(ctx, GATB_ERR_INVALID, "colacc_add: no slab or row_stride < n_cols");
+    if ((what & GATB_COLACC_SUMS) && c->rows + n_rows > c->l)
+        return fail(ctx, GATB_ERR_INVALID, "colacc_add: more rows than n_samples_total");
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    unsigned long long *acc = c->acc.p;
+    if (what & GATB_COLACC_SUMS) {
+        if (ctx->stats_stream && row_stride == A && stats_stream_fits(counts, n_rows, A, ctx->smem_optin)) {
+            StreamStatsParams p;
+            memset(&p, 0, sizeof(p));
+            p.counts = counts; p.n_samples = n_rows; p.n_cols = A;
+            stats_stream_geometry(p);
+            p.lt_thr = c->thr.p; p.eq_val = c->thr.p + A; p.col_flags = c->thr.p + 2 * (size_t)A;
+            p.isum = acc; p.n_lt = acc + A; p.n_eq = acc + 2 * (size_t)A; p.sq_lo = acc + 3 * (size_t)A; p.sq_hi = acc + 4 * (size_t)A;
+            p.col_min = c->mm.p; p.col_max = c->mm.p + A;
+            p.vmax = c->mm.p + 2 * (size_t)A; p.error = c->mm.p + 2 * (size_t)A + 1;
+            ProfScope ps(ctx, PROF_OTHER);
+            CU(ctx, launch_stats_stream_pass1(st, p, ctx->sm_count));
+        } else {
+            // wider than a ring stage, strided or unaligned slabs: the column-tiled pass 1 (count.cu), accumulating
+            StatsParams p;
+            memset(&p, 0, sizeof(p));
+            p.counts = counts; p.n_samples = n_rows; p.n_cols = A; p.row_stride = row_stride; p.observed = c->d_obs.p;
+            p.accumulate = 1;
+            p.isum = acc; p.n_lt = acc + A; p.n_eq = acc + 2 * (size_t)A; p.sq_lo = acc + 3 * (size_t)A; p.sq_hi = acc + 4 * (size_t)A;
+            p.col_min = c->mm.p; p.col_max = c->mm.p + A;
+            ProfScope ps(ctx, PROF_OTHER);
+            launch_stats_pass1(st, p);
+            CU(ctx, cudaGetLastError());
+        }
+        c->rows += n_rows;
+    }
+    if (what & GATB_COLACC_HIST) {
+        ColHistParams h;
+        memset(&h, 0, sizeof(h));
+        h.counts = counts; h.n_rows = n_rows; h.row_stride = row_stride; h.n_cols = A;
+        h.lo = c->win.p; h.width = c->win.p + A; h.bin_off = c->bin_off.p; h.bins = c->bins.p; h.outside = acc + 5 * (size_t)A;
+        ProfScope ps(ctx, PROF_OTHER);
+        CU(ctx, launch_colacc_hist(st, h, ctx->sm_count));
+    }
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_state(gatb_colacc *c, uint64_t *rows, uint64_t *moments, uint32_t *minmax, uint64_t *outside,
+                                 uint32_t *bins)
+{
+    if (!c) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const size_t A = c->A;
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    if (const int rc = colacc_error_check(c)) return rc;
+    if (rows) *rows = c->rows;
+    if (moments) CU(ctx, cudaMemcpyAsync(moments, c->acc.p, 5 * A * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (outside) CU(ctx, cudaMemcpyAsync(outside, c->acc.p + 5 * A, 2 * A * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (minmax) CU(ctx, cudaMemcpyAsync(minmax, c->mm.p, 2 * A * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    if (bins && c->n_bins) CU(ctx, cudaMemcpyAsync(bins, c->bins.p, c->n_bins * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_merge(gatb_colacc *c, uint64_t rows, const uint64_t *moments, const uint32_t *minmax,
+                                 const uint64_t *outside, const uint32_t *bins)
+{
+    if (!c) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const size_t A = c->A;
+    if (c->rows + rows > c->l) return fail(ctx, GATB_ERR_INVALID, "colacc_merge: more rows than n_samples_total");
+    std::vector<uint64_t> m(5 * A), o(2 * A);
+    std::vector<uint32_t> mm(2 * A), b(c->n_bins);
+    uint64_t mine = 0;
+    if (const int rc = gatb_colacc_state(c, &mine, m.data(), mm.data(), o.data(), b.data())) return rc;
+    cudaStream_t st = ctx->stream;
+    if (moments) {
+        for (size_t a = 0; a < A; a++) {
+            const unsigned __int128 x = ((unsigned __int128)m[4 * A + a] << 64) | m[3 * A + a];
+            const unsigned __int128 y = ((unsigned __int128)moments[4 * A + a] << 64) | moments[3 * A + a];
+            const unsigned __int128 z = x + y;
+            m[3 * A + a] = (uint64_t)z; m[4 * A + a] = (uint64_t)(z >> 64);
+            for (int k = 0; k < 3; k++) m[k * A + a] += moments[k * A + a];
+        }
+        CU(ctx, cudaMemcpyAsync(c->acc.p, m.data(), 5 * A * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+        c->rows += rows;
+    }
+    if (minmax) {
+        for (size_t a = 0; a < A; a++) { mm[a] = std::min(mm[a], minmax[a]); mm[A + a] = std::max(mm[A + a], minmax[A + a]); }
+        CU(ctx, cudaMemcpyAsync(c->mm.p, mm.data(), 2 * A * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    }
+    if (outside) {
+        for (size_t i = 0; i < 2 * A; i++) o[i] += outside[i];
+        CU(ctx, cudaMemcpyAsync(c->acc.p + 5 * A, o.data(), 2 * A * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    }
+    if (bins && c->n_bins) {
+        for (uint64_t i = 0; i < c->n_bins; i++) b[i] += bins[i];
+        CU(ctx, cudaMemcpyAsync(c->bins.p, b.data(), c->n_bins * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    }
+    CU(ctx, cudaStreamSynchronize(st));
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_finish(gatb_colacc *c, double pseudo_count, double *expected, double *stddev, double *lower95,
+                                  double *upper95, double *fold, double *pvalue, uint8_t *missed)
+{
+    if (!c) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const uint32_t A = c->A;
+    const uint64_t l = c->l;
+    if (c->rows != l)
+        return fail(ctx, GATB_ERR_INVALID, "colacc_finish: the sums hold " + std::to_string(c->rows) + " of " +
+                                               std::to_string(l) + " samples");
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    DevBuf<uint32_t> d_q;                           // q [2][A] | missed [A]
+    DevBuf<unsigned long long> d_total;
+    CU(ctx, d_q.alloc(3 * (size_t)A));
+    CU(ctx, d_total.alloc(A));
+    ColHistParams h;
+    memset(&h, 0, sizeof(h));
+    h.n_cols = A; h.lo = c->win.p; h.width = c->win.p + A; h.bin_off = c->bin_off.p; h.bins = c->bins.p;
+    h.outside = c->acc.p + 5 * (size_t)A;
+    h.n_samples = l; h.rank_lo = c->rank_lo; h.rank_hi = c->rank_hi;
+    h.q = d_q.p; h.missed = d_q.p + 2 * (size_t)A; h.total = d_total.p;
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_pick(st, h)); }
+    std::vector<unsigned long long> m(5 * (size_t)A), total(A);
+    std::vector<uint32_t> q(3 * (size_t)A);
+    CU(ctx, cudaMemcpyAsync(m.data(), c->acc.p, m.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaMemcpyAsync(q.data(), d_q.p, q.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaMemcpyAsync(total.data(), d_total.p, A * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    if (const int rc = colacc_error_check(c)) return rc;
+    std::vector<double> mean(A), sq(A), qlo(A), qhi(A);
+    for (uint32_t a = 0; a < A; a++) {
+        if (total[a] != l)
+            return fail(ctx, GATB_ERR_INVALID, "colacc_finish: the histogram of column " + std::to_string(a) + " holds " +
+                                                   std::to_string(total[a]) + " of " + std::to_string(l) + " samples");
+        mean[a] = (double)m[a] / (double)l;
+        sq[a] = exact_sumsq_dev(l, m[a], m[3 * (size_t)A + a], m[4 * (size_t)A + a]);
+        const bool miss = q[2 * (size_t)A + a] != 0;
+        qlo[a] = miss ? NAN : (double)q[a];
+        qhi[a] = miss ? NAN : (double)q[A + a];
+        if (missed) missed[a] = miss ? 1 : 0;
+    }
+    finish_columns(l, A, c->observed.data(), c->obs_eff.data(), c->ref.empty() ? nullptr : c->ref.data(), pseudo_count,
+                   mean.data(), sq.data(), qlo.data(), qhi.data(), m.data() + A, m.data() + 2 * (size_t)A,
+                   expected, stddev, lower95, upper95, fold, pvalue);
+    return GATB_OK;
+}
+
+extern "C" void gatb_colacc_destroy(gatb_colacc *c)
+{
+    if (!c) return;
+    cudaSetDevice(c->ctx->device);
+    tl_stream = c->ctx->stream;
+    delete c;                                       // (the buffers go back to the pool in stream order)
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -628,25 +628,30 @@ __global__ void __launch_bounds__(STATS_COLS * STATS_ROWS) stats_pass1_kernel(St
 {
     __shared__ unsigned long long su[5][STATS_ROWS][STATS_COLS];
     __shared__ double sd[STATS_ROWS][STATS_COLS];
+    __shared__ uint32_t smm[2][STATS_ROWS][STATS_COLS];
     const StatsThread t = stats_thread(p);
     const double obs = t.live ? p.observed[t.col] : 0.0;
+    const uint64_t ld = p.row_stride ? p.row_stride : p.n_cols;
     unsigned long long isum = 0, nlt = 0, neq = 0, sq_lo = 0, sq_hi = 0;
+    uint32_t vmin = 0xffffffffu, vmax = 0u;
     double fsum = 0.0;
     if (t.live)
         for (uint64_t s = t.r; s < p.n_samples; s += STATS_ROWS) {
             double x;
-            if (p.is_float) { x = reinterpret_cast<const double *>(p.counts)[s * p.n_cols + t.col]; fsum += x; }
+            if (p.is_float) { x = reinterpret_cast<const double *>(p.counts)[s * ld + t.col]; fsum += x; }
             else {
-                const uint32_t v = reinterpret_cast<const uint32_t *>(p.counts)[s * p.n_cols + t.col];
+                const uint32_t v = reinterpret_cast<const uint32_t *>(p.counts)[s * ld + t.col];
                 const unsigned long long v2 = (unsigned long long)v * v;
                 isum += v; x = (double)v;
                 sq_lo += v2; sq_hi += (sq_lo < v2) ? 1ull : 0ull;       // exact sum of squares (as in stats_stream.cu)
+                vmin = min(vmin, v); vmax = max(vmax, v);
             }
             nlt += (x < obs) ? 1ull : 0ull;      // searchargsorted + cmpDouble (gat/Engine.pyx:122-127, 1549-1557)
             neq += (x == obs) ? 1ull : 0ull;
         }
     su[0][t.r][t.c] = nlt; su[1][t.r][t.c] = neq; su[2][t.r][t.c] = isum; su[3][t.r][t.c] = sq_lo; su[4][t.r][t.c] = sq_hi;
     sd[t.r][t.c] = fsum;
+    smm[0][t.r][t.c] = vmin; smm[1][t.r][t.c] = vmax;
     __syncthreads();
     if (t.r == 0 && t.live) {
         unsigned long long a = 0, b = 0, c = 0, lo = 0, hi = 0;
@@ -655,6 +660,15 @@ __global__ void __launch_bounds__(STATS_COLS * STATS_ROWS) stats_pass1_kernel(St
             a += su[0][r][t.c]; b += su[1][r][t.c]; c += su[2][r][t.c]; f += sd[r][t.c];
             const unsigned long long l2 = su[3][r][t.c];
             lo += l2; hi += su[4][r][t.c] + ((lo < l2) ? 1ull : 0ull);
+            vmin = min(vmin, smm[0][r][t.c]); vmax = max(vmax, smm[1][r][t.c]);
+        }
+        if (p.accumulate) {
+            // (the low word's atomic reports its own carry into the high word, whatever the order of the adds)
+            atomicAdd(p.n_lt + t.col, a); atomicAdd(p.n_eq + t.col, b); atomicAdd(p.isum + t.col, c);
+            const unsigned long long old = atomicAdd(p.sq_lo + t.col, lo);
+            atomicAdd(p.sq_hi + t.col, hi + ((old + lo < old) ? 1ull : 0ull));
+            if (p.n_samples) { atomicMin(p.col_min + t.col, vmin); atomicMax(p.col_max + t.col, vmax); }
+            return;
         }
         p.n_lt[t.col] = a; p.n_eq[t.col] = b;
         p.sum[t.col] = p.is_float ? f : (double)c;

@@ -146,6 +146,12 @@ struct StatsParams {
     double *q_lo, *q_hi;            // order statistics at ranks rank_lo / rank_hi
     uint64_t rank_lo, rank_hi;
     const double *mean;             // device [n_cols] (second pass)
+    // pass 1 of a column accumulator (gatb_colacc_add, uint32 only): the integer results are ADDED to n_lt / n_eq /
+    // isum / sq_lo / sq_hi and the per-column extremes folded into col_min / col_max, so that successive slabs of
+    // rows give what one pass over all of them gives; rows are row_stride elements apart
+    int accumulate;
+    uint64_t row_stride;
+    uint32_t *col_min, *col_max;
 };
 // gat-compare (scripts/gat-compare.py:218-241, :300-323): the sampled log ratio of two fold-change columns,
 //   out[s][p] = log((obs1[p] / (m1[s][col1[p]] + pc) + 1e-4) / (obs2[p] / (m2[s][col2[p]] + pc) + 1e-4)) + delta[p]
@@ -184,6 +190,7 @@ struct StreamStatsParams {
     unsigned long long *isum, *n_lt, *n_eq;
     unsigned long long *sq_lo, *sq_hi;   // sum of squares, 128 bits
     uint32_t *vmax;                 // largest value of the matrix
+    uint32_t *col_min, *col_max;    // pass 1 of a column accumulator: extremes of every column (NULL: not wanted)
     // select pass at bit `shift` (4 bits): prefix / rank per (which rank, column), [2][n_cols]
     uint32_t shift;
     uint32_t *prefix, *prefix_out;
@@ -197,6 +204,26 @@ void stats_stream_geometry(StreamStatsParams &p);
 void stats_stream_thresholds(const double *observed, uint32_t n_cols, uint32_t *lt_thr, uint32_t *eq_val, uint32_t *flags);
 cudaError_t launch_stats_stream_pass1(cudaStream_t st, StreamStatsParams p, int sm_count);
 cudaError_t launch_stats_stream_select(cudaStream_t st, StreamStatsParams p, int sm_count, size_t smem_optin);
+
+// Quantile-window histograms of a column accumulator (gatb_colacc_*).  Column a owns the unit-width uint32 bins
+// [lo[a], lo[a] + width[a]) at bins + bin_off[a]; a value below / above its window counts into outside[a] /
+// outside[n_cols + a].
+struct ColHistParams {
+    const uint32_t *counts;         // slab [n_rows][row_stride], the first n_cols of every row
+    uint64_t n_rows, row_stride;
+    uint32_t n_cols;
+    const uint32_t *lo, *width;
+    const unsigned long long *bin_off;
+    uint32_t *bins;
+    unsigned long long *outside;    // [2][n_cols]
+    // pick: the values of ranks rank_lo / rank_hi of n_samples (the whole column: below + bins + above)
+    uint64_t n_samples, rank_lo, rank_hi;
+    uint32_t *q;                    // out [2][n_cols]
+    unsigned long long *total;      // out [n_cols]: samples the histogram of the column holds
+    uint32_t *missed;               // out [n_cols]: 1 when a rank falls below or above the window
+};
+cudaError_t launch_colacc_hist(cudaStream_t st, const ColHistParams &p, int sm_count);
+cudaError_t launch_colacc_pick(cudaStream_t st, const ColHistParams &p);
 
 void launch_stats_pass1(cudaStream_t st, const StatsParams &p);
 void launch_stats_pass2(cudaStream_t st, const StatsParams &p);

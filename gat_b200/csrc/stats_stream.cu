@@ -11,6 +11,7 @@
 //   pass 1   sum x (uint64), sum x^2 (128 bits), #{x < observed}, #{x == observed}, max -- all integers, accumulated
 //            with atomics: exact, so the results do not depend on the grid, the GPU or the column layout.  The
 //            variance follows on the host from the exact n * sum x^2 - (sum x)^2 (no second pass over the matrix)
+//            (pass 1 of a column accumulator, MODE 2: the same, plus the smallest and largest value of every column)
 //   select   radix select of the two order statistics (CI bounds), 4 bits per pass from the highest non-zero
 //            nibble of the matrix maximum: per-CTA histograms [rank][nibble][column] in shared memory, flushed to
 //            global counters; stats_pick_kernel narrows prefix and rank between passes
@@ -53,7 +54,7 @@ struct ChunkSeq {
 // the bits above the nibble a select pass at `shift` decides
 __host__ __device__ __forceinline__ uint32_t hmask_of(uint32_t shift) { return shift >= 28u ? 0u : (0xffffffffu << (shift + 4u)); }
 
-// MODE 0: pass 1, 1: select pass.  KC = columns per thread (thread (c, r) owns columns c, c + CW, ...).  The inner
+// MODE 0: pass 1, 1: select pass, 2: pass 1 with per-column extremes.  KC = columns per thread (thread (c, r) owns columns c, c + CW, ...).  The inner
 // loops address shared memory by 32-bit shared address and keep every per-element step to a handful of integer
 // instructions (about 12 in pass 1, 8 in a select pass): at 4 bytes per element the passes only stay HBM-bound if
 // the SMs can issue an element's work in the time its 4 bytes take to arrive.
@@ -61,6 +62,7 @@ template <int MODE, int KC>
 __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
 {
     extern __shared__ __align__(16) uint8_t smem[];
+    constexpr bool P1 = MODE != 1, MM = MODE == 2;
     const uint32_t T = blockDim.x, tid = threadIdx.x;
     const uint32_t CW = p.col_width, RW = T / CW;           // threads across columns, row lanes
     const uint32_t c = tid % CW, r = tid / CW;
@@ -101,14 +103,15 @@ __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
     uint32_t neg_thr[KC], inv_eq[KC];                       // pass 1: 2^32 - lt_thr and ~eq_val (count_carry)
     unsigned long long sum[KC], sq_lo[KC];
     uint32_t sq_hi[KC], nge[KC], ngt[KC], vmax = 0, nrows = 0;
+    uint32_t cmin[KC], cmax[KC];                            // MODE 2
     uint32_t pre0[KC], pre1[KC], h0[KC];                    // select: prefixes, shared address of the column's counters
 #pragma unroll
     for (int k = 0; k < KC; k++) {
         const uint32_t col = c + (uint32_t)k * CW;
         live[k] = col < p.n_cols;
         coff[k] = live[k] ? col * 4u : 0u;
-        neg_thr[k] = (MODE == 0 && live[k]) ? 0u - p.lt_thr[col] : 0u;
-        inv_eq[k] = (MODE == 0 && live[k]) ? ~p.eq_val[col] : 0u;
+        neg_thr[k] = (P1 && live[k]) ? 0u - p.lt_thr[col] : 0u;
+        inv_eq[k] = (P1 && live[k]) ? ~p.eq_val[col] : 0u;
         pre0[k] = (MODE == 1 && live[k]) ? p.prefix[col] : 0u;
         pre1[k] = (MODE == 1 && live[k]) ? p.prefix[p.n_cols + col] : 0u;
         // (a dead column counts into the padding slot HS - 1 of its rows, which is never flushed)
@@ -120,6 +123,7 @@ __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
         coff[k] = pin_reg(coff[k]);
         sum[k] = sq_lo[k] = 0ull;
         sq_hi[k] = nge[k] = ngt[k] = 0u;
+        cmin[k] = 0xffffffffu; cmax[k] = 0u;
     }
     const uint32_t hmask = pin_reg(hmask_of(p.shift));      // bits already decided
     const uint32_t HS4 = pin_reg(4u * HS), H1 = pin_reg(4u * 16u * HS), shift = pin_reg(p.shift);
@@ -148,16 +152,17 @@ __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
 #pragma unroll 4
         for (uint32_t row = r; row < rows; row += RW) {
             const uint32_t rowa = stage + row * row_bytes;
-            if (MODE == 0) nrows++;
+            if (P1) nrows++;
 #pragma unroll
             for (int k = 0; k < KC; k++) {
                 const uint32_t v = lds32(rowa + coff[k]);
-                if (MODE == 0) {
+                if (P1) {
                     sum[k] += v;
                     add96_sq(sq_lo[k], sq_hi[k], v);
                     count_carry(nge[k], v, neg_thr[k]);          // v >= lt_thr; searchargsorted + cmpDouble (gat/Engine.pyx:122-127, 1549-1557)
                     count_carry(ngt[k], v, inv_eq[k]);           // v > eq_val (#equal = #(>= t) - #(> t) when observed is an integer t)
                     vmax = max(vmax, v);
+                    if (MM) { cmin[k] = min(cmin[k], v); cmax[k] = max(cmax[k], v); }
                 } else {
                     // unconditional reductions (ptxas branches around a predicated one): an element that does not
                     // carry the prefix counts into a padding slot, where the hardware merges the lanes' increments
@@ -177,7 +182,7 @@ __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
         if (++s == n_stages) { s = 0; parity ^= 1u; }
     }
 
-    if (MODE == 0) {
+    if (P1) {
         // integers: exact and order-independent, one atomic per column, row lane and CTA.  The 128-bit sum of
         // squares: every atomic on the low word reports its own carry, whatever the order
 #pragma unroll
@@ -199,6 +204,7 @@ __global__ void __launch_bounds__(1024) stats_stream_kernel(StreamStatsParams p)
                 const uint32_t lt = (fl & SS_ALL_LESS) ? nrows : nrows - ge, eq = (fl & SS_HAS_EQUAL) ? ge - ngt[k] : 0u;
                 if (lt) atomicAdd(p.n_lt + col, (unsigned long long)lt);
                 if (eq) atomicAdd(p.n_eq + col, (unsigned long long)eq);
+                if (MM) { atomicMin(p.col_min + col, cmin[k]); atomicMax(p.col_max + col, cmax[k]); }
             }
         }
         vmax = __reduce_max_sync(GATB_FULL, vmax);
@@ -307,7 +313,7 @@ void stats_stream_thresholds(const double *observed, uint32_t n_cols, uint32_t *
 cudaError_t launch_stats_stream_pass1(cudaStream_t st, StreamStatsParams p, int sm_count)
 {
     p.n_stages = 3;
-    return launch_stream_mode<0>(st, p, sm_count);
+    return p.col_min ? launch_stream_mode<2>(st, p, sm_count) : launch_stream_mode<0>(st, p, sm_count);
 }
 
 // one 4-bit select pass at p.shift (prefix / rank / hist as the previous pass left them)
@@ -322,6 +328,103 @@ cudaError_t launch_stats_stream_select(cudaStream_t st, StreamStatsParams p, int
     const unsigned nb = (2u * p.n_cols + 255u) / 256u;
     stats_pick_kernel<<<nb, 256, 0, st>>>(p);
     stats_pick_commit_kernel<<<nb, 256, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Quantile-window histograms (gatb_colacc_*): the two CI95 order statistics of a column without its samples.  Bins
+// are exact values, so the ranks stay exact.  Thread = column of a row, CTAs stride over the rows: the 32 increments
+// of a warp go to 32 different columns' windows, never to one address, and the arena (columns x window width x 4
+// bytes) stays in L2, where the reductions (RED, no return value) are served.  Increments of the same bin from
+// different rows are spread over time by the row stride of the grid.
+constexpr uint32_t CH_THREADS = 256, CH_UNROLL = 4;
+
+__global__ void __launch_bounds__(CH_THREADS) colacc_hist_kernel(ColHistParams p)
+{
+    const uint32_t a = blockIdx.x * CH_THREADS + threadIdx.x;
+    if (a >= p.n_cols) return;
+    const uint32_t lo = p.lo[a], w = p.width[a];
+    uint32_t *bins = p.bins + p.bin_off[a];
+    uint32_t below = 0, above = 0;
+    const uint64_t step = gridDim.y;
+    uint64_t row = blockIdx.y;
+    for (; row + (CH_UNROLL - 1) * step < p.n_rows; row += CH_UNROLL * step) {
+        uint32_t v[CH_UNROLL];
+#pragma unroll
+        for (uint32_t u = 0; u < CH_UNROLL; u++) v[u] = p.counts[(row + u * step) * p.row_stride + a];
+#pragma unroll
+        for (uint32_t u = 0; u < CH_UNROLL; u++) {
+            const uint32_t d = v[u] - lo;               // (a value below the window wraps to >= w)
+            if (d < w) atomicAdd(bins + d, 1u);
+            else if (v[u] < lo) below++;
+            else above++;
+        }
+    }
+    for (; row < p.n_rows; row += step) {
+        const uint32_t v = p.counts[row * p.row_stride + a], d = v - lo;
+        if (d < w) atomicAdd(bins + d, 1u);
+        else if (v < lo) below++;
+        else above++;
+    }
+    if (below) atomicAdd(p.outside + a, (unsigned long long)below);
+    if (above) atomicAdd(p.outside + p.n_cols + a, (unsigned long long)above);
+}
+
+// one CTA per column: the bins are cut into one run per thread, a scan of the run totals finds the run that holds
+// each rank, and that thread walks its run to the bin
+__global__ void __launch_bounds__(CH_THREADS) colacc_pick_kernel(ColHistParams p)
+{
+    __shared__ unsigned long long part[CH_THREADS + 1];
+    const uint32_t a = blockIdx.x, tid = threadIdx.x;
+    const uint32_t w = p.width[a];
+    const uint32_t *bins = p.bins + p.bin_off[a];
+    const unsigned long long below = p.outside[a], above = p.outside[p.n_cols + a];
+    const uint32_t run = (w + CH_THREADS - 1u) / CH_THREADS;
+    const uint32_t b0 = min(w, tid * run), b1 = min(w, b0 + run);
+    unsigned long long s = 0;
+    for (uint32_t b = b0; b < b1; b++) s += bins[b];
+    part[tid + 1] = s;
+    __syncthreads();
+    if (tid == 0) {
+        part[0] = below;
+        for (uint32_t i = 1; i <= CH_THREADS; i++) part[i] += part[i - 1];     // part[i] = below + bins before run i
+        const unsigned long long inside_end = part[CH_THREADS];
+        p.total[a] = inside_end + above;
+        const bool miss = p.rank_lo < below || p.rank_lo >= inside_end || p.rank_hi < below || p.rank_hi >= inside_end;
+        p.missed[a] = miss ? 1u : 0u;
+        if (miss) { p.q[a] = 0u; p.q[p.n_cols + a] = 0u; }
+    }
+    __syncthreads();
+    const unsigned long long first = part[tid], last = part[tid + 1];
+#pragma unroll
+    for (int which = 0; which < 2; which++) {
+        const unsigned long long rank = which ? p.rank_hi : p.rank_lo;
+        if (rank < first || rank >= last) continue;
+        unsigned long long cum = first;
+        uint32_t b = b0;
+        for (; b < b1; b++) {
+            cum += bins[b];
+            if (cum > rank) break;
+        }
+        p.q[(uint64_t)which * p.n_cols + a] = p.lo[a] + b;
+    }
+}
+
+cudaError_t launch_colacc_hist(cudaStream_t st, const ColHistParams &p, int sm_count)
+{
+    if (p.n_rows == 0 || p.n_cols == 0) return cudaSuccess;
+    const uint32_t gx = (p.n_cols + CH_THREADS - 1u) / CH_THREADS;
+    // about 8 CTAs of 256 threads per SM, every CTA at least a few unrolled steps of rows
+    const uint64_t gy = std::max<uint64_t>(1, std::min<uint64_t>((p.n_rows + 2 * CH_UNROLL - 1) / (2 * CH_UNROLL),
+                                                                 std::max<uint64_t>(1, (uint64_t)sm_count * 8u / gx)));
+    colacc_hist_kernel<<<dim3(gx, (unsigned)std::min<uint64_t>(gy, 65535u)), CH_THREADS, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_colacc_pick(cudaStream_t st, const ColHistParams &p)
+{
+    if (p.n_cols == 0) return cudaSuccess;
+    colacc_pick_kernel<<<p.n_cols, CH_THREADS, 0, st>>>(p);
     return cudaGetLastError();
 }
 

@@ -214,6 +214,73 @@ class Context(object):
         return dict(zip(["expected", "stddev", "lower95", "upper95", "fold", "pvalue"], outs))
 
 
+class ColumnAccumulator(object):
+    """the statistics of one uint32 counter plane [n_samples][n_cols] from slabs of rows, without the matrix
+    (gatb_colacc): exact sums per column, and unit-width histogram windows for the two CI95 order statistics."""
+
+    STATS = ["expected", "stddev", "lower95", "upper95", "fold", "pvalue"]
+
+    def __init__(self, ctx, n_cols, n_samples, observed, ref_fold=None):
+        self.ctx = ctx
+        self.n_cols, self.n_samples = int(n_cols), int(n_samples)
+        obs = np.ascontiguousarray(observed, dtype=np.float64)
+        ref = None if ref_fold is None else np.ascontiguousarray(ref_fold, dtype=np.float64)
+        h = ctypes.c_void_p()
+        ctx.check(ctx.lib.gatb_colacc_create(ctx.handle, self.n_cols, self.n_samples, _p(obs), _p(ref), ctypes.byref(h)))
+        self.handle = h
+        self.n_bins = 0
+
+    def set_windows(self, lo, width):
+        """column a counts the values lo[a] .. lo[a] + width[a] - 1 into bins; clears the histograms"""
+        lo = np.ascontiguousarray(lo, dtype=np.uint32)
+        width = np.ascontiguousarray(width, dtype=np.uint32)
+        self.ctx.check(self.ctx.lib.gatb_colacc_set_windows(self.handle, _p(lo), _p(width)))
+        self.n_bins = int(width.astype(np.uint64).sum())
+
+    def add(self, device_ptr, n_rows, row_stride=None, sums=True, hist=True):
+        """count a device slab of n_rows rows (enqueued on the context's stream)"""
+        what = (_lib.COLACC_SUMS if sums else 0) | (_lib.COLACC_HIST if hist else 0)
+        self.ctx.check(self.ctx.lib.gatb_colacc_add(self.handle, ctypes.c_void_p(device_ptr), int(n_rows),
+                                                    int(row_stride or self.n_cols), what))
+
+    def state(self):
+        """-> dict of the integer state (rows, moments [5][A], minmax [2][A], outside [2][A], bins)"""
+        A = self.n_cols
+        rows = np.zeros(1, dtype=np.uint64)
+        st = dict(moments=np.zeros((5, A), dtype=np.uint64), minmax=np.zeros((2, A), dtype=np.uint32),
+                  outside=np.zeros((2, A), dtype=np.uint64), bins=np.zeros(max(self.n_bins, 1), dtype=np.uint32))
+        self.ctx.check(self.ctx.lib.gatb_colacc_state(self.handle, _p(rows), _p(st["moments"]), _p(st["minmax"]),
+                                                      _p(st["outside"]), _p(st["bins"])))
+        st["rows"] = int(rows[0])
+        return st
+
+    def merge(self, st, sums=True):
+        """add another accumulator's state (sums=False: only its histograms) into this one"""
+        self.ctx.check(self.ctx.lib.gatb_colacc_merge(
+            self.handle, st["rows"] if sums else 0, _p(st["moments"]) if sums else None,
+            _p(st["minmax"]) if sums else None, _p(st["outside"]), _p(st["bins"])))
+
+    def finish(self, pseudo_count=1.0):
+        """-> (statistics dict as Context.column_stats returns it, missed bool [A])"""
+        outs = [np.zeros(self.n_cols, dtype=np.float64) for _ in self.STATS]
+        missed = np.zeros(self.n_cols, dtype=np.uint8)
+        self.ctx.check(self.ctx.lib.gatb_colacc_finish(self.handle, float(pseudo_count), *[_p(o) for o in outs],
+                                                       _p(missed)))
+        return dict(zip(self.STATS, outs)), missed.astype(bool)
+
+    def close(self):
+        if getattr(self, "handle", None):
+            if self.ctx.handle:
+                self.ctx.lib.gatb_colacc_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Lists(object):
     """interval lists resident on the GPU as CSR (gatb_lists): the device side of input preparation."""
 

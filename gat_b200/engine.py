@@ -925,6 +925,24 @@ class SampleMatrix(object):
         return getContext().format_counts(counts=self._host)
 
 
+class SamplesNotKept(SampleMatrix):
+    """Stands in for the sample matrix of a run with keep_samples=False (gat_b200.run): the statistics were
+    computed from slabs of samples that no longer exist, so the samples themselves cannot be handed out."""
+
+    def __init__(self, nsamples, ncolumns):
+        self._tensor = self._host = None
+        self._as_uint32 = True
+        self.nsamples = int(nsamples)
+        self.first_column = 0
+        self.ncolumns = int(ncolumns)
+
+    def _refuse(self, *args):
+        raise RuntimeError("the samples of this result were not kept (gat_b200.run with keep_samples=False computes "
+                           "the statistics without the sample matrix); run with keep_samples=True to keep them")
+
+    host = column = text = _refuse
+
+
 class AnnotatorResult(object):
     """observed vs simulated counts of one (track, annotation, counter) with expected, CI95, stddev,
     fold, empirical p-value and q-value (gat/Engine.pyx:1725-1852).  The statistics are computed on

@@ -313,6 +313,49 @@ int  gatb_column_pvalue(gatb_ctx *ctx, const void *counts, int is_float, int cou
                         uint64_t n_samples, int n_cols, const double *values, const double *expected,
                         double *pvalue);
 
+/* ---- per-column statistics without the sample matrix ----------------------------------------------
+ * Replaces makeEnrichmentStatistics + getTwoSidedPValue (gat/Engine.pyx:1635-1718, :1543-1576) like
+ * gatb_column_stats, for a uint32 counter plane [n_samples_total][n_cols] that is never held whole: the rows
+ * arrive as slabs in device memory (e.g. what gatb_run writes with out_is_device), are counted and may then be
+ * overwritten.  The accumulator keeps exact integers per column -- sum, 128-bit sum of squares, #{x < observed},
+ * #{x == observed}, smallest and largest value -- plus, for the two CI95 order statistics, a window of unit-width
+ * uint32 bins [lo[a], lo[a] + width[a]) per column and the counts below / above it.  Integers add across slabs (and
+ * across ranks, gatb_colacc_state / gatb_colacc_merge), so for every column whose two CI ranks fall inside its
+ * window gatb_colacc_finish returns exactly the doubles gatb_column_stats returns for the whole matrix.  A column
+ * whose rank falls outside ("missed") needs its histogram again with a wider window ([min, max] of the column
+ * always holds it): set new windows and add the same rows once more with GATB_COLACC_HIST only. */
+typedef struct gatb_colacc gatb_colacc;
+#define GATB_COLACC_SUMS 1   /* gatb_colacc_add: count the rows into the sums (each row of the plane once)    */
+#define GATB_COLACC_HIST 2   /*                  count the rows into the windows' histograms                 */
+
+/* observed[n_cols], ref_fold[n_cols] (NULL = no --null reference): host, as in gatb_column_stats;
+ * 1 <= n_samples_total < 2^32.  Every column starts with an empty window (every value counts as above it). */
+int  gatb_colacc_create(gatb_ctx *ctx, int n_cols, uint64_t n_samples_total, const double *observed,
+                        const double *ref_fold, gatb_colacc **out);
+/* lo[n_cols], width[n_cols] (host): the windows; clears the histograms (and below / above), keeps the sums.  The
+ * bins of all columns live in one device arena of sum(width) uint32 (lo + width <= 2^32). */
+int  gatb_colacc_set_windows(gatb_colacc *acc, const uint32_t *lo, const uint32_t *width);
+/* counts (dev): n_rows rows of n_cols uint32, row_stride (>= n_cols) elements apart.  what: GATB_COLACC_SUMS
+ * and/or GATB_COLACC_HIST.  Enqueued on the context's stream, no synchronisation: the slab may be reused by
+ * work enqueued after it on that stream. */
+int  gatb_colacc_add(gatb_colacc *acc, const uint32_t *counts, uint64_t n_rows, uint64_t row_stride, int what);
+/* the integer state, host arrays, any of them NULL: rows counted into the sums, moments [5][n_cols] (sum,
+ * #{x < observed}, #{x == observed}, sum x^2 low 64 bits, high 64 bits), minmax [2][n_cols], outside [2][n_cols]
+ * (below, above), bins [sum(width)]. */
+int  gatb_colacc_state(gatb_colacc *acc, uint64_t *rows, uint64_t *moments, uint32_t *minmax, uint64_t *outside,
+                       uint32_t *bins);
+/* adds another accumulator's state (same columns, observed values and windows; gatb_colacc_state layout) into
+ * this one: the sum of squares with its carry, min / max, counts. */
+int  gatb_colacc_merge(gatb_colacc *acc, uint64_t rows, const uint64_t *moments, const uint32_t *minmax,
+                       const uint64_t *outside, const uint32_t *bins);
+/* the statistics of gatb_column_stats (host outputs of n_cols doubles, any may be NULL) once the sums hold
+ * n_samples_total rows and every histogram n_samples_total values (GATB_ERR_INVALID otherwise).  missed[n_cols]
+ * (host, may be NULL): 1 where a CI rank fell outside the column's window -- lower95 / upper95 are NaN there,
+ * every other output is exact. */
+int  gatb_colacc_finish(gatb_colacc *acc, double pseudo_count, double *expected, double *stddev, double *lower95,
+                        double *upper95, double *fold, double *pvalue, uint8_t *missed);
+void gatb_colacc_destroy(gatb_colacc *acc);
+
 /* ---- gat-compare: pairwise comparison of fold changes ----------------------------------------------
  * Replaces the inner loop of scripts/gat-compare.py (:218-241 within one counts file, :300-323 between
  * two): for pair q of columns (col1[q] of m1, col2[q] of m2)
