@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <chrono>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -1519,15 +1520,17 @@ extern "C" int gatb_count_work(gatb_sampler *s, const gatb_annotations *annos, u
 
 // ---------------------------------------------------------------------------------------------------
 // column statistics
-// The streaming passes of stats_stream.cu on a device-resident uint32 matrix (what gatb_run leaves behind):
-// pass 1 always; with `full`, pass 2 and the select passes as well.  Outputs as host vectors.
-// sum (x - mean)^2 of n uint32 values from their exact sums: (n * sum x^2 - (sum x)^2) / n with the numerator exact in
-// 128 bits (x < 2^32, n < 2^32: both products stay below 2^128), rounded once when it becomes a double
-static double exact_sumsq_dev(uint64_t n, unsigned long long sum, unsigned long long sq_lo, unsigned long long sq_hi)
+// getTwoSidedPValue (gat/Engine.pyx:1543-1576) from counts instead of a sorted copy of the l samples: n_lt = lower_bound
+// of value in them, n_eq = #{x == value}; value above centre (the column's expectation) takes the upper tail
+static double two_sided_pvalue(uint64_t l, uint64_t n_lt, uint64_t n_eq, double value, double centre)
 {
-    const unsigned __int128 sq = ((unsigned __int128)sq_hi << 64) | sq_lo;
-    const unsigned __int128 num = (unsigned __int128)n * sq - (unsigned __int128)sum * sum;
-    return (double)num / (double)n;
+    uint64_t idx = n_lt;
+    if (n_lt == l) idx = 1;
+    else if (value > centre) {
+        if (n_eq > 0 && n_lt > 0) idx = n_lt - 1;                           // sorted[n_lt] == value
+        idx = l - (idx + 1);
+    } else if (n_eq > 0) idx = n_lt + n_eq;
+    return std::max(1.0 / (double)l, (double)idx / (double)l);
 }
 
 // The per-column doubles of makeEnrichmentStatistics (gat/Engine.pyx:1635-1718) from a column's reduced integers /
@@ -1546,24 +1549,12 @@ static void finish_columns(uint64_t l, uint32_t A, const double *observed, const
         const double fo = (exp_ != 0) ? (observed[a] + pseudo_count) / (exp_ + pseudo_count) : 1.0;   // :1679-1682
         double lo = qlo[a], hi = qhi[a];
         if (ref_fold) { lo *= ref_fold[a]; hi *= ref_fold[a]; }              // :1713-1714
-        // getTwoSidedPValue (:1543-1576) from counts instead of a sorted copy
-        const uint64_t idx0 = n_lt[a];                                        // lower_bound of val in the sorted samples
-        const bool first_is_eq = n_eq[a] > 0;                                 // sorted[idx0] == val
-        uint64_t idx = idx0;
-        if (idx0 == l) idx = 1;
-        else if (obs_eff[a] > exp_) {
-            if (first_is_eq && idx0 > 0) idx = idx0 - 1;
-            idx = l - (idx + 1);
-        } else {
-            if (first_is_eq) idx = idx0 + n_eq[a];
-        }
-        const double pv = std::max(1.0 / (double)l, (double)idx / (double)l);
         if (expected) expected[a] = exp_;
         if (stddev) stddev[a] = std::sqrt(sumsq[a] / (double)l);             // numpy.std ddof 0 (:1684)
         if (lower95) lower95[a] = lo;
         if (upper95) upper95[a] = hi;
         if (fold) fold[a] = fo;
-        if (pvalue) pvalue[a] = pv;
+        if (pvalue) pvalue[a] = two_sided_pvalue(l, n_lt[a], n_eq[a], obs_eff[a], exp_);
     }
 }
 
@@ -1586,74 +1577,222 @@ static void ci_ranks(uint64_t l, uint64_t &rank_lo, uint64_t &rank_hi)
     else { rank_lo = 0; rank_hi = l - 1; }
 }
 
-struct StreamStatsOut {
-    std::vector<double> sum, sumsq, qlo, qhi;       // sumsq = sum (x - mean)^2
-    std::vector<unsigned long long> n_lt, n_eq;
-};
-static int stream_stats(gatb_ctx *ctx, const uint32_t *dc, uint64_t l, uint32_t A, const double *obs_eff,
-                        uint64_t rank_lo, uint64_t rank_hi, bool full, StreamStatsOut &o)
+// the context's device and stream for a statistics call, and its input matrix on the device: the caller's own, or a
+// copy of the host one held by `copy`
+static int device_matrix(gatb_ctx *ctx, const void *counts, int is_float, int counts_is_device, uint64_t n,
+                         DevBuf<uint8_t> &copy, const void *&dc)
 {
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    dc = counts;
+    if (counts_is_device) return GATB_OK;
+    CU(ctx, copy.upload((const uint8_t *)counts, n * (is_float ? sizeof(double) : sizeof(uint32_t)), ctx->stream));
+    dc = copy.p;
+    return GATB_OK;
+}
+
+// The exact integers of statistics pass 1 over a uint32 counter plane (gatb_column_stats, gatb_column_pvalue, the column
+// accumulator): every kernel that counts rows ADDS its integers here, so any split of the rows and any choice of kernel
+// gives the same integers, and finish_columns() the same doubles.
+struct ColumnSums {
+    enum { ISUM, N_LT, N_EQ, SQ_LO, SQ_HI, N_INTS };   // sum, #{x < obs_eff}, #{x == obs_eff}, 128-bit sum of squares
+    gatb_ctx *ctx = nullptr;
+    uint32_t A = 0;
+    std::vector<double> obs_eff;
+    std::vector<uint32_t> h_thr;                    // lt_thr | eq_val | flags: obs_eff as integer tests (streamed pass 1)
+    DevBuf<uint32_t> thr;
+    DevBuf<double> d_obs;                           // obs_eff (column-tiled pass 1)
+    DevBuf<unsigned long long> ints;                // [N_INTS][A]: gatb_colacc_state's `moments`
+    DevBuf<uint32_t> mm;                            // min | max [2][A], then vmax, error (a TMA copy did not complete)
+    std::vector<unsigned long long> h_ints;         // host copies (fetch)
+    std::vector<uint32_t> h_mm;
+    uint64_t rows = 0;                              // rows counted so far
+    bool streamed = false;                          // the last add took the streamed pass (and vmax is the matrix maximum)
+    unsigned long long *dev(int k) { return ints.p + (size_t)k * A; }
+    const unsigned long long *host(int k) const { return h_ints.data() + (size_t)k * A; }
+    uint32_t *error() { return mm.p + 2 * (size_t)A + 1; }
+    uint32_t vmax() const { return h_mm[2 * (size_t)A]; }
+    int init(gatb_ctx *c, uint32_t n_cols, const double *observed, const double *ref_fold)
+    {
+        ctx = c; A = n_cols;
+        if (const int rc = effective_observed(ctx, A, observed, ref_fold, obs_eff)) return rc;
+        cudaStream_t st = ctx->stream;
+        h_thr.resize(3 * (size_t)A);
+        stats_stream_thresholds(obs_eff.data(), A, h_thr.data(), h_thr.data() + A, h_thr.data() + 2 * (size_t)A);
+        h_mm.assign(2 * (size_t)A + 2, 0u);
+        std::fill(h_mm.begin(), h_mm.begin() + A, 0xffffffffu);
+        CU(ctx, thr.upload(h_thr.data(), h_thr.size(), st));
+        CU(ctx, d_obs.upload(obs_eff.data(), A, st));
+        CU(ctx, ints.alloc(N_INTS * (size_t)A));
+        CU(ctx, cudaMemsetAsync(ints.p, 0, N_INTS * (size_t)A * sizeof(unsigned long long), st));
+        CU(ctx, mm.upload(h_mm.data(), h_mm.size(), st));
+        return GATB_OK;
+    }
+    // counts the first A values of n_rows rows, row_stride apart, into the sums (`extremes`: into min | max as well).
+    // The TMA-streamed pass of stats_stream.cu unless GATB_STATS_STREAM=0 or the rows are strided, wider than a ring
+    // stage or not 4-byte aligned; then the column-tiled pass of count.cu
+    int add(const uint32_t *counts, uint64_t n_rows, uint64_t row_stride, bool extremes)
+    {
+        cudaStream_t st = ctx->stream;
+        streamed = row_stride == A && ctx->stats_stream && stats_stream_fits(counts, n_rows, A, ctx->smem_optin);
+        if (streamed) {
+            StreamStatsParams p;
+            memset(&p, 0, sizeof(p));
+            p.counts = counts; p.n_samples = n_rows; p.n_cols = A;
+            stats_stream_geometry(p);
+            p.lt_thr = thr.p; p.eq_val = thr.p + A; p.col_flags = thr.p + 2 * (size_t)A;
+            p.isum = dev(ISUM); p.n_lt = dev(N_LT); p.n_eq = dev(N_EQ); p.sq_lo = dev(SQ_LO); p.sq_hi = dev(SQ_HI);
+            if (extremes) { p.col_min = mm.p; p.col_max = mm.p + A; }
+            p.vmax = mm.p + 2 * (size_t)A; p.error = error();
+            ProfScope ps(ctx, PROF_OTHER);
+            CU(ctx, launch_stats_stream_pass1(st, p, ctx->sm_count));
+        } else {
+            StatsParams p;
+            memset(&p, 0, sizeof(p));
+            p.counts = counts; p.n_samples = n_rows; p.n_cols = A; p.row_stride = row_stride; p.observed = d_obs.p;
+            p.isum = dev(ISUM); p.n_lt = dev(N_LT); p.n_eq = dev(N_EQ); p.sq_lo = dev(SQ_LO); p.sq_hi = dev(SQ_HI);
+            if (extremes) { p.col_min = mm.p; p.col_max = mm.p + A; }
+            ProfScope ps(ctx, PROF_OTHER);
+            launch_stats_pass1(st, p);
+            CU(ctx, cudaGetLastError());
+        }
+        rows += n_rows;
+        return GATB_OK;
+    }
+    // the integers and min | max | vmax to h_ints / h_mm, with the stream drained
+    int fetch()
+    {
+        cudaStream_t st = ctx->stream;
+        h_ints.resize(N_INTS * (size_t)A);
+        CU(ctx, cudaMemcpyAsync(h_ints.data(), ints.p, h_ints.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(h_mm.data(), mm.p, h_mm.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        if (h_mm[2 * (size_t)A + 1]) return fail(ctx, GATB_ERR_CUDA, "column statistics: a TMA copy did not complete");
+        return GATB_OK;
+    }
+    // once the sums hold all l samples of every column: mean = sum / l and sumsq = sum (x - mean)^2 = (l * sum x^2 -
+    // (sum x)^2) / l with the numerator exact in 128 bits (x < 2^32, l < 2^32: both products stay below 2^128), rounded
+    // once when it becomes a double; host(N_LT), host(N_EQ) and vmax() hold the rest
+    int read(uint64_t l, std::vector<double> &mean, std::vector<double> &sumsq)
+    {
+        if (const int rc = fetch()) return rc;
+        mean.resize(A); sumsq.resize(A);
+        for (uint32_t a = 0; a < A; a++) {
+            const unsigned long long sum = host(ISUM)[a];
+            const unsigned __int128 sq = ((unsigned __int128)host(SQ_HI)[a] << 64) | host(SQ_LO)[a];
+            mean[a] = (double)sum / (double)l;                              // numpy.mean (:1671)
+            sumsq[a] = (double)((unsigned __int128)l * sq - (unsigned __int128)sum * sum) / (double)l;
+        }
+        return GATB_OK;
+    }
+    // adds another state (gatb_colacc_state layout; either part may be NULL) into this one: the sums of its n_rows rows
+    // with the carry into the high word of the sum of squares, the extremes folded
+    int merge(uint64_t n_rows, const uint64_t *ints_in, const uint32_t *minmax)
+    {
+        if (const int rc = fetch()) return rc;
+        cudaStream_t st = ctx->stream;
+        const size_t n = A;
+        if (ints_in) {
+            for (size_t a = 0; a < n; a++) {
+                unsigned long long *m = h_ints.data() + a;
+                const uint64_t *o = ints_in + a;
+                const unsigned __int128 z = (((unsigned __int128)m[SQ_HI * n] << 64) | m[SQ_LO * n]) +
+                                            (((unsigned __int128)o[SQ_HI * n] << 64) | o[SQ_LO * n]);
+                m[SQ_LO * n] = (uint64_t)z; m[SQ_HI * n] = (uint64_t)(z >> 64);
+                for (const size_t k : {ISUM, N_LT, N_EQ}) m[k * n] += o[k * n];
+            }
+            CU(ctx, cudaMemcpyAsync(ints.p, h_ints.data(), h_ints.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
+            rows += n_rows;
+        }
+        if (minmax) {
+            for (size_t a = 0; a < n; a++) { h_mm[a] = std::min(h_mm[a], minmax[a]); h_mm[n + a] = std::max(h_mm[n + a], minmax[n + a]); }
+            CU(ctx, cudaMemcpyAsync(mm.p, h_mm.data(), 2 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        }
+        return GATB_OK;
+    }
+};
+
+// q = the values at ranks[0] | ranks[1] of every column of the uint32 matrix [l][A] that `sums` has counted: the streamed
+// radix select (4 bits per pass from the top nibble of the matrix maximum) where pass 1 was streamed, else the tiled one
+static int order_stats_u32(ColumnSums &sums, const uint32_t *dc, uint64_t l, const uint64_t *ranks, std::vector<double> &q)
+{
+    gatb_ctx *ctx = sums.ctx;
+    const uint32_t A = sums.A;
     cudaStream_t st = ctx->stream;
     DevBuf<double> d_q;
-    DevBuf<uint32_t> d_thr;                         // lt_thr | eq_val | flags
-    DevBuf<unsigned long long> d_acc, d_rank;       // isum | n_lt | n_eq | sq_lo | sq_hi ; rank | rank_out
-    DevBuf<uint32_t> d_small, d_prefix, d_hist;     // vmax, error ; prefix | prefix_out
-    std::vector<uint32_t> h_thr(3 * (size_t)A);
-    stats_stream_thresholds(obs_eff, A, h_thr.data(), h_thr.data() + A, h_thr.data() + 2 * (size_t)A);
-    CU(ctx, d_thr.upload(h_thr.data(), h_thr.size(), st));
-    CU(ctx, d_acc.alloc(5 * (size_t)A));
-    CU(ctx, d_small.alloc(2));
-    CU(ctx, cudaMemsetAsync(d_acc.p, 0, 5 * (size_t)A * sizeof(unsigned long long), st));
-    CU(ctx, cudaMemsetAsync(d_small.p, 0, 2 * sizeof(uint32_t), st));
-    StreamStatsParams p;
-    memset(&p, 0, sizeof(p));
-    p.counts = dc; p.n_samples = l; p.n_cols = A;
-    stats_stream_geometry(p);
-    p.lt_thr = d_thr.p; p.eq_val = d_thr.p + A; p.col_flags = d_thr.p + 2 * (size_t)A; p.isum = d_acc.p; p.n_lt = d_acc.p + A; p.n_eq = d_acc.p + 2 * (size_t)A;
-    p.sq_lo = d_acc.p + 3 * (size_t)A; p.sq_hi = d_acc.p + 4 * (size_t)A;
-    p.vmax = d_small.p; p.error = d_small.p + 1;
-    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_stats_stream_pass1(st, p, ctx->sm_count)); }
-    std::vector<unsigned long long> h_acc(5 * (size_t)A);
-    uint32_t h_small[2] = {0, 0};
-    CU(ctx, cudaMemcpyAsync(h_acc.data(), d_acc.p, h_acc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CU(ctx, cudaMemcpyAsync(h_small, d_small.p, sizeof(h_small), cudaMemcpyDeviceToHost, st));
-    CU(ctx, cudaStreamSynchronize(st));
-    if (h_small[1]) return fail(ctx, GATB_ERR_CUDA, "column statistics: a TMA copy did not complete");
-    o.sum.resize(A); o.sumsq.resize(A);
-    o.n_lt.assign(h_acc.begin() + A, h_acc.begin() + 2 * (size_t)A);
-    o.n_eq.assign(h_acc.begin() + 2 * (size_t)A, h_acc.begin() + 3 * (size_t)A);
-    for (uint32_t a = 0; a < A; a++) {
-        o.sum[a] = (double)h_acc[a];
-        o.sumsq[a] = exact_sumsq_dev(l, h_acc[a], h_acc[3 * (size_t)A + a], h_acc[4 * (size_t)A + a]);
-    }
-    if (!full) return GATB_OK;
-
-    // radix select, 4 bits per pass, from the highest non-zero nibble of the largest value
-    std::vector<unsigned long long> h_rank(2 * (size_t)A);
-    for (uint32_t a = 0; a < A; a++) { h_rank[a] = rank_lo; h_rank[A + a] = rank_hi; }
-    CU(ctx, d_rank.alloc(4 * (size_t)A));
-    CU(ctx, cudaMemcpyAsync(d_rank.p, h_rank.data(), h_rank.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
-    CU(ctx, d_prefix.alloc(4 * (size_t)A));
-    CU(ctx, cudaMemsetAsync(d_prefix.p, 0, 4 * (size_t)A * sizeof(uint32_t), st));
-    CU(ctx, d_hist.alloc(32 * (size_t)A));
-    CU(ctx, cudaMemsetAsync(d_hist.p, 0, 32 * (size_t)A * sizeof(uint32_t), st));
     CU(ctx, d_q.alloc(2 * (size_t)A));
-    p.prefix = d_prefix.p; p.prefix_out = d_prefix.p + 2 * (size_t)A;
-    p.rank = d_rank.p; p.rank_out = d_rank.p + 2 * (size_t)A;
-    p.hist = d_hist.p; p.q_lo = d_q.p; p.q_hi = d_q.p + A;
-    int top = 0;
-    while (top < 28 && (h_small[0] >> (top + 4)) != 0u) top += 4;
-    for (int shift = top; shift >= 0; shift -= 4) {
-        p.shift = (uint32_t)shift;
-        ProfScope ps(ctx, PROF_OTHER);
-        CU(ctx, launch_stats_stream_select(st, p, ctx->sm_count, ctx->smem_optin));
+    DevBuf<unsigned long long> d_rank;              // rank | rank_out
+    DevBuf<uint32_t> d_prefix, d_hist;              // prefix | prefix_out
+    std::vector<unsigned long long> h_rank(4 * (size_t)A, ranks[1]);
+    if (sums.streamed) {
+        std::fill_n(h_rank.begin(), A, ranks[0]);
+        CU(ctx, d_rank.upload(h_rank.data(), h_rank.size(), st));
+        CU(ctx, d_prefix.alloc(4 * (size_t)A));
+        CU(ctx, cudaMemsetAsync(d_prefix.p, 0, 4 * (size_t)A * sizeof(uint32_t), st));
+        CU(ctx, d_hist.alloc(32 * (size_t)A));
+        CU(ctx, cudaMemsetAsync(d_hist.p, 0, 32 * (size_t)A * sizeof(uint32_t), st));
+        StreamStatsParams p;
+        memset(&p, 0, sizeof(p));
+        p.counts = dc; p.n_samples = l; p.n_cols = A;
+        stats_stream_geometry(p);
+        p.prefix = d_prefix.p; p.prefix_out = d_prefix.p + 2 * (size_t)A;
+        p.rank = d_rank.p; p.rank_out = d_rank.p + 2 * (size_t)A;
+        p.hist = d_hist.p; p.q_lo = d_q.p; p.q_hi = d_q.p + A; p.error = sums.error();
+        int top = 0;
+        while (top < 28 && (sums.vmax() >> (top + 4)) != 0u) top += 4;
+        for (int shift = top; shift >= 0; shift -= 4) {
+            p.shift = (uint32_t)shift;
+            ProfScope ps(ctx, PROF_OTHER);
+            CU(ctx, launch_stats_stream_select(st, p, ctx->sm_count, ctx->smem_optin));
+        }
+    } else {
+        StatsParams p;
+        memset(&p, 0, sizeof(p));
+        p.counts = dc; p.n_samples = l; p.n_cols = A;
+        p.q_lo = d_q.p; p.q_hi = d_q.p + A; p.rank_lo = ranks[0]; p.rank_hi = ranks[1];
+        { ProfScope ps(ctx, PROF_OTHER); launch_stats_select(st, p); }
+        CU(ctx, cudaGetLastError());
     }
-    o.qlo.resize(A); o.qhi.resize(A);
-    CU(ctx, cudaMemcpyAsync(o.qlo.data(), d_q.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(ctx, cudaMemcpyAsync(o.qhi.data(), d_q.p + A, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(ctx, cudaMemcpyAsync(h_small, d_small.p, sizeof(h_small), cudaMemcpyDeviceToHost, st));
+    q.resize(2 * (size_t)A);
+    CU(ctx, cudaMemcpyAsync(q.data(), d_q.p, q.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    return sums.fetch();                            // (synchronises; fails if a copy of a select pass did not complete)
+}
+
+// float64 matrices (nucleotide-density, gat-compare) keep the column-tiled kernels of count.cu.  Pass 1: cnt = n_lt |
+// n_eq against obs and the column means; with `ranks`, pass 2 for sum (x - mean)^2 and the 8-bit radix select for
+// q = the values at ranks[0] | ranks[1]
+static int float_stats(gatb_ctx *ctx, const double *dc, uint64_t l, uint32_t A, const double *obs, const uint64_t *ranks,
+                       std::vector<unsigned long long> &cnt, std::vector<double> &mean, std::vector<double> &sumsq,
+                       std::vector<double> &q)
+{
+    cudaStream_t st = ctx->stream;
+    DevBuf<double> d_obs, d_sum, d_mean, d_sq, d_q;
+    DevBuf<unsigned long long> d_cnt;
+    CU(ctx, d_obs.upload(obs, A, st));
+    CU(ctx, d_sum.alloc(A));
+    CU(ctx, d_cnt.alloc(2 * (size_t)A));
+    StatsParams p;
+    memset(&p, 0, sizeof(p));
+    p.counts = dc; p.is_float = 1; p.n_samples = l; p.n_cols = A; p.observed = d_obs.p;
+    p.sum = d_sum.p; p.n_lt = d_cnt.p; p.n_eq = d_cnt.p + A;
+    { ProfScope ps(ctx, PROF_OTHER); launch_stats_pass1(st, p); }
+    CU(ctx, cudaGetLastError());
+    cnt.resize(2 * (size_t)A); mean.resize(A);
+    CU(ctx, cudaMemcpyAsync(cnt.data(), d_cnt.p, cnt.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaMemcpyAsync(mean.data(), d_sum.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaStreamSynchronize(st));
-    if (h_small[1]) return fail(ctx, GATB_ERR_CUDA, "column statistics: a TMA copy did not complete");
+    for (uint32_t a = 0; a < A; a++) mean[a] /= (double)l;                  // numpy.mean (:1671)
+    if (!ranks) return GATB_OK;
+    CU(ctx, d_mean.upload(mean.data(), A, st));
+    CU(ctx, d_sq.alloc(A)); CU(ctx, d_q.alloc(2 * (size_t)A));
+    p.mean = d_mean.p; p.sumsq_dev = d_sq.p; p.q_lo = d_q.p; p.q_hi = d_q.p + A; p.rank_lo = ranks[0]; p.rank_hi = ranks[1];
+    { ProfScope ps(ctx, PROF_OTHER); launch_stats_pass2(st, p); }
+    { ProfScope ps(ctx, PROF_OTHER); launch_stats_select(st, p); }
+    CU(ctx, cudaGetLastError());
+    sumsq.resize(A); q.resize(2 * (size_t)A);
+    CU(ctx, cudaMemcpyAsync(sumsq.data(), d_sq.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaMemcpyAsync(q.data(), d_q.p, q.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
     return GATB_OK;
 }
 
@@ -1664,76 +1803,32 @@ extern "C" int gatb_column_stats(gatb_ctx *ctx, const void *counts, int is_float
 {
     if (!ctx || !counts || !observed || n_cols <= 0) return GATB_ERR_INVALID;
     if (n_samples < 1) return fail(ctx, GATB_ERR_INVALID, "column_stats: no samples");
-    CU(ctx, cudaSetDevice(ctx->device));
-    tl_stream = ctx->stream;
-    cudaStream_t st = ctx->stream;
     const uint32_t A = (uint32_t)n_cols;
     const uint64_t l = n_samples;
-    const size_t esz = is_float ? sizeof(double) : sizeof(uint32_t);
     DevBuf<uint8_t> d_counts;
-    const void *dc = counts;
-    if (!counts_is_device) {
-        CU(ctx, d_counts.upload((const uint8_t *)counts, l * A * esz, st));
-        dc = d_counts.p;
-    }
-    std::vector<double> obs_eff;
-    if (const int rc = effective_observed(ctx, A, observed, ref_fold, obs_eff)) return rc;
-    uint64_t rank_lo, rank_hi;
-    ci_ranks(l, rank_lo, rank_hi);
-    std::vector<double> h_sum(A), h_sq(A), h_qlo(A), h_qhi(A), h_mean(A);
-    std::vector<unsigned long long> h_cnt(2 * (size_t)A);
-    if (!is_float && ctx->stats_stream && stats_stream_fits(dc, l, A, ctx->smem_optin)) {
-        // uint32 counts: HBM-bound streaming passes (stats_stream.cu)
-        StreamStatsOut o;
-        const int rc = stream_stats(ctx, (const uint32_t *)dc, l, A, obs_eff.data(), rank_lo, rank_hi, true, o);
-        if (rc != GATB_OK) return rc;
-        for (uint32_t a = 0; a < A; a++) {
-            h_sum[a] = o.sum[a]; h_sq[a] = o.sumsq[a]; h_qlo[a] = o.qlo[a]; h_qhi[a] = o.qhi[a];
-            h_mean[a] = h_sum[a] / (double)l;
-            h_cnt[a] = o.n_lt[a]; h_cnt[A + a] = o.n_eq[a];
-        }
+    const void *dc = nullptr;
+    int rc = device_matrix(ctx, counts, is_float, counts_is_device, l * A, d_counts, dc);
+    if (rc) return rc;
+    uint64_t ranks[2];
+    ci_ranks(l, ranks[0], ranks[1]);
+    ColumnSums sums;
+    std::vector<double> obs_eff, mean, sumsq, q;
+    std::vector<unsigned long long> cnt;            // float64: n_lt | n_eq
+    const unsigned long long *n_lt, *n_eq;
+    if (!is_float) {
+        rc = sums.init(ctx, A, observed, ref_fold);
+        if (!rc) rc = sums.add((const uint32_t *)dc, l, A, false);
+        if (!rc) rc = sums.read(l, mean, sumsq);
+        if (!rc) rc = order_stats_u32(sums, (const uint32_t *)dc, l, ranks, q);
+        obs_eff = sums.obs_eff; n_lt = sums.host(ColumnSums::N_LT); n_eq = sums.host(ColumnSums::N_EQ);
     } else {
-        // float64 matrices (nucleotide-density, gat-compare), very wide or unaligned ones: column-tiled kernels (count.cu)
-        DevBuf<double> d_obs, d_sum, d_sq, d_mean, d_qlo, d_qhi;
-        DevBuf<unsigned long long> d_cnt;               // n_lt | n_eq | sq_lo | sq_hi | isum
-        CU(ctx, d_obs.upload(obs_eff.data(), A, st));
-        CU(ctx, d_sum.alloc(A)); CU(ctx, d_sq.alloc(A)); CU(ctx, d_qlo.alloc(A)); CU(ctx, d_qhi.alloc(A));
-        CU(ctx, d_cnt.alloc(5 * (size_t)A));
-        StatsParams p;
-        memset(&p, 0, sizeof(p));
-        p.counts = dc; p.is_float = is_float; p.n_samples = l; p.n_cols = A; p.observed = d_obs.p;
-        p.sum = d_sum.p; p.sumsq_dev = d_sq.p; p.n_lt = d_cnt.p; p.n_eq = d_cnt.p + A;
-        if (!is_float) { p.sq_lo = d_cnt.p + 2 * (size_t)A; p.sq_hi = d_cnt.p + 3 * (size_t)A; p.isum = d_cnt.p + 4 * (size_t)A; }
-        p.q_lo = d_qlo.p; p.q_hi = d_qhi.p;
-        p.rank_lo = rank_lo; p.rank_hi = rank_hi;
-        { ProfScope ps(ctx, PROF_OTHER); launch_stats_pass1(st, p); }
-        CU(ctx, cudaGetLastError());
-        CU(ctx, cudaMemcpyAsync(h_sum.data(), d_sum.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaStreamSynchronize(st));
-        for (uint32_t a = 0; a < A; a++) h_mean[a] = h_sum[a] / (double)l;        // numpy.mean (:1671)
-        CU(ctx, d_mean.upload(h_mean.data(), A, st));
-        p.mean = d_mean.p;
-        // float64 matrices: second pass for sum (x - mean)^2; uint32 matrices: the exact integer formula of the streamed
-        // passes, so that a column's statistics do not depend on which of the two kernels its matrix was given to
-        std::vector<unsigned long long> h_sqi;
-        if (is_float) { ProfScope ps(ctx, PROF_OTHER); launch_stats_pass2(st, p); }
-        else {
-            h_sqi.resize(3 * (size_t)A);
-            CU(ctx, cudaMemcpyAsync(h_sqi.data(), d_cnt.p + 2 * (size_t)A, h_sqi.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        }
-        { ProfScope ps(ctx, PROF_OTHER); launch_stats_select(st, p); }
-        CU(ctx, cudaGetLastError());
-        if (is_float) CU(ctx, cudaMemcpyAsync(h_sq.data(), d_sq.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaMemcpyAsync(h_qlo.data(), d_qlo.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaMemcpyAsync(h_qhi.data(), d_qhi.p, A * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaMemcpyAsync(h_cnt.data(), d_cnt.p, 2 * (size_t)A * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaStreamSynchronize(st));
-        if (!is_float)
-            for (uint32_t a = 0; a < A; a++) h_sq[a] = exact_sumsq_dev(l, h_sqi[2 * (size_t)A + a], h_sqi[a], h_sqi[A + a]);
+        rc = effective_observed(ctx, A, observed, ref_fold, obs_eff);
+        if (!rc) rc = float_stats(ctx, (const double *)dc, l, A, obs_eff.data(), ranks, cnt, mean, sumsq, q);
+        n_lt = cnt.data(); n_eq = cnt.data() + A;
     }
-
-    finish_columns(l, A, observed, obs_eff.data(), ref_fold, pseudo_count, h_mean.data(), h_sq.data(), h_qlo.data(),
-                   h_qhi.data(), h_cnt.data(), h_cnt.data() + A, expected, stddev, lower95, upper95, fold, pvalue);
+    if (rc) return rc;
+    finish_columns(l, A, observed, obs_eff.data(), ref_fold, pseudo_count, mean.data(), sumsq.data(), q.data(), q.data() + A,
+                   n_lt, n_eq, expected, stddev, lower95, upper95, fold, pvalue);
     return GATB_OK;
 }
 
@@ -1747,85 +1842,48 @@ extern "C" int gatb_column_pvalue(gatb_ctx *ctx, const void *counts, int is_floa
 {
     if (!ctx || !counts || !values || !expected || !pvalue || n_cols <= 0) return GATB_ERR_INVALID;
     if (n_samples < 1) return fail(ctx, GATB_ERR_INVALID, "column_pvalue: no samples");
-    CU(ctx, cudaSetDevice(ctx->device));
-    tl_stream = ctx->stream;
-    cudaStream_t st = ctx->stream;
     const uint32_t A = (uint32_t)n_cols;
     const uint64_t l = n_samples;
-    const size_t esz = is_float ? sizeof(double) : sizeof(uint32_t);
     DevBuf<uint8_t> d_counts;
-    const void *dc = counts;
-    if (!counts_is_device) {
-        CU(ctx, d_counts.upload((const uint8_t *)counts, l * A * esz, st));
-        dc = d_counts.p;
-    }
-    std::vector<unsigned long long> h_cnt(2 * (size_t)A);
-    if (!is_float && ctx->stats_stream && stats_stream_fits(dc, l, A, ctx->smem_optin)) {
-        StreamStatsOut o;
-        const int rc = stream_stats(ctx, (const uint32_t *)dc, l, A, values, 0, 0, false, o);
-        if (rc != GATB_OK) return rc;
-        for (uint32_t a = 0; a < A; a++) { h_cnt[a] = o.n_lt[a]; h_cnt[A + a] = o.n_eq[a]; }
+    const void *dc = nullptr;
+    int rc = device_matrix(ctx, counts, is_float, counts_is_device, l * A, d_counts, dc);
+    if (rc) return rc;
+    ColumnSums sums;
+    std::vector<double> mean, sumsq, unused;
+    std::vector<unsigned long long> cnt;            // float64: n_lt | n_eq
+    const unsigned long long *n_lt, *n_eq;
+    if (!is_float) {
+        rc = sums.init(ctx, A, values, nullptr);
+        if (!rc) rc = sums.add((const uint32_t *)dc, l, A, false);
+        if (!rc) rc = sums.read(l, mean, sumsq);
+        n_lt = sums.host(ColumnSums::N_LT); n_eq = sums.host(ColumnSums::N_EQ);
     } else {
-        DevBuf<double> d_obs, d_sum;
-        DevBuf<unsigned long long> d_cnt;
-        CU(ctx, d_obs.upload(values, A, st));
-        CU(ctx, d_sum.alloc(A));
-        CU(ctx, d_cnt.alloc(2 * (size_t)A));
-        StatsParams p;
-        memset(&p, 0, sizeof(p));
-        p.counts = dc; p.is_float = is_float; p.n_samples = l; p.n_cols = A; p.observed = d_obs.p;
-        p.sum = d_sum.p; p.n_lt = d_cnt.p; p.n_eq = d_cnt.p + A;
-        { ProfScope ps(ctx, PROF_OTHER); launch_stats_pass1(st, p); }
-        CU(ctx, cudaGetLastError());
-        CU(ctx, cudaMemcpyAsync(h_cnt.data(), d_cnt.p, 2 * (size_t)A * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaStreamSynchronize(st));
+        rc = float_stats(ctx, (const double *)dc, l, A, values, nullptr, cnt, mean, unused, unused);
+        n_lt = cnt.data(); n_eq = cnt.data() + A;
     }
-    for (uint32_t a = 0; a < A; a++) {
-        const uint64_t n_lt = h_cnt[a], n_eq = h_cnt[A + a];
-        uint64_t idx = n_lt;
-        if (n_lt == l) idx = 1;
-        else if (values[a] > expected[a]) {
-            if (n_eq > 0 && n_lt > 0) idx = n_lt - 1;
-            idx = l - (idx + 1);
-        } else if (n_eq > 0) idx = n_lt + n_eq;
-        pvalue[a] = std::max(1.0 / (double)l, (double)idx / (double)l);
-    }
+    if (rc) return rc;
+    for (uint32_t a = 0; a < A; a++) pvalue[a] = two_sided_pvalue(l, n_lt[a], n_eq[a], values[a], expected[a]);
     return GATB_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------
 // column statistics without the sample matrix: an accumulator of one uint32 counter plane, fed slab by slab.
-// Pass 1 of the streamed statistics ADDS its exact integers (sum, 128-bit sum of squares, #{x < obs}, #{x == obs},
-// extremes) into the accumulator's own arrays, so any split of the rows into slabs gives the integers of one pass
-// over the whole matrix; the two order statistics come from per-column windows of unit-width bins (exact values,
-// so exact ranks).  gatb_colacc_finish turns the integers into doubles with the same finish_columns() as
-// gatb_column_stats: same integers, same doubles.
+// Pass 1 of the statistics ADDS its exact integers into the accumulator's ColumnSums, so any split of the rows into
+// slabs gives the integers of one pass over the whole matrix; the two order statistics come from per-column windows
+// of unit-width bins (exact values, so exact ranks).  gatb_colacc_finish turns the integers into doubles with the
+// same finish_columns() as gatb_column_stats: same integers, same doubles.
 struct gatb_colacc {
     gatb_ctx *ctx = nullptr;
     uint32_t A = 0;
-    uint64_t l = 0, rows = 0;                       // samples of the whole column / rows counted into the sums so far
-    uint64_t rank_lo = 0, rank_hi = 0;
-    std::vector<double> observed, ref, obs_eff;
-    std::vector<uint32_t> lo, width;
+    uint64_t l = 0;                                 // samples of the whole column
+    std::vector<double> observed, ref;
+    ColumnSums sums;
     uint64_t n_bins = 0;
-    DevBuf<uint32_t> thr;                           // lt_thr | eq_val | flags (stream pass 1)
-    DevBuf<double> d_obs;                           // obs_eff (column-tiled pass 1)
-    DevBuf<unsigned long long> acc;                 // isum | n_lt | n_eq | sq_lo | sq_hi | below | above   [7][A]
-    DevBuf<uint32_t> mm;                            // min | max [2][A], then vmax, error
+    DevBuf<unsigned long long> outside;             // below | above [2][A]
     DevBuf<uint32_t> win;                           // lo | width [2][A]
     DevBuf<unsigned long long> bin_off;             // [A]
     DevBuf<uint32_t> bins;                          // [n_bins]
 };
-
-static int colacc_error_check(gatb_colacc *c)
-{
-    gatb_ctx *ctx = c->ctx;
-    uint32_t err = 0;
-    CU(ctx, cudaMemcpyAsync(&err, c->mm.p + 2 * (size_t)c->A + 1, sizeof(err), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    if (err) return fail(ctx, GATB_ERR_CUDA, "column accumulator: a TMA copy did not complete");
-    return GATB_OK;
-}
 
 extern "C" int gatb_colacc_create(gatb_ctx *ctx, int n_cols, uint64_t n_samples_total, const double *observed,
                                   const double *ref_fold, gatb_colacc **out)
@@ -1837,31 +1895,19 @@ extern "C" int gatb_colacc_create(gatb_ctx *ctx, int n_cols, uint64_t n_samples_
     CU(ctx, cudaSetDevice(ctx->device));
     tl_stream = ctx->stream;
     cudaStream_t st = ctx->stream;
-    gatb_colacc *c = new gatb_colacc();
+    std::unique_ptr<gatb_colacc> c(new gatb_colacc());
     c->ctx = ctx; c->A = (uint32_t)n_cols; c->l = n_samples_total;
     const uint32_t A = c->A;
     c->observed.assign(observed, observed + A);
     if (ref_fold) c->ref.assign(ref_fold, ref_fold + A);
-    int rc = effective_observed(ctx, A, observed, ref_fold, c->obs_eff);
-    if (rc) { delete c; return rc; }
-    ci_ranks(c->l, c->rank_lo, c->rank_hi);
-    std::vector<uint32_t> h_thr(3 * (size_t)A);
-    stats_stream_thresholds(c->obs_eff.data(), A, h_thr.data(), h_thr.data() + A, h_thr.data() + 2 * (size_t)A);
-    std::vector<uint32_t> h_mm(2 * (size_t)A + 2, 0u);
-    std::fill(h_mm.begin(), h_mm.begin() + A, 0xffffffffu);
-    c->lo.assign(A, 0u); c->width.assign(A, 0u);
-    std::vector<uint32_t> h_win(2 * (size_t)A, 0u);
-    std::vector<unsigned long long> h_off(A, 0ull);
-    cudaError_t e = c->thr.upload(h_thr.data(), h_thr.size(), st);
-    if (e == cudaSuccess) e = c->d_obs.upload(c->obs_eff.data(), A, st);
-    if (e == cudaSuccess) e = c->acc.alloc(7 * (size_t)A);
-    if (e == cudaSuccess) e = cudaMemsetAsync(c->acc.p, 0, 7 * (size_t)A * sizeof(unsigned long long), st);
-    if (e == cudaSuccess) e = c->mm.upload(h_mm.data(), h_mm.size(), st);
-    if (e == cudaSuccess) e = c->win.upload(h_win.data(), h_win.size(), st);
-    if (e == cudaSuccess) e = c->bin_off.upload(h_off.data(), A, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);          // (the host vectors above go out of scope)
-    if (e != cudaSuccess) { delete c; return fail(ctx, GATB_ERR_CUDA, std::string("colacc_create: ") + cudaGetErrorString(e)); }
-    *out = c;
+    if (const int rc = c->sums.init(ctx, A, observed, ref_fold)) return rc;
+    CU(ctx, c->outside.alloc(2 * (size_t)A));
+    CU(ctx, cudaMemsetAsync(c->outside.p, 0, 2 * (size_t)A * sizeof(unsigned long long), st));
+    CU(ctx, c->win.alloc(2 * (size_t)A));
+    CU(ctx, cudaMemsetAsync(c->win.p, 0, 2 * (size_t)A * sizeof(uint32_t), st));
+    CU(ctx, c->bin_off.alloc(A));
+    CU(ctx, cudaMemsetAsync(c->bin_off.p, 0, A * sizeof(unsigned long long), st));
+    *out = c.release();
     return GATB_OK;
 }
 
@@ -1880,15 +1926,12 @@ extern "C" int gatb_colacc_set_windows(gatb_colacc *c, const uint32_t *lo, const
         h_off[a] = n;
         n += width[a];
     }
-    c->lo.assign(lo, lo + A); c->width.assign(width, width + A);
-    std::vector<uint32_t> h_win(2 * (size_t)A);
-    std::copy(lo, lo + A, h_win.begin());
-    std::copy(width, width + A, h_win.begin() + A);
     CU(ctx, c->bins.alloc(std::max<uint64_t>(n, 1)));
     c->n_bins = n;
     CU(ctx, cudaMemsetAsync(c->bins.p, 0, std::max<uint64_t>(n, 1) * sizeof(uint32_t), st));
-    CU(ctx, cudaMemsetAsync(c->acc.p + 5 * (size_t)A, 0, 2 * (size_t)A * sizeof(unsigned long long), st));
-    CU(ctx, cudaMemcpyAsync(c->win.p, h_win.data(), h_win.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(ctx, cudaMemsetAsync(c->outside.p, 0, 2 * (size_t)A * sizeof(unsigned long long), st));
+    CU(ctx, cudaMemcpyAsync(c->win.p, lo, A * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(ctx, cudaMemcpyAsync(c->win.p + A, width, A * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     CU(ctx, cudaMemcpyAsync(c->bin_off.p, h_off.data(), A * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
     CU(ctx, cudaStreamSynchronize(st));
     return GATB_OK;
@@ -1902,45 +1945,19 @@ extern "C" int gatb_colacc_add(gatb_colacc *c, const uint32_t *counts, uint64_t 
     if (what & ~(GATB_COLACC_SUMS | GATB_COLACC_HIST)) return fail(ctx, GATB_ERR_INVALID, "colacc_add: unknown flags");
     if (n_rows == 0) return GATB_OK;
     if (!counts || row_stride < A) return fail(ctx, GATB_ERR_INVALID, "colacc_add: no slab or row_stride < n_cols");
-    if ((what & GATB_COLACC_SUMS) && c->rows + n_rows > c->l)
+    if ((what & GATB_COLACC_SUMS) && c->sums.rows + n_rows > c->l)
         return fail(ctx, GATB_ERR_INVALID, "colacc_add: more rows than n_samples_total");
     CU(ctx, cudaSetDevice(ctx->device));
     tl_stream = ctx->stream;
-    cudaStream_t st = ctx->stream;
-    unsigned long long *acc = c->acc.p;
-    if (what & GATB_COLACC_SUMS) {
-        if (ctx->stats_stream && row_stride == A && stats_stream_fits(counts, n_rows, A, ctx->smem_optin)) {
-            StreamStatsParams p;
-            memset(&p, 0, sizeof(p));
-            p.counts = counts; p.n_samples = n_rows; p.n_cols = A;
-            stats_stream_geometry(p);
-            p.lt_thr = c->thr.p; p.eq_val = c->thr.p + A; p.col_flags = c->thr.p + 2 * (size_t)A;
-            p.isum = acc; p.n_lt = acc + A; p.n_eq = acc + 2 * (size_t)A; p.sq_lo = acc + 3 * (size_t)A; p.sq_hi = acc + 4 * (size_t)A;
-            p.col_min = c->mm.p; p.col_max = c->mm.p + A;
-            p.vmax = c->mm.p + 2 * (size_t)A; p.error = c->mm.p + 2 * (size_t)A + 1;
-            ProfScope ps(ctx, PROF_OTHER);
-            CU(ctx, launch_stats_stream_pass1(st, p, ctx->sm_count));
-        } else {
-            // wider than a ring stage, strided or unaligned slabs: the column-tiled pass 1 (count.cu), accumulating
-            StatsParams p;
-            memset(&p, 0, sizeof(p));
-            p.counts = counts; p.n_samples = n_rows; p.n_cols = A; p.row_stride = row_stride; p.observed = c->d_obs.p;
-            p.accumulate = 1;
-            p.isum = acc; p.n_lt = acc + A; p.n_eq = acc + 2 * (size_t)A; p.sq_lo = acc + 3 * (size_t)A; p.sq_hi = acc + 4 * (size_t)A;
-            p.col_min = c->mm.p; p.col_max = c->mm.p + A;
-            ProfScope ps(ctx, PROF_OTHER);
-            launch_stats_pass1(st, p);
-            CU(ctx, cudaGetLastError());
-        }
-        c->rows += n_rows;
-    }
+    if (what & GATB_COLACC_SUMS)
+        if (const int rc = c->sums.add(counts, n_rows, row_stride, true)) return rc;
     if (what & GATB_COLACC_HIST) {
         ColHistParams h;
         memset(&h, 0, sizeof(h));
         h.counts = counts; h.n_rows = n_rows; h.row_stride = row_stride; h.n_cols = A;
-        h.lo = c->win.p; h.width = c->win.p + A; h.bin_off = c->bin_off.p; h.bins = c->bins.p; h.outside = acc + 5 * (size_t)A;
+        h.lo = c->win.p; h.width = c->win.p + A; h.bin_off = c->bin_off.p; h.bins = c->bins.p; h.outside = c->outside.p;
         ProfScope ps(ctx, PROF_OTHER);
-        CU(ctx, launch_colacc_hist(st, h, ctx->sm_count));
+        CU(ctx, launch_colacc_hist(ctx->stream, h, ctx->sm_count));
     }
     return GATB_OK;
 }
@@ -1953,11 +1970,11 @@ extern "C" int gatb_colacc_state(gatb_colacc *c, uint64_t *rows, uint64_t *momen
     const size_t A = c->A;
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    if (const int rc = colacc_error_check(c)) return rc;
-    if (rows) *rows = c->rows;
-    if (moments) CU(ctx, cudaMemcpyAsync(moments, c->acc.p, 5 * A * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (outside) CU(ctx, cudaMemcpyAsync(outside, c->acc.p + 5 * A, 2 * A * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (minmax) CU(ctx, cudaMemcpyAsync(minmax, c->mm.p, 2 * A * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    if (const int rc = c->sums.fetch()) return rc;
+    if (rows) *rows = c->sums.rows;
+    if (moments) std::copy(c->sums.h_ints.begin(), c->sums.h_ints.end(), moments);
+    if (minmax) std::copy(c->sums.h_mm.begin(), c->sums.h_mm.begin() + 2 * A, minmax);
+    if (outside) CU(ctx, cudaMemcpyAsync(outside, c->outside.p, 2 * A * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     if (bins && c->n_bins) CU(ctx, cudaMemcpyAsync(bins, c->bins.p, c->n_bins * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaStreamSynchronize(st));
     return GATB_OK;
@@ -1969,30 +1986,15 @@ extern "C" int gatb_colacc_merge(gatb_colacc *c, uint64_t rows, const uint64_t *
     if (!c) return GATB_ERR_INVALID;
     gatb_ctx *ctx = c->ctx;
     const size_t A = c->A;
-    if (c->rows + rows > c->l) return fail(ctx, GATB_ERR_INVALID, "colacc_merge: more rows than n_samples_total");
-    std::vector<uint64_t> m(5 * A), o(2 * A);
-    std::vector<uint32_t> mm(2 * A), b(c->n_bins);
-    uint64_t mine = 0;
-    if (const int rc = gatb_colacc_state(c, &mine, m.data(), mm.data(), o.data(), b.data())) return rc;
+    if (c->sums.rows + rows > c->l) return fail(ctx, GATB_ERR_INVALID, "colacc_merge: more rows than n_samples_total");
+    std::vector<uint64_t> o(2 * A);
+    std::vector<uint32_t> b(c->n_bins);
+    if (const int rc = gatb_colacc_state(c, nullptr, nullptr, nullptr, o.data(), b.data())) return rc;
+    if (const int rc = c->sums.merge(rows, moments, minmax)) return rc;
     cudaStream_t st = ctx->stream;
-    if (moments) {
-        for (size_t a = 0; a < A; a++) {
-            const unsigned __int128 x = ((unsigned __int128)m[4 * A + a] << 64) | m[3 * A + a];
-            const unsigned __int128 y = ((unsigned __int128)moments[4 * A + a] << 64) | moments[3 * A + a];
-            const unsigned __int128 z = x + y;
-            m[3 * A + a] = (uint64_t)z; m[4 * A + a] = (uint64_t)(z >> 64);
-            for (int k = 0; k < 3; k++) m[k * A + a] += moments[k * A + a];
-        }
-        CU(ctx, cudaMemcpyAsync(c->acc.p, m.data(), 5 * A * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-        c->rows += rows;
-    }
-    if (minmax) {
-        for (size_t a = 0; a < A; a++) { mm[a] = std::min(mm[a], minmax[a]); mm[A + a] = std::max(mm[A + a], minmax[A + a]); }
-        CU(ctx, cudaMemcpyAsync(c->mm.p, mm.data(), 2 * A * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    }
     if (outside) {
         for (size_t i = 0; i < 2 * A; i++) o[i] += outside[i];
-        CU(ctx, cudaMemcpyAsync(c->acc.p + 5 * A, o.data(), 2 * A * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+        CU(ctx, cudaMemcpyAsync(c->outside.p, o.data(), 2 * A * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     }
     if (bins && c->n_bins) {
         for (uint64_t i = 0; i < c->n_bins; i++) b[i] += bins[i];
@@ -2009,8 +2011,8 @@ extern "C" int gatb_colacc_finish(gatb_colacc *c, double pseudo_count, double *e
     gatb_ctx *ctx = c->ctx;
     const uint32_t A = c->A;
     const uint64_t l = c->l;
-    if (c->rows != l)
-        return fail(ctx, GATB_ERR_INVALID, "colacc_finish: the sums hold " + std::to_string(c->rows) + " of " +
+    if (c->sums.rows != l)
+        return fail(ctx, GATB_ERR_INVALID, "colacc_finish: the sums hold " + std::to_string(c->sums.rows) + " of " +
                                                std::to_string(l) + " samples");
     CU(ctx, cudaSetDevice(ctx->device));
     tl_stream = ctx->stream;
@@ -2022,31 +2024,28 @@ extern "C" int gatb_colacc_finish(gatb_colacc *c, double pseudo_count, double *e
     ColHistParams h;
     memset(&h, 0, sizeof(h));
     h.n_cols = A; h.lo = c->win.p; h.width = c->win.p + A; h.bin_off = c->bin_off.p; h.bins = c->bins.p;
-    h.outside = c->acc.p + 5 * (size_t)A;
-    h.n_samples = l; h.rank_lo = c->rank_lo; h.rank_hi = c->rank_hi;
+    h.outside = c->outside.p;
+    h.n_samples = l; ci_ranks(l, h.rank_lo, h.rank_hi);
     h.q = d_q.p; h.missed = d_q.p + 2 * (size_t)A; h.total = d_total.p;
     { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_pick(st, h)); }
-    std::vector<unsigned long long> m(5 * (size_t)A), total(A);
+    std::vector<unsigned long long> total(A);
     std::vector<uint32_t> q(3 * (size_t)A);
-    CU(ctx, cudaMemcpyAsync(m.data(), c->acc.p, m.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaMemcpyAsync(q.data(), d_q.p, q.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaMemcpyAsync(total.data(), d_total.p, A * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    if (const int rc = colacc_error_check(c)) return rc;
-    std::vector<double> mean(A), sq(A), qlo(A), qhi(A);
+    std::vector<double> mean, sq, qlo(A), qhi(A);
+    if (const int rc = c->sums.read(l, mean, sq)) return rc;       // (synchronises the stream: q and total are here)
     for (uint32_t a = 0; a < A; a++) {
         if (total[a] != l)
             return fail(ctx, GATB_ERR_INVALID, "colacc_finish: the histogram of column " + std::to_string(a) + " holds " +
                                                    std::to_string(total[a]) + " of " + std::to_string(l) + " samples");
-        mean[a] = (double)m[a] / (double)l;
-        sq[a] = exact_sumsq_dev(l, m[a], m[3 * (size_t)A + a], m[4 * (size_t)A + a]);
         const bool miss = q[2 * (size_t)A + a] != 0;
         qlo[a] = miss ? NAN : (double)q[a];
         qhi[a] = miss ? NAN : (double)q[A + a];
         if (missed) missed[a] = miss ? 1 : 0;
     }
-    finish_columns(l, A, c->observed.data(), c->obs_eff.data(), c->ref.empty() ? nullptr : c->ref.data(), pseudo_count,
-                   mean.data(), sq.data(), qlo.data(), qhi.data(), m.data() + A, m.data() + 2 * (size_t)A,
-                   expected, stddev, lower95, upper95, fold, pvalue);
+    finish_columns(l, A, c->observed.data(), c->sums.obs_eff.data(), c->ref.empty() ? nullptr : c->ref.data(), pseudo_count,
+                   mean.data(), sq.data(), qlo.data(), qhi.data(), c->sums.host(ColumnSums::N_LT),
+                   c->sums.host(ColumnSums::N_EQ), expected, stddev, lower95, upper95, fold, pvalue);
     return GATB_OK;
 }
 

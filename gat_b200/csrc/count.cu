@@ -662,17 +662,13 @@ __global__ void __launch_bounds__(STATS_COLS * STATS_ROWS) stats_pass1_kernel(St
             lo += l2; hi += su[4][r][t.c] + ((lo < l2) ? 1ull : 0ull);
             vmin = min(vmin, smm[0][r][t.c]); vmax = max(vmax, smm[1][r][t.c]);
         }
-        if (p.accumulate) {
-            // (the low word's atomic reports its own carry into the high word, whatever the order of the adds)
-            atomicAdd(p.n_lt + t.col, a); atomicAdd(p.n_eq + t.col, b); atomicAdd(p.isum + t.col, c);
-            const unsigned long long old = atomicAdd(p.sq_lo + t.col, lo);
-            atomicAdd(p.sq_hi + t.col, hi + ((old + lo < old) ? 1ull : 0ull));
-            if (p.n_samples) { atomicMin(p.col_min + t.col, vmin); atomicMax(p.col_max + t.col, vmax); }
-            return;
-        }
-        p.n_lt[t.col] = a; p.n_eq[t.col] = b;
-        p.sum[t.col] = p.is_float ? f : (double)c;
-        if (p.sq_lo) { p.sq_lo[t.col] = lo; p.sq_hi[t.col] = hi; p.isum[t.col] = c; }
+        if (p.is_float) { p.n_lt[t.col] = a; p.n_eq[t.col] = b; p.sum[t.col] = f; return; }
+        // uint32: added to the caller's sums (the CTA owns its columns, so these atomics meet no other CTA's; the low
+        // word's atomic reports its own carry into the high word, whatever the order of the adds)
+        atomicAdd(p.n_lt + t.col, a); atomicAdd(p.n_eq + t.col, b); atomicAdd(p.isum + t.col, c);
+        const unsigned long long old = atomicAdd(p.sq_lo + t.col, lo);
+        atomicAdd(p.sq_hi + t.col, hi + ((old + lo < old) ? 1ull : 0ull));
+        if (p.col_min) { atomicMin(p.col_min + t.col, vmin); atomicMax(p.col_max + t.col, vmax); }
     }
 }
 

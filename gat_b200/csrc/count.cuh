@@ -129,7 +129,10 @@ cudaError_t launch_count(cudaStream_t st, int counter, const CountParams &p, int
 // diagnostic: segments and index entries in the runs of the placed segments (bench.py roofline)
 void launch_count_work(cudaStream_t st, const CountParams &p, unsigned long long *out);
 
-// column statistics (K5)
+// column statistics (K5), column-tiled.  Pass 1 of a float64 matrix STORES sum, n_lt and n_eq; pass 1 of a uint32
+// matrix ADDS its exact integers to isum, n_lt, n_eq, sq_lo and sq_hi (zeroed by the caller), so that successive slabs
+// of rows give what one pass over all of them gives, and folds each column's extremes into col_min / col_max when
+// col_min is set
 struct StatsParams {
     const void *counts;             // [n_samples][n_cols] uint32 or float64
     int is_float;
@@ -137,21 +140,17 @@ struct StatsParams {
     uint32_t n_cols;
     const double *observed;         // device [n_cols]; already divided by ref fold where applicable
     // outputs, device [n_cols]
-    double *sum;                    // exact integer sum (as double) or float sum
-    double *sumsq_dev;              // sum (x-mean)^2
+    double *sum;                    // float64: sum (pass 1)
+    double *sumsq_dev;              // float64: sum (x-mean)^2 (pass 2)
     unsigned long long *n_lt;       // #{ x < obs } = insertion point of obs (gat/Engine.pyx:1549-1557)
     unsigned long long *n_eq;       // #{ x == obs }
-    unsigned long long *sq_lo, *sq_hi;   // uint32 matrices: exact sum of squares, 128 bits (the variance follows on the host)
-    unsigned long long *isum;       // uint32 matrices: the exact integer sum
-    double *q_lo, *q_hi;            // order statistics at ranks rank_lo / rank_hi
+    unsigned long long *sq_lo, *sq_hi;   // uint32: exact sum of squares, 128 bits (the variance follows on the host)
+    unsigned long long *isum;       // uint32: the exact integer sum
+    double *q_lo, *q_hi;            // order statistics at ranks rank_lo / rank_hi (select)
     uint64_t rank_lo, rank_hi;
-    const double *mean;             // device [n_cols] (second pass)
-    // pass 1 of a column accumulator (gatb_colacc_add, uint32 only): the integer results are ADDED to n_lt / n_eq /
-    // isum / sq_lo / sq_hi and the per-column extremes folded into col_min / col_max, so that successive slabs of
-    // rows give what one pass over all of them gives; rows are row_stride elements apart
-    int accumulate;
-    uint64_t row_stride;
-    uint32_t *col_min, *col_max;
+    const double *mean;             // float64: device [n_cols] (pass 2)
+    uint64_t row_stride;            // pass 1: elements from one row to the next (0: n_cols)
+    uint32_t *col_min, *col_max;    // uint32: per-column extremes, or NULL
 };
 // gat-compare (scripts/gat-compare.py:218-241, :300-323): the sampled log ratio of two fold-change columns,
 //   out[s][p] = log((obs1[p] / (m1[s][col1[p]] + pc) + 1e-4) / (obs2[p] / (m2[s][col2[p]] + pc) + 1e-4)) + delta[p]
@@ -183,14 +182,14 @@ struct StreamStatsParams {
     uint32_t n_chunks;              // chunks of rows_per_stage rows, dealt to the CTAs round-robin
     uint32_t n_stages, col_width;   // set by the launchers
     int use_tma;                    // 0: the matrix is not 16-byte aligned, the threads copy the chunks themselves
-    // pass 1 (outputs zeroed by the caller, accumulated with integer atomics)
+    // pass 1: the integers are ADDED to the caller's sums (ColumnSums in api.cu) with integer atomics
     // the comparison with the observed value as integer tests (set by stats_stream_thresholds):
     //   (double)v < observed  <=>  v < lt_thr  (or every v, flag 1);   (double)v == observed  <=>  flag 2 and v == eq_val
     const uint32_t *lt_thr, *eq_val, *col_flags;
     unsigned long long *isum, *n_lt, *n_eq;
     unsigned long long *sq_lo, *sq_hi;   // sum of squares, 128 bits
     uint32_t *vmax;                 // largest value of the matrix
-    uint32_t *col_min, *col_max;    // pass 1 of a column accumulator: extremes of every column (NULL: not wanted)
+    uint32_t *col_min, *col_max;    // extremes of every column folded in as well (MODE 2), or NULL (MODE 0)
     // select pass at bit `shift` (4 bits): prefix / rank per (which rank, column), [2][n_cols]
     uint32_t shift;
     uint32_t *prefix, *prefix_out;

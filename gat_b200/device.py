@@ -48,6 +48,17 @@ def to_csr(lists):
     return offs, start, end
 
 
+def _host_matrix(counts):
+    """a host sample matrix as the statistics entry points take it -> (matrix, is_float, n_samples, n_cols): float64
+    stays float64, anything else becomes uint32, both C-contiguous"""
+    counts = np.ascontiguousarray(counts)
+    is_float = int(counts.dtype == np.float64)
+    if not is_float:
+        counts = np.ascontiguousarray(counts, dtype=np.uint32)
+    n_samples, n_cols = counts.shape
+    return counts, is_float, n_samples, n_cols
+
+
 def counter_ids(counters):
     ids = []
     for c in counters:
@@ -112,13 +123,7 @@ class Context(object):
 
         counts: host ndarray [n_samples][n_cols] uint32 or float64; or pass device_ptr (+ shape)."""
         if device_ptr is None:
-            counts = np.ascontiguousarray(counts)
-            if counts.dtype == np.float64:
-                is_float = 1
-            else:
-                counts = np.ascontiguousarray(counts, dtype=np.uint32)
-                is_float = 0
-            n_samples, n_cols = counts.shape
+            counts, is_float, n_samples, n_cols = _host_matrix(counts)
             ptr, on_dev = _p(counts), 0
         else:
             ptr, on_dev = ctypes.c_void_p(device_ptr), 1
@@ -166,13 +171,7 @@ class Context(object):
     def column_pvalue(self, counts, values, expected):
         """AnnotatorResult.getEmpiricalPValue (gat/Engine.pyx:1829-1831): p-value of values[a] among the samples
         of column a against the STORED expectation expected[a]; counts: host ndarray [n_samples][n_cols]"""
-        counts = np.ascontiguousarray(counts)
-        if counts.dtype == np.float64:
-            is_float = 1
-        else:
-            counts = np.ascontiguousarray(counts, dtype=np.uint32)
-            is_float = 0
-        n_samples, n_cols = counts.shape
+        counts, is_float, n_samples, n_cols = _host_matrix(counts)
         v = np.ascontiguousarray(values, dtype=np.float64)
         e = np.ascontiguousarray(expected, dtype=np.float64)
         out = np.zeros(n_cols, dtype=np.float64)
