@@ -28,9 +28,6 @@ struct gatb_ctx {
     cudaStream_t upload_stream = nullptr;   // gatb_annotations_create_async: copies (+ a rebuild), off the compute stream
     cudaStream_t build_stream = nullptr;    // index build kernels, chunk by chunk behind the copies
     cudaStream_t copy_stream = nullptr;     // gatb_run with host outputs: device-to-host copies of batch i overlap batch i+1
-    cudaStream_t place_stream = nullptr;    // GATB_OVERLAP: placement kernels, beside the counting kernels on `stream`
-    cudaEvent_t ev_placed[2] = {nullptr, nullptr}, ev_count_done[2] = {nullptr, nullptr};
-    bool overlap = false;
     cudaEvent_t ev_counted[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     uint32_t *err_slots = nullptr;          // pinned words of pending asynchronous creates: 4 per set (validation, -, entries needed lo/hi)
     uint8_t *small_stage = nullptr;         // pinned: 16 KB per pending set for its small host-built tables (a copy from
@@ -51,8 +48,6 @@ struct gatb_ctx {
     // possibly peer GPUs, by the counting kernel's epilogue
     std::vector<gatb_route> routes;
     bool stats_stream = true;           // uint32 column statistics as TMA-streamed passes (GATB_STATS_STREAM=0: the column-tiled kernels)
-    bool discard_scratch = false;       // GATB_DISCARD=1: the placement kernels discard their dead buffer tails from L2 (halves
-                                        // their DRAM writes, costs 1-3 % of their time: profiles/r02_discard_ab.txt)
     bool route_copy = true;             // routes are served by copy engines from a staging slab (false: by the kernel's stores)
     bool trace = false;                 // GATB_TRACE=1: host-side phase times of gatb_run on stderr
     // optional per-kernel timing (bench.py roofline): CUDA events around every launch
@@ -193,8 +188,7 @@ struct PlaceBufs {                        // one batch of placed samples
     DevBuf<uint8_t> status;
 };
 struct BatchScratch {
-    PlaceBufs pb[2];                      // two sets: with GATB_OVERLAP the placement of batch i + 1 runs (on its own
-                                          // stream) beside the counting of batch i
+    PlaceBufs pb;
     DevBuf<uint32_t> out_tmp[2];          // host-output runs: two staging slabs, so that the copy of batch i
     DevBuf<double> out_tmp_f[2];          // to the host overlaps the kernels of batch i + 1
 };
@@ -230,12 +224,9 @@ extern "C" int gatb_create(int device, gatb_ctx **out)
     e = cudaStreamCreateWithFlags(&ctx->upload_stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->build_stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->place_stream, cudaStreamNonBlocking);
     for (int i = 0; i < 2 && e == cudaSuccess; i++) {
         e = cudaEventCreateWithFlags(&ctx->ev_counted[i], cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_placed[i], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_count_done[i], cudaEventDisableTiming);
     }
     if (e == cudaSuccess) e = cudaMallocHost(&ctx->err_slots, 256 * 4 * sizeof(uint32_t));
     if (e == cudaSuccess) e = cudaMallocHost(&ctx->small_stage, 256 * SMALL_STAGE_BYTES);
@@ -256,9 +247,6 @@ extern "C" int gatb_create(int device, gatb_ctx **out)
     ctx->schunk_max = env_u32("GATB_SCHUNK", 0);
     ctx->kgrp_max = env_u32("GATB_KEY_GROUP", 0);
     ctx->trace = env_u32("GATB_TRACE", 0) != 0;
-    ctx->overlap = env_u32("GATB_OVERLAP", 0) != 0;
-    ctx->route_copy = env_u32("GATB_ROUTE_KERNEL", 0) == 0;
-    ctx->discard_scratch = env_u32("GATB_DISCARD", 0) != 0;
     ctx->stats_stream = env_u32("GATB_STATS_STREAM", 1) != 0;
     ctx->scratch = new BatchScratch();
     ctx->blocks = new BlockCache();
@@ -278,12 +266,9 @@ extern "C" void gatb_destroy(gatb_ctx *ctx)
     if (ctx->upload_stream) cudaStreamDestroy(ctx->upload_stream);
     if (ctx->build_stream) cudaStreamDestroy(ctx->build_stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    if (ctx->place_stream) cudaStreamDestroy(ctx->place_stream);
     for (int i = 0; i < 2; i++) {
         if (ctx->ev_counted[i]) cudaEventDestroy(ctx->ev_counted[i]);
         if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
-        if (ctx->ev_placed[i]) cudaEventDestroy(ctx->ev_placed[i]);
-        if (ctx->ev_count_done[i]) cudaEventDestroy(ctx->ev_count_done[i]);
     }
     if (ctx->err_slots) cudaFreeHost(ctx->err_slots);
     if (ctx->small_stage) cudaFreeHost(ctx->small_stage);
@@ -1085,19 +1070,17 @@ static uint32_t pick_batch(const gatb_sampler *s, uint64_t n_samples)
     return (uint32_t)std::max<uint64_t>(b, 1);
 }
 
-static int ensure_batch(gatb_sampler *s, uint32_t B, int n_sets = 1)
+static int ensure_batch(gatb_sampler *s, uint32_t B)
 {
     gatb_ctx *ctx = s->ctx;
-    for (int i = 0; i < n_sets; i++) {
-        PlaceBufs &pb = ctx->scratch->pb[i];
-        CU(ctx, pb.placed.ensure((uint64_t)B * s->placed_stride));
-        CU(ctx, pb.placed_n.ensure((uint64_t)B * s->n_contigs));
-        if (s->has_iso) {
-            CU(ctx, pb.unit_buf.ensure((uint64_t)B * s->unit_stride));
-            CU(ctx, pb.unit_n.ensure((uint64_t)B * s->n_units));
-        }
-        CU(ctx, pb.status.ensure((uint64_t)B * s->n_units));
+    PlaceBufs &pb = ctx->scratch->pb;
+    CU(ctx, pb.placed.ensure((uint64_t)B * s->placed_stride));
+    CU(ctx, pb.placed_n.ensure((uint64_t)B * s->n_contigs));
+    if (s->has_iso) {
+        CU(ctx, pb.unit_buf.ensure((uint64_t)B * s->unit_stride));
+        CU(ctx, pb.unit_n.ensure((uint64_t)B * s->n_units));
     }
+    CU(ctx, pb.status.ensure((uint64_t)B * s->n_units));
     return GATB_OK;
 }
 
@@ -1124,12 +1107,11 @@ __global__ void tally_kernel(const uint32_t *placed_n, uint64_t n_placed, const 
 }
 
 // enqueue K1 (+K2) for one batch; result in s->placed / s->placed_n
-static int place_batch(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t sample_begin, uint32_t B, int set = 0,
-                       cudaStream_t on = nullptr)
+static int place_batch(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t sample_begin, uint32_t B)
 {
     gatb_ctx *ctx = s->ctx;
-    cudaStream_t st = on ? on : ctx->stream;
-    PlaceBufs &pb = ctx->scratch->pb[set];
+    cudaStream_t st = ctx->stream;
+    PlaceBufs &pb = ctx->scratch->pb;
     PlaceParams p;
     memset(&p, 0, sizeof(p));
     p.units = s->units.p; p.order = s->order.p;
@@ -1146,7 +1128,6 @@ static int place_batch(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t 
     p.seed = seed; p.track = track; p.sampler_kind = s->kind;
     p.seg_start = s->seg_start.p; p.seg_end = s->seg_end.p;
     p.shift_half_radius = s->shift_radius / 2; p.shift_extension = s->shift_extension;
-    p.discard_scratch = ctx->discard_scratch ? 1 : 0;
     { ProfScope ps(ctx, PROF_PLACE, st); launch_place(st, p); }
     CU(ctx, cudaGetLastError());
     if (s->has_iso) {
@@ -1156,7 +1137,6 @@ static int place_batch(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t 
         m.contig_base = s->contig_base.p; m.unit_buf = pb.unit_buf.p; m.unit_stride = s->unit_stride;
         m.unit_n = pb.unit_n.p; m.placed = pb.placed.p; m.placed_stride = s->placed_stride;
         m.placed_n = pb.placed_n.p; m.n_units = s->n_units; m.n_contigs = s->n_contigs; m.n_samples = B;
-        m.discard_scratch = ctx->discard_scratch ? 1 : 0;
         { ProfScope ps(ctx, PROF_MERGE, st); launch_contig_merge(st, m); }
         CU(ctx, cudaGetLastError());
     }
@@ -1213,7 +1193,7 @@ static int place_once(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t s
 {
     gatb_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
-    PlaceBufs *sc = &ctx->scratch->pb[0];
+    PlaceBufs *sc = &ctx->scratch->pb;
     const bool from_units = by_unit && s->has_iso;          // the unit-level buffers (before fromIsochores)
     const uint64_t stride = from_units ? s->unit_stride : s->placed_stride;
     const uint32_t n_lists = by_unit ? s->n_units : s->n_contigs;
@@ -1314,21 +1294,15 @@ static int run_once(gatb_sampler *s, const gatb_annotations *annos, int n_counte
     const auto t_begin = std::chrono::steady_clock::now();
     auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
     double t_alloc = 0, t_placeq = 0, t_annos = 0, t_countq = 0;
-    // GATB_OVERLAP: the placement of batch i + 1 runs on its own stream beside the counting of batch i (two sets of
-    // placement buffers; the two kernels stress different units: placement is latency-bound, counting saturates the
-    // L1 data pipe)
-    const bool overlap = ctx->overlap && n_samples > B;
-    cudaStream_t pst = overlap ? ctx->place_stream : st;
-    int rc = ensure_batch(s, B, overlap ? 2 : 1);
+    int rc = ensure_batch(s, B);
     if (rc) return rc;
     t_alloc = since();
     BatchScratch *sc = ctx->scratch;
-    bool count_pending[2] = {false, false};
-    // Output routes, two ways to serve them: (a) the counting kernel's epilogue stores every row to every route
-    // itself (GATB_ROUTE_KERNEL=1), (b) the kernel writes a plain staging slab and COPY ENGINES scatter its rows /
-    // column blocks to the routes (2-D device-to-device copies on the copy stream, peer GPUs included) while the
-    // compute stream goes on with the next batch -- the default: (a) put 7 x 16 MB of NVLink stores at the very end
-    // of every 1.2 ms kernel, where nothing overlaps them (8 GPUs: 60.3 ms per step against 55.9 on one GPU).
+    // Output routes, two ways to serve them (gatb_set_route_mode): (a) the counting kernel's epilogue stores every
+    // row to every route itself (by_kernel = 1), (b) the kernel writes a plain staging slab and COPY ENGINES scatter
+    // its rows / column blocks to the routes (2-D device-to-device copies on the copy stream, peer GPUs included)
+    // while the compute stream goes on with the next batch -- the default: (a) put 7 x 16 MB of NVLink stores at the
+    // very end of every 1.2 ms kernel, where nothing overlaps them (8 GPUs: 60.3 ms per step against 55.9 on one GPU).
     const bool routed = !ctx->routes.empty();
     const bool staged = !out_is_device || (routed && ctx->route_copy);
     const int n_stage = (staged && (n_samples > B || n_counters > 1)) ? 2 : 1;
@@ -1343,27 +1317,15 @@ static int run_once(gatb_sampler *s, const gatb_annotations *annos, int n_counte
     // the compute stream goes on with the next (counter, batch), which uses the other slab
     uint64_t n_staged = 0;
     bool copied_pending[2] = {false, false};
-
-    if (overlap) {                       // the placement stream starts behind the memsets above
-        CU(ctx, cudaEventRecord(ctx->ev_placed[0], st));
-        CU(ctx, cudaStreamWaitEvent(pst, ctx->ev_placed[0], 0));
-    }
-    uint64_t batch_no = 0;
-    for (uint64_t done = 0; done < n_samples; done += B, batch_no++) {
+    for (uint64_t done = 0; done < n_samples; done += B) {
         const uint32_t b = (uint32_t)std::min<uint64_t>(B, n_samples - done);
-        const int set = overlap ? (int)(batch_no & 1) : 0;
-        if (overlap && count_pending[set]) CU(ctx, cudaStreamWaitEvent(pst, ctx->ev_count_done[set], 0));   // buffers free again
-        rc = place_batch(s, seed, track, sample_begin + done, b, set, pst);
+        rc = place_batch(s, seed, track, sample_begin + done, b);
         if (rc) return rc;
-        if (overlap) {
-            CU(ctx, cudaEventRecord(ctx->ev_placed[set], pst));
-            CU(ctx, cudaStreamWaitEvent(st, ctx->ev_placed[set], 0));
-        }
         if (done == 0) t_placeq = since();
         CountParams p;
         memset(&p, 0, sizeof(p));
-        p.placed = sc->pb[set].placed.p; p.sample_stride = s->placed_stride; p.key_base = s->contig_base.p;
-        p.placed_n = sc->pb[set].placed_n.p; p.key_present = nullptr;
+        p.placed = sc->pb.placed.p; p.sample_stride = s->placed_stride; p.key_base = s->contig_base.p;
+        p.placed_n = sc->pb.placed_n.p; p.key_present = nullptr;
         for (int c = 0; c < n_counters; c++) {
             const bool dens = counters[c] == GATB_NUCLEOTIDE_DENSITY;
             rc = count_params_annos(annos, b, dens, p);
@@ -1423,14 +1385,6 @@ static int run_once(gatb_sampler *s, const gatb_annotations *annos, int n_counte
                 n_staged++;
             }
         }
-        if (overlap) {
-            CU(ctx, cudaEventRecord(ctx->ev_count_done[set], st));
-            count_pending[set] = true;
-        }
-    }
-    if (overlap) {                       // the tally (placement stream) is read back through `st` below
-        CU(ctx, cudaEventRecord(ctx->ev_placed[0], pst));
-        CU(ctx, cudaStreamWaitEvent(st, ctx->ev_placed[0], 0));
     }
     // the compute stream joins the last copies: one synchronisation point for the caller
     for (int i = 0; i < 2; i++)
@@ -1496,14 +1450,14 @@ extern "C" int gatb_count_work(gatb_sampler *s, const gatb_annotations *annos, u
     if (rc) return rc;
     tl_stream = ctx->stream;
     cudaStream_t st = ctx->stream;
-    if (ctx->scratch->pb[0].placed.n < (uint64_t)n_samples * s->placed_stride || ctx->scratch->pb[0].placed_n.n < (uint64_t)n_samples * s->n_contigs)
+    if (ctx->scratch->pb.placed.n < (uint64_t)n_samples * s->placed_stride || ctx->scratch->pb.placed_n.n < (uint64_t)n_samples * s->n_contigs)
         return fail(ctx, GATB_ERR_INVALID, "count_work: no batch of that size has been placed");
     CountParams p;
     memset(&p, 0, sizeof(p));
     rc = count_params_annos(annos, n_samples, false, p);
     if (rc) return rc;
-    p.placed = ctx->scratch->pb[0].placed.p; p.sample_stride = s->placed_stride; p.key_base = s->contig_base.p;
-    p.placed_n = ctx->scratch->pb[0].placed_n.p;
+    p.placed = ctx->scratch->pb.placed.p; p.sample_stride = s->placed_stride; p.key_base = s->contig_base.p;
+    p.placed_n = ctx->scratch->pb.placed_n.p;
     DevBuf<unsigned long long> d_out;
     CU(ctx, d_out.alloc(2));
     CU(ctx, cudaMemsetAsync(d_out.p, 0, 2 * sizeof(unsigned long long), st));

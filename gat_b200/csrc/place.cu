@@ -9,19 +9,8 @@
 // dropped: late turns are `certain` ones whose draw is already put off, so it saved nothing and cost registers.)  The result is bit-identical to the sequential restatement in oracle/gat_oracle.c
 // driven by the same Philox stream (tests/test_gpu_parity.py).
 #include "place.cuh"
-#include "ptx.cuh"
 
 namespace gatb {
-
-// What lies behind a finished list in its buffer -- the sorts' scratch, placements dropped by a merge -- is dead, but
-// its lines sit dirty in L2 and would be written to HBM like the list itself: half of the kernels' DRAM writes.
-// Discard the lines that lie entirely inside buf[n, cap).
-__device__ __forceinline__ void warp_discard_tail(const uint64_t *buf, uint64_t n, uint64_t cap)
-{
-    const uint64_t first = ((uint64_t)(uintptr_t)(buf + n) + 127ull) & ~127ull;
-    const uint64_t last = (uint64_t)(uintptr_t)(buf + cap) & ~127ull;
-    for (uint64_t a = first + (uint64_t)lane_id() * 128ull; a < last; a += 32ull * 128ull) discard_l2_line(a);
-}
 
 // ---------------------------------------------------------------------------------------------------
 // draws of one loop turn (RNG contract, DESIGN.md)
@@ -379,7 +368,6 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
         if (orphans) nu = warp_filter_ws(buf, nu, ws);
     }
     __syncwarp();
-    if (p.discard_scratch) warp_discard_tail(buf, nu, d.cap);
     if (lane == 0) {
         uint32_t slot = p.out_by_contig ? d.contig : unit;
         p.out_n[(uint64_t)sl * p.out_n_stride + slot] = (status & UNIT_OVERFLOW) ? 0u : nu;
@@ -563,7 +551,6 @@ __global__ void __launch_bounds__(128) shift_kernel(PlaceParams p)
     if (n > d.cap) status |= UNIT_OVERFLOW;
     else nu = warp_sort_merge0<true>(buf, n, 2u * n <= d.cap ? buf + n : nullptr, sort_cnt[threadIdx.x >> 5]);
     __syncwarp();
-    if (p.discard_scratch) warp_discard_tail(buf, nu, d.cap);
     if (lane == 0) {
         const uint32_t slot = p.out_by_contig ? d.contig : unit;
         p.out_n[(uint64_t)sl * p.out_n_stride + slot] = nu;
@@ -606,7 +593,6 @@ __global__ void __launch_bounds__(128) contig_merge_kernel(MergeParams p)
     const uint64_t cap = (c + 1 < p.n_contigs ? p.contig_base[c + 1] : p.placed_stride) - p.contig_base[c];
     uint32_t n = warp_sort_merge0(dst, total, 2ull * total <= cap ? dst + total : nullptr, sort_cnt[threadIdx.x >> 5]);
     __syncwarp();
-    if (p.discard_scratch) warp_discard_tail(dst, n, cap);
     if (lane == 0) p.placed_n[(uint64_t)sl * p.n_contigs + c] = n;
 }
 

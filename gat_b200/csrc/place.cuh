@@ -55,7 +55,6 @@ struct PlaceParams {
     const uint32_t *seg_start, *seg_end;   // raw segments of the units (UnitDesc.seg_off / seg_n); kind 2 only
     double shift_half_radius;    // SamplerShift: radius / 2 (:1054)
     int32_t shift_extension;     // SamplerShift: extension (0 = use the radius, :1074-1077)
-    int discard_scratch;         // 1: dead sort scratch is discarded from L2 instead of being written back (place.cu)
 };
 
 struct MergeParams {             // K2: per (sample, contig) concat + merge(0) of the contig's units
@@ -70,7 +69,6 @@ struct MergeParams {             // K2: per (sample, contig) concat + merge(0) o
     uint64_t placed_stride;
     uint32_t *placed_n;                // [n_samples][n_contigs]
     uint32_t n_units, n_contigs, n_samples;
-    int discard_scratch;               // as in PlaceParams
 };
 
 void launch_prep_units(cudaStream_t st, UnitDesc *units, uint32_t n_units,

@@ -1,7 +1,6 @@
 // ptx.cuh -- the inline-PTX accessors of the kernels (sm_100a).  Counting kernel: shared memory by 32-bit shared
 // address, read-only vector loads by 64-bit global address, a clamping shift and the accumulator address as one IMAD.
-// Placement kernels: L2 discard of dead scratch lines.  Statistics: TMA bulk copies global -> shared with mbarrier
-// completion.
+// Statistics: TMA bulk copies global -> shared with mbarrier completion.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -68,12 +67,6 @@ __device__ __forceinline__ uint32_t acc_cell(uint32_t wy, uint32_t acc_addr)
     uint32_t cell;
     asm("mad.lo.u32 %0, %1, 4, %2;" : "=r"(cell) : "r"(wy & 0xfffu), "r"(acc_addr));
     return cell;
-}
-// The 128-byte line at `addr` (128-byte aligned, global) holds nothing anyone will read again: L2 may drop it instead
-// of writing it back to HBM (discard.global.L2; the line's content is undefined afterwards)
-__device__ __forceinline__ void discard_l2_line(uint64_t addr)
-{
-    asm volatile("discard.global.L2 [%0], 128;" ::"l"(addr) : "memory");
 }
 
 // ---- TMA bulk copy global -> shared, completion counted in bytes on an mbarrier (shared addresses as above) ----

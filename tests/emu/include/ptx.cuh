@@ -22,10 +22,6 @@ __device__ __forceinline__ uint2 ldg_nc_u2(uint64_t addr) { uint2 v; memcpy(&v, 
 __device__ __forceinline__ uint4 ldg_nc_u4(uint64_t addr) { uint4 v; memcpy(&v, (const void *)addr, sizeof(v)); return v; }
 __device__ __forceinline__ uint32_t shl_clamp(uint32_t v, uint32_t n) { return n >= 32u ? 0u : v << n; }
 __device__ __forceinline__ uint32_t acc_cell(uint32_t wy, uint32_t acc_addr) { return (wy & 0xfffu) * 4u + acc_addr; }
-__device__ __forceinline__ void discard_l2_line(uint64_t addr)
-{
-    memset((void *)addr, 0xDD, 128);                // "undefined afterwards": make a later read of it visible
-}
 
 // mbarrier + TMA bulk copy: the copy happens at once, the barrier word counts completed phases
 __device__ __forceinline__ void mbar_init(uint32_t mbar, uint32_t) { emu_sts<uint64_t>(mbar, 0ull); }

@@ -79,21 +79,3 @@ def test_engine_refuses_the_emulated_build(emu_lib, monkeypatch):
     monkeypatch.setattr(_lib, "LIB_PATH", build_emu.LIB)
     with pytest.raises(ImportError):
         _lib.load()
-
-
-def test_l2_discard_of_dead_buffer_tails_changes_nothing(oracle, monkeypatch):
-    """GATB_DISCARD=1 (place.cu warp_discard_tail): the emulation overwrites every discarded line, so a discard that
-    reached into live data would show up as a difference from the oracle"""
-    import emu_context
-    from tests import test_gpu_parity as G
-    monkeypatch.setenv("GATB_DISCARD", "1")
-    c = emu_context.context()
-    monkeypatch.delenv("GATB_DISCARD")
-    try:
-        G.test_place_single_units_match_oracle(c, oracle)
-        for n_iso in (0, 3):
-            G.test_place_problem_matches_oracle(c, oracle, n_iso)
-            G.test_run_matches_oracle(c, oracle, n_iso)
-        G.test_sampler_shift_matches_oracle(c, oracle)
-    finally:
-        c.close()

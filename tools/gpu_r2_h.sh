@@ -1,5 +1,5 @@
 #!/bin/bash
-# round 2, GPU call H (1 GPU): placement / counting overlap experiment (GATB_OVERLAP, GATB_COUNT_THREADS)
+# round 2, GPU call H (1 GPU): counting CTA size experiment (GATB_COUNT_THREADS)
 mkdir -p gpurun_out
 cd "$(dirname "$0")/.."
 run() {
@@ -15,7 +15,4 @@ except Exception as e:
 PY
 }
 run base GATB_X=0
-run overlap512 GATB_OVERLAP=1 GATB_COUNT_THREADS=512
-run overlap1024 GATB_OVERLAP=1
 run threads512 GATB_COUNT_THREADS=512
-run overlap768 GATB_OVERLAP=1 GATB_COUNT_THREADS=768

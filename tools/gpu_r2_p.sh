@@ -1,5 +1,5 @@
 #!/bin/bash
-# round 2, GPU call P (1 GPU): compute-sanitizer on the TMA-streamed statistics and the discarding placement kernels
+# round 2, GPU call P (1 GPU): compute-sanitizer on the TMA-streamed statistics and the placement kernels
 mkdir -p gpurun_out
 cd "$(dirname "$0")/.."
 for tool in memcheck racecheck synccheck; do

@@ -1,6 +1,5 @@
-"""Small run of the TMA-streamed column statistics and of the placement kernels with the L2 discard, for
-compute-sanitizer (memcheck / racecheck / synccheck): shapes that use the bulk-copy path, the partial last chunk and
-several select passes.
+"""Small run of the TMA-streamed column statistics and of the placement kernels, for compute-sanitizer (memcheck /
+racecheck / synccheck): shapes that use the bulk-copy path, the partial last chunk and several select passes.
 
     compute-sanitizer --tool racecheck python tools/sanitizer_stats.py
 """
@@ -12,7 +11,6 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(
 
 import numpy as np  # noqa: E402
 
-os.environ["GATB_DISCARD"] = "1"
 from gat_b200 import device  # noqa: E402
 import helpers  # noqa: E402
 
