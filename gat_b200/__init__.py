@@ -512,7 +512,22 @@ def _dumpSamples(smp, track, track_index, segs, workspace, num_samples, pattern)
 
 
 def fromCounts(filename):
-    """annotator results from a counts table written with output_counts_pattern (gat/__init__.py:1091-1119)"""
+    """annotator results from a counts table written with output_counts_pattern (gat/__init__.py:1091-1119).  The
+    table is parsed on the GPU (Engine.readCountsTable) and the statistics of all rows come from one call; the samples
+    stay on the device, as after run().  Tables the GPU reader does not take go through _fromCountsHost."""
+    table = Engine.readCountsTable(filename)
+    if table is None:
+        return _fromCountsHost(filename)
+    rows, matrix = table
+    st = getContext().column_stats(None, [r[2] for r in rows], pseudo_count=1.0, device_ptr=matrix._tensor.data_ptr(),
+                                   n_samples=matrix.nsamples, n_cols=matrix.ncolumns, is_float=0)
+    return [AnnotatorResult(track=track, annotation=annotation, counter="na", observed=observed, samples=(matrix, i),
+                            stats=dict((k, float(v[i])) for k, v in st.items()))
+            for i, (track, annotation, observed) in enumerate(rows)]
+
+
+def _fromCountsHost(filename):
+    """fromCounts parsed on the host, line by line as the reference does"""
     results = []
     with _open(filename, "r") as infile:
         header = infile.readline()

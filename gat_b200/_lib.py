@@ -23,7 +23,7 @@ SYMBOLS = [
     "gatb_sampler_create", "gatb_sampler_destroy", "gatb_sampler_sample_capacity",
     "gatb_sampler_unit_capacity", "gatb_sampler_set_kind", "gatb_sampler_set_shift", "gatb_sampler_place",
     "gatb_sampler_place_units", "gatb_run", "gatb_column_stats", "gatb_column_pvalue", "gatb_compare_stats",
-    "gatb_format_counts", "gatb_count_work", "gatb_microbench",
+    "gatb_compare_stats_device", "gatb_format_counts", "gatb_parse_counts", "gatb_count_work", "gatb_microbench",
     "gatb_lists_from_rows", "gatb_lists_from_csr", "gatb_lists_restrict", "gatb_lists_collapse", "gatb_lists_select",
     "gatb_lists_info", "gatb_lists_sizes", "gatb_lists_download", "gatb_lists_destroy",
     "gatb_annotations_create_from_lists",
@@ -127,8 +127,13 @@ def bind(L):
     L.gatb_column_stats.argtypes = [vp, vp, i32, i32, u64, i32, vp, vp, dbl, vp, vp, vp, vp, vp, vp]
     L.gatb_compare_stats.restype = i32
     L.gatb_compare_stats.argtypes = [vp, u64, vp, i32, vp, i32, u64, vp, vp, vp, vp, vp, dbl, vp, vp, vp, vp, vp, vp]
+    L.gatb_compare_stats_device.restype = i32
+    L.gatb_compare_stats_device.argtypes = [vp, u64, vp, i32, i32, vp, i32, i32, u64, vp, vp, vp, vp, vp, dbl,
+                                            vp, vp, vp, vp, vp, vp]
     L.gatb_format_counts.restype = i32
     L.gatb_format_counts.argtypes = [vp, vp, i32, u64, i32, vp, vp, u64]
+    L.gatb_parse_counts.restype = i32
+    L.gatb_parse_counts.argtypes = [vp, vp, u64, u64, vp, vp, vp, vp, vp, vp]
     L.gatb_count_work.restype = i32
     L.gatb_count_work.argtypes = [vp, vp, u32, vp]
     L.gatb_microbench.restype = i32

@@ -50,7 +50,23 @@ def buildParser():
 
 def fromCountsBatched(filename):
     """gat.fromCounts (gat/__init__.py:1091-1119) with ONE statistics call for all rows of the file.
-    -> (results, matrix [n_samples][n_rows] float64)"""
+    -> (results, matrix [n_samples][n_rows]): the uint32 SampleMatrix of the GPU reader (Engine.readCountsTable), or
+    the float64 host array of _fromCountsHost for tables that reader does not take"""
+    table = Engine.readCountsTable(filename)
+    if table is None:
+        return _fromCountsHost(filename)
+    rows, matrix = table
+    st = Engine.getContext().column_stats(None, [r[2] for r in rows], pseudo_count=1.0,
+                                          device_ptr=matrix._tensor.data_ptr(), n_samples=matrix.nsamples,
+                                          n_cols=matrix.ncolumns, is_float=0)
+    results = [Engine.AnnotatorResult(track, annotation, "na", observed, (matrix, i),
+                                      stats=dict((k, float(v[i])) for k, v in st.items()))
+               for i, (track, annotation, observed) in enumerate(rows)]
+    return results, matrix
+
+
+def _fromCountsHost(filename):
+    """fromCountsBatched parsed on the host, line by line -> (results, matrix [n_samples][n_rows] float64)"""
     rows = []
     with IO.openFile(filename, "r") as infile:
         header = infile.readline()
@@ -78,6 +94,11 @@ def _as_counts(matrix):
     if matrix.size and np.all(matrix == np.floor(matrix)) and matrix.min() >= 0 and matrix.max() < 2 ** 32:
         return matrix.astype(np.uint32)
     return matrix
+
+
+def _nsamples(matrix):
+    """samples of a host array or of a SampleMatrix"""
+    return matrix.nsamples if isinstance(matrix, Engine.SampleMatrix) else matrix.shape[0]
 
 
 def comparePairs(pairs, m1, m2, pseudo_count):
@@ -144,7 +165,7 @@ def main(argv=None):
     else:
         for i1, i2 in itertools.combinations(range(len(loaded)), 2):
             (a, ma), (b, mb) = loaded[i1], loaded[i2]
-            if ma.shape[0] != mb.shape[0]:
+            if _nsamples(ma) != _nsamples(mb):
                 raise ValueError("count tables differ in the number of samples")
             aa = dict(((x.track, x.annotation), (x, i)) for i, x in enumerate(a))
             bb = dict(((x.track, x.annotation), (x, i)) for i, x in enumerate(b))

@@ -2012,27 +2012,16 @@ extern "C" void gatb_colacc_destroy(gatb_colacc *c)
 }
 
 // ---------------------------------------------------------------------------------------------------
-// gat-compare: statistics of the sampled log ratio of two fold-change columns, pair by pair
-extern "C" int gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const double *m1, int n_cols1,
-                                  const double *m2, int n_cols2, uint64_t n_pairs, const int32_t *col1,
-                                  const int32_t *col2, const double *obs1, const double *obs2, const double *delta,
-                                  double pseudo_count, double *expected, double *stddev, double *lower95,
-                                  double *upper95, double *fold, double *pvalue)
+// gat-compare: statistics of the sampled log ratio of two fold-change columns, pair by pair.  m1 / m2: device matrices,
+// uint32 or float64 each (is_float1 / is_float2); the derived samples are the same doubles either way
+static int compare_stats(gatb_ctx *ctx, uint64_t n_samples, const void *m1, int is_float1, int n_cols1, const void *m2,
+                         int is_float2, int n_cols2, uint64_t n_pairs, const int32_t *col1, const int32_t *col2,
+                         const double *obs1, const double *obs2, const double *delta, double pseudo_count,
+                         double *expected, double *stddev, double *lower95, double *upper95, double *fold, double *pvalue)
 {
-    if (!ctx || !m1 || !m2 || !col1 || !col2 || !obs1 || !obs2 || !delta || n_cols1 <= 0 || n_cols2 <= 0)
-        return GATB_ERR_INVALID;
-    if (n_samples < 1) return fail(ctx, GATB_ERR_INVALID, "compare_stats: no samples");
-    for (uint64_t q = 0; q < n_pairs; q++)
-        if (col1[q] < 0 || col1[q] >= n_cols1 || col2[q] < 0 || col2[q] >= n_cols2)
-            return fail(ctx, GATB_ERR_INVALID, "compare_stats: column index out of range");
-    if (n_pairs == 0) return GATB_OK;
-    CU(ctx, cudaSetDevice(ctx->device));
-    tl_stream = ctx->stream;
     cudaStream_t st = ctx->stream;
-    DevBuf<double> d_m1, d_m2, d_o1, d_o2, d_delta, d_out;
+    DevBuf<double> d_o1, d_o2, d_delta, d_out;
     DevBuf<int32_t> d_c1, d_c2;
-    CU(ctx, d_m1.upload(m1, n_samples * (uint64_t)n_cols1, st));
-    if (m2 != m1) CU(ctx, d_m2.upload(m2, n_samples * (uint64_t)n_cols2, st));
     CU(ctx, d_c1.upload(col1, n_pairs, st)); CU(ctx, d_c2.upload(col2, n_pairs, st));
     CU(ctx, d_o1.upload(obs1, n_pairs, st)); CU(ctx, d_o2.upload(obs2, n_pairs, st));
     CU(ctx, d_delta.upload(delta, n_pairs, st));
@@ -2042,7 +2031,7 @@ extern "C" int gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const doubl
     for (uint64_t p0 = 0; p0 < n_pairs; p0 += chunk) {
         const uint32_t np = (uint32_t)std::min<uint64_t>(chunk, n_pairs - p0);
         CompareParams cp;
-        cp.m1 = d_m1.p; cp.m2 = (m2 != m1) ? d_m2.p : d_m1.p;
+        cp.m1 = m1; cp.m2 = m2; cp.is_float1 = is_float1; cp.is_float2 = is_float2;
         cp.n_cols1 = (uint32_t)n_cols1; cp.n_cols2 = (uint32_t)n_cols2; cp.n_samples = n_samples;
         cp.col1 = d_c1.p + p0; cp.col2 = d_c2.p + p0;
         cp.obs1 = d_o1.p + p0; cp.obs2 = d_o2.p + p0; cp.delta = d_delta.p + p0;
@@ -2057,6 +2046,49 @@ extern "C" int gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const doubl
         if (rc) return rc;
     }
     return GATB_OK;
+}
+
+static int compare_check(gatb_ctx *ctx, uint64_t n_samples, int n_cols1, int n_cols2, uint64_t n_pairs, const int32_t *col1,
+                         const int32_t *col2)
+{
+    if (n_samples < 1) return fail(ctx, GATB_ERR_INVALID, "compare_stats: no samples");
+    for (uint64_t q = 0; q < n_pairs; q++)
+        if (col1[q] < 0 || col1[q] >= n_cols1 || col2[q] < 0 || col2[q] >= n_cols2)
+            return fail(ctx, GATB_ERR_INVALID, "compare_stats: column index out of range");
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    return GATB_OK;
+}
+
+extern "C" int gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const double *m1, int n_cols1,
+                                  const double *m2, int n_cols2, uint64_t n_pairs, const int32_t *col1,
+                                  const int32_t *col2, const double *obs1, const double *obs2, const double *delta,
+                                  double pseudo_count, double *expected, double *stddev, double *lower95,
+                                  double *upper95, double *fold, double *pvalue)
+{
+    if (!ctx || !m1 || !m2 || !col1 || !col2 || !obs1 || !obs2 || !delta || n_cols1 <= 0 || n_cols2 <= 0)
+        return GATB_ERR_INVALID;
+    if (const int rc = compare_check(ctx, n_samples, n_cols1, n_cols2, n_pairs, col1, col2)) return rc;
+    if (n_pairs == 0) return GATB_OK;
+    DevBuf<double> d_m1, d_m2;
+    CU(ctx, d_m1.upload(m1, n_samples * (uint64_t)n_cols1, ctx->stream));
+    if (m2 != m1) CU(ctx, d_m2.upload(m2, n_samples * (uint64_t)n_cols2, ctx->stream));
+    return compare_stats(ctx, n_samples, d_m1.p, 1, n_cols1, m2 != m1 ? d_m2.p : d_m1.p, 1, n_cols2, n_pairs, col1, col2,
+                         obs1, obs2, delta, pseudo_count, expected, stddev, lower95, upper95, fold, pvalue);
+}
+
+extern "C" int gatb_compare_stats_device(gatb_ctx *ctx, uint64_t n_samples, const void *m1, int is_float1, int n_cols1,
+                                         const void *m2, int is_float2, int n_cols2, uint64_t n_pairs, const int32_t *col1,
+                                         const int32_t *col2, const double *obs1, const double *obs2, const double *delta,
+                                         double pseudo_count, double *expected, double *stddev, double *lower95,
+                                         double *upper95, double *fold, double *pvalue)
+{
+    if (!ctx || !m1 || !m2 || !col1 || !col2 || !obs1 || !obs2 || !delta || n_cols1 <= 0 || n_cols2 <= 0)
+        return GATB_ERR_INVALID;
+    if (const int rc = compare_check(ctx, n_samples, n_cols1, n_cols2, n_pairs, col1, col2)) return rc;
+    if (n_pairs == 0) return GATB_OK;
+    return compare_stats(ctx, n_samples, m1, is_float1 ? 1 : 0, n_cols1, m2, is_float2 ? 1 : 0, n_cols2, n_pairs, col1, col2,
+                         obs1, obs2, delta, pseudo_count, expected, stddev, lower95, upper95, fold, pvalue);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -2484,5 +2516,85 @@ extern "C" int gatb_peer_close(gatb_ctx *ctx, void *ptr)
     if (!ctx) return GATB_ERR_INVALID;
     CU(ctx, cudaSetDevice(ctx->device));
     if (ptr) CU(ctx, cudaIpcCloseMemHandle(ptr));
+    return GATB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// counts table reader (--input-counts-file, gat-compare): the passes of count.cu ("counts table parsing").  The first
+// call (counts == NULL) checks the grammar; the second repeats the passes and stores the numbers, so that no state
+// lives between the calls (the passes cost a few reads of the text).
+extern "C" int gatb_parse_counts(gatb_ctx *ctx, const char *text, uint64_t n_bytes, uint64_t line_capacity,
+                                 uint64_t *n_rows, uint64_t *n_samples, int *plain, uint64_t *bad_offset,
+                                 uint64_t *lines, uint32_t *counts)
+{
+    if (!ctx || (!text && n_bytes) || !n_rows || !n_samples || !plain || !bad_offset || (line_capacity && !lines))
+        return GATB_ERR_INVALID;
+    *n_rows = 0; *n_samples = 0; *plain = 1; *bad_offset = PARSE_NONE;
+    if (n_bytes == 0) return counts ? fail(ctx, GATB_ERR_INVALID, "parse_counts: empty table") : GATB_OK;
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    ParseParams p;
+    memset(&p, 0, sizeof(p));
+    p.text = (const uint8_t *)text; p.n = n_bytes;
+    p.n_tiles = (n_bytes + PARSE_TILE - 1) / PARSE_TILE;
+    const uint64_t nt1 = p.n_tiles + 1;
+    DevBuf<unsigned long long> d_tiles, d_lines;
+    DevBuf<uint8_t> scan_tmp;
+    CU(ctx, d_tiles.alloc(3 * nt1 + 1));
+    CU(ctx, cudaMemsetAsync(d_tiles.p, 0, 3 * nt1 * sizeof(unsigned long long), st));
+    CU(ctx, cudaMemsetAsync(d_tiles.p + 3 * nt1, 0xff, sizeof(unsigned long long), st));
+    p.tile_nl = d_tiles.p; p.tile_tab = d_tiles.p + nt1; p.tile_comma = d_tiles.p + 2 * nt1; p.bad = d_tiles.p + 3 * nt1;
+    const size_t scan_bytes = parse_scan_bytes(p.n_tiles);
+    CU(ctx, scan_tmp.alloc(std::max<size_t>(scan_bytes, 1)));
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_parse_tiles(st, p, scan_tmp.p, scan_bytes)); }
+    unsigned long long bad = PARSE_NONE;
+    CU(ctx, cudaMemcpyAsync(&p.n_lines, p.tile_nl + p.n_tiles, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    if (p.n_lines) {
+        const uint64_t R = p.n_lines;
+        CU(ctx, d_lines.alloc(5 * R));
+        p.line_end = d_lines.p; p.tabs_end = d_lines.p + R; p.commas_end = d_lines.p + 2 * R;
+        p.counts_start = d_lines.p + 3 * R; p.comma0 = d_lines.p + 4 * R;
+        CU(ctx, cudaMemsetAsync(p.counts_start, 0xff, R * sizeof(unsigned long long), st));
+        CU(ctx, cudaMemsetAsync(p.comma0, 0, R * sizeof(unsigned long long), st));
+        { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_parse_marks(st, p)); }
+        { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_parse_lines(st, p)); }
+        unsigned long long first[3];                    // the first line: commas at its end, counts start, commas before it
+        CU(ctx, cudaMemcpyAsync(first, p.commas_end, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(first + 1, p.counts_start, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(first + 2, p.comma0, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(&bad, p.bad, sizeof(bad), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        p.n_values = first[1] == PARSE_NONE ? 0 : first[0] - first[2] + 1;
+    } else bad = 0;                                     // no '\n' at all: one unterminated line
+    DevBuf<uint32_t> d_rows;                            // [line][value]
+    if (p.n_lines && counts && bad == PARSE_NONE) {
+        CU(ctx, d_rows.alloc(p.n_lines * p.n_values));
+        p.values = d_rows.p;
+    }
+    if (p.n_lines) {
+        { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_parse_values(st, p)); }
+        CU(ctx, cudaMemcpyAsync(&bad, p.bad, sizeof(bad), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+    }
+    *plain = bad == PARSE_NONE;
+    *bad_offset = bad;
+    if (!*plain) return counts ? fail(ctx, GATB_ERR_INVALID, "parse_counts: not a plain counts table (offending byte at offset " +
+                                                                 std::to_string(bad) + ")") : GATB_OK;
+    *n_rows = p.n_lines; *n_samples = p.n_values;
+    if (lines) {
+        const uint64_t R = std::min<uint64_t>(p.n_lines, line_capacity);
+        std::vector<unsigned long long> h(2 * R);
+        CU(ctx, cudaMemcpyAsync(h.data(), p.line_end, R * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(h.data() + R, p.counts_start, R * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        for (uint64_t l = 0; l < R; l++) { lines[2 * l] = l ? h[l - 1] + 1 : 0; lines[2 * l + 1] = h[R + l]; }
+    }
+    if (counts) {
+        { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_transpose_u32(st, p.values, p.n_lines, p.n_values, counts)); }
+        CU(ctx, cudaStreamSynchronize(st));
+    }
+    if (p.n_lines > line_capacity) return fail(ctx, GATB_ERR_CAPACITY, "parse_counts: line table too small");
     return GATB_OK;
 }

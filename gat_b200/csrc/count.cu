@@ -750,15 +750,20 @@ __global__ void __launch_bounds__(STATS_COLS * STATS_ROWS) stats_select_kernel(S
     }
 }
 
+// T1 / T2: element types of the two matrices (uint32 or double); a uint32 converted to double is exact, so the
+// derived samples are those of the same values stored as float64
+template <typename T1, typename T2>
 __global__ void __launch_bounds__(256) compare_derive_kernel(CompareParams p)
 {
+    const T1 *__restrict__ m1 = reinterpret_cast<const T1 *>(p.m1);
+    const T2 *__restrict__ m2 = reinterpret_cast<const T2 *>(p.m2);
     const uint64_t total = p.n_samples * p.n_pairs;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t s = i / p.n_pairs;
         const uint32_t q = (uint32_t)(i % p.n_pairs);
         // same operation order as the numpy expressions: divide, add the fold pseudo-count, divide, log, shift
-        const double f1 = p.obs1[q] / (p.m1[s * p.n_cols1 + (uint32_t)p.col1[q]] + p.pseudo_count) + 0.0001;
-        const double f2 = p.obs2[q] / (p.m2[s * p.n_cols2 + (uint32_t)p.col2[q]] + p.pseudo_count) + 0.0001;
+        const double f1 = p.obs1[q] / ((double)m1[s * p.n_cols1 + (uint32_t)p.col1[q]] + p.pseudo_count) + 0.0001;
+        const double f2 = p.obs2[q] / ((double)m2[s * p.n_cols2 + (uint32_t)p.col2[q]] + p.pseudo_count) + 0.0001;
         p.out[i] = log(f1 / f2) + p.delta[q];
     }
 }
@@ -768,7 +773,10 @@ void launch_compare_derive(cudaStream_t st, const CompareParams &p)
     const uint64_t total = p.n_samples * p.n_pairs;
     if (total == 0) return;
     const unsigned blocks = (unsigned)std::min<uint64_t>((total + 255) / 256, 148u * 16u);
-    compare_derive_kernel<<<blocks, 256, 0, st>>>(p);
+    if (p.is_float1 && p.is_float2) compare_derive_kernel<double, double><<<blocks, 256, 0, st>>>(p);
+    else if (p.is_float1) compare_derive_kernel<double, uint32_t><<<blocks, 256, 0, st>>>(p);
+    else if (p.is_float2) compare_derive_kernel<uint32_t, double><<<blocks, 256, 0, st>>>(p);
+    else compare_derive_kernel<uint32_t, uint32_t><<<blocks, 256, 0, st>>>(p);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -818,6 +826,222 @@ void launch_format_counts(cudaStream_t st, const uint32_t *counts, uint64_t n_sa
     if (n_cols == 0) return;
     if (text == nullptr) format_counts_kernel<false><<<n_cols, 256, 0, st>>>(counts, n_samples, n_cols, col_len, col_off, text);
     else format_counts_kernel<true><<<n_cols, 256, 0, st>>>(counts, n_samples, n_cols, col_len, col_off, text);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// counts table parsing (gatb_parse_counts), the inverse of format_counts_kernel.  The body of a table is plain when
+// every line is   field \t field \t field \t D(,D)* \n   -- D = 1 to 10 digits of value <= 2^32 - 1, the same number of
+// D on every line, the last byte '\n' and no '\r' anywhere; the three leading fields may hold any other byte.
+// Anything else is reported as the offset of the first byte outside that grammar, never guessed at.
+//   tiles    CTA = tile of PARSE_TILE bytes: its '\n', '\t', ',' (and the first '\r'); a cub exclusive sum per
+//            kind then gives every tile the global index of its first line, tab and comma
+//   marks    per line: where its '\n' is, and the tabs and commas before it; at the line's third tab the start of
+//            its counts field and the commas before that.  The in-line index of a tab is (its global index) -
+//            3 * (its line): exact up to the first line with a tab count other than 3, so the first fourth tab is found
+//   lines    thread = line: exactly 3 tabs, and no fewer values than the first line
+//   values   thread = 16 bytes of a tile: checks every byte of the counts fields (digits, and ',' / '\n' only after a
+//            digit, and no comma that would start a value past the first line's number) and parses every number that STARTS in its bytes (reading up to 11 bytes past them).  Its
+//            value index in the line = the commas of the text before it - the commas before the counts field; it is
+//            stored row-major [line][value], so consecutive numbers go to consecutive addresses
+//   transpose  [line][value] -> [value][line] = [sample][column], the layout of the column statistics
+constexpr int PARSE_THREADS = 256, PARSE_BYTES = PARSE_TILE / PARSE_THREADS, PARSE_HALO = 16;
+static_assert(PARSE_BYTES == 16, "a thread reads its bytes of the staged tile as one uint4");
+
+__device__ __forceinline__ bool is_digit(uint8_t b) { return (uint8_t)(b - '0') < 10u; }
+
+// the tile's bytes [t0 - PARSE_HALO, t0 + PARSE_TILE + PARSE_HALO) into shared memory, 0 outside the text
+__device__ __forceinline__ void parse_stage(const ParseParams &p, uint64_t t0, uint8_t *s)
+{
+    for (uint32_t i = threadIdx.x; i < PARSE_TILE + 2 * PARSE_HALO; i += PARSE_THREADS) {
+        const uint64_t q = t0 + i - PARSE_HALO;       // (wraps past 0 for the first tile: >= n, so 0)
+        s[i] = q < p.n ? p.text[q] : 0;
+    }
+    __syncthreads();
+}
+
+// the thread's 16 bytes, and (tile counts before them, per kind) packed '\n' | '\t' << 21 | ',' << 42
+struct ParseBytes {
+    uint8_t b[PARSE_BYTES];
+    unsigned long long excl, total;
+};
+__device__ __forceinline__ unsigned long long parse_kinds(uint8_t c)
+{
+    return (c == '\n' ? 1ull : 0ull) | (c == '\t' ? 1ull << 21 : 0ull) | (c == ',' ? 1ull << 42 : 0ull);
+}
+__device__ __forceinline__ uint64_t kind_nl(unsigned long long v) { return v & 0x1fffffull; }
+__device__ __forceinline__ uint64_t kind_tab(unsigned long long v) { return (v >> 21) & 0x1fffffull; }
+__device__ __forceinline__ uint64_t kind_comma(unsigned long long v) { return v >> 42; }
+
+template <class Scan>
+__device__ __forceinline__ ParseBytes parse_bytes(const uint8_t *s, typename Scan::TempStorage &tmp)
+{
+    ParseBytes r;
+    const uint4 w = *reinterpret_cast<const uint4 *>(s + PARSE_HALO + threadIdx.x * PARSE_BYTES);
+    const uint32_t words[4] = {w.x, w.y, w.z, w.w};
+    unsigned long long mine = 0;
+    for (int i = 0; i < PARSE_BYTES; i++) {
+        r.b[i] = (uint8_t)(words[i >> 2] >> (8 * (i & 3)));
+        mine += parse_kinds(r.b[i]);
+    }
+    Scan(tmp).ExclusiveSum(mine, r.excl, r.total);
+    return r;
+}
+
+__global__ void __launch_bounds__(PARSE_THREADS) parse_tiles_kernel(ParseParams p)
+{
+    typedef cub::BlockScan<unsigned long long, PARSE_THREADS> Scan;
+    __shared__ typename Scan::TempStorage tmp;
+    __shared__ uint4 s16[(PARSE_TILE + 2 * PARSE_HALO) / 16];
+    uint8_t *s = reinterpret_cast<uint8_t *>(s16);
+    const uint64_t t0 = (uint64_t)blockIdx.x * PARSE_TILE;
+    parse_stage(p, t0, s);
+    const ParseBytes r = parse_bytes<Scan>(s, tmp);
+    for (int i = 0; i < PARSE_BYTES; i++)
+        if (r.b[i] == '\r') { atomicMin(p.bad, (unsigned long long)(t0 + threadIdx.x * PARSE_BYTES + i)); break; }
+    if (threadIdx.x == 0) {
+        p.tile_nl[blockIdx.x] = kind_nl(r.total);
+        p.tile_tab[blockIdx.x] = kind_tab(r.total);
+        p.tile_comma[blockIdx.x] = kind_comma(r.total);
+    }
+}
+
+__global__ void __launch_bounds__(PARSE_THREADS) parse_marks_kernel(ParseParams p)
+{
+    typedef cub::BlockScan<unsigned long long, PARSE_THREADS> Scan;
+    __shared__ typename Scan::TempStorage tmp;
+    __shared__ uint4 s16[(PARSE_TILE + 2 * PARSE_HALO) / 16];
+    uint8_t *s = reinterpret_cast<uint8_t *>(s16);
+    const uint64_t t0 = (uint64_t)blockIdx.x * PARSE_TILE;
+    parse_stage(p, t0, s);
+    const ParseBytes r = parse_bytes<Scan>(s, tmp);
+    uint64_t nl = p.tile_nl[blockIdx.x] + kind_nl(r.excl);          // line of the next byte
+    uint64_t tab = p.tile_tab[blockIdx.x] + kind_tab(r.excl);       // tabs / commas before it
+    uint64_t comma = p.tile_comma[blockIdx.x] + kind_comma(r.excl);
+    for (int i = 0; i < PARSE_BYTES; i++) {
+        const uint64_t q = t0 + threadIdx.x * PARSE_BYTES + i;
+        const uint8_t c = r.b[i];
+        if (q >= p.n || nl >= p.n_lines) break;     // (bytes after the last '\n': the values pass reports them)
+        if (c == '\n') {
+            p.line_end[nl] = q; p.tabs_end[nl] = tab; p.commas_end[nl] = comma;
+            nl++;
+        } else if (c == '\t') {
+            if (tab >= 3 * nl) {
+                const uint64_t k = tab - 3 * nl;
+                if (k == 2) { p.counts_start[nl] = q + 1; p.comma0[nl] = comma; }
+                else if (k > 2) atomicMin(p.bad, (unsigned long long)q);
+            }
+            tab++;
+        } else if (c == ',') comma++;
+    }
+}
+
+__global__ void __launch_bounds__(256) parse_lines_kernel(ParseParams p)
+{
+    const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (l >= p.n_lines) return;
+    const uint64_t tabs = p.tabs_end[l] - (l ? p.tabs_end[l - 1] : 0ull);
+    if (tabs < 3) { atomicMin(p.bad, p.line_end[l]); return; }           // the '\n' came before the third tab
+    if (tabs > 3 || p.counts_start[0] == PARSE_NONE || p.counts_start[l] == PARSE_NONE) return;    // reported elsewhere
+    // values = commas of the counts field + 1; a line with fewer values than the first: its '\n' (where a comma was
+    // due; one with more: its first extra comma, which the values pass reports)
+    if (p.commas_end[l] - p.comma0[l] < p.commas_end[0] - p.comma0[0]) atomicMin(p.bad, p.line_end[l]);
+}
+
+__global__ void __launch_bounds__(PARSE_THREADS) parse_values_kernel(ParseParams p)
+{
+    typedef cub::BlockScan<unsigned long long, PARSE_THREADS> Scan;
+    __shared__ typename Scan::TempStorage tmp;
+    __shared__ uint4 s16[(PARSE_TILE + 2 * PARSE_HALO) / 16];
+    uint8_t *s = reinterpret_cast<uint8_t *>(s16);
+    const uint64_t t0 = (uint64_t)blockIdx.x * PARSE_TILE;
+    parse_stage(p, t0, s);
+    const ParseBytes r = parse_bytes<Scan>(s, tmp);
+    uint64_t nl = p.tile_nl[blockIdx.x] + kind_nl(r.excl);
+    uint64_t comma = p.tile_comma[blockIdx.x] + kind_comma(r.excl);
+    uint64_t line = PARSE_NONE, cs = PARSE_NONE, c0 = 0;
+    unsigned long long bad = PARSE_NONE;
+    for (int i = 0; i < PARSE_BYTES; i++) {
+        const uint32_t j = PARSE_HALO + threadIdx.x * PARSE_BYTES + i;      // in s[]
+        const uint64_t q = t0 + threadIdx.x * PARSE_BYTES + i;
+        if (q >= p.n) break;
+        if (nl >= p.n_lines) { bad = min(bad, (unsigned long long)q); break; }      // a last line without '\n'
+        if (nl != line) { line = nl; cs = p.counts_start[nl]; c0 = p.comma0[nl]; }
+        const uint8_t c = r.b[i];
+        if (q >= cs) {
+            if (is_digit(c)) {
+                if (!is_digit(s[j - 1])) {              // a number starts: after the field's tab or a comma
+                    unsigned long long v = 0;
+                    uint32_t d = 0;
+                    while (d < 11u && is_digit(s[j + d])) { v = v * 10u + (uint32_t)(s[j + d] - '0'); d++; }
+                    if (d > 10u || v > 0xffffffffull) bad = min(bad, (unsigned long long)q);
+                    else if (p.values && comma - c0 < p.n_values) p.values[line * p.n_values + (comma - c0)] = (uint32_t)v;
+                }
+            } else if (!((c == ',' || c == '\n') && is_digit(s[j - 1])) ||
+                       (c == ',' && p.n_values && comma - c0 == p.n_values - 1))   // a value past the first line's last
+                bad = min(bad, (unsigned long long)q);
+        }
+        if (c == '\n') nl++;
+        else if (c == ',') comma++;
+    }
+    if (bad != PARSE_NONE) atomicMin(p.bad, bad);
+}
+
+size_t parse_scan_bytes(uint64_t n_tiles)
+{
+    size_t bytes = 0;
+    cub::DeviceScan::ExclusiveSum((void *)nullptr, bytes, (unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                  (int)(n_tiles + 1));
+    return bytes;
+}
+
+cudaError_t launch_parse_tiles(cudaStream_t st, const ParseParams &p, void *scan_tmp, size_t scan_bytes)
+{
+    if (p.n_tiles == 0) return cudaSuccess;
+    parse_tiles_kernel<<<(unsigned)p.n_tiles, PARSE_THREADS, 0, st>>>(p);
+    cudaError_t e = cudaGetLastError();
+    for (unsigned long long *t : {p.tile_nl, p.tile_tab, p.tile_comma})
+        if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, t, t, (int)(p.n_tiles + 1), st);
+    return e;
+}
+cudaError_t launch_parse_marks(cudaStream_t st, const ParseParams &p)
+{
+    if (p.n_tiles) parse_marks_kernel<<<(unsigned)p.n_tiles, PARSE_THREADS, 0, st>>>(p);
+    return cudaGetLastError();
+}
+cudaError_t launch_parse_lines(cudaStream_t st, const ParseParams &p)
+{
+    if (p.n_lines) parse_lines_kernel<<<(unsigned)((p.n_lines + 255) / 256), 256, 0, st>>>(p);
+    return cudaGetLastError();
+}
+cudaError_t launch_parse_values(cudaStream_t st, const ParseParams &p)
+{
+    if (p.n_tiles) parse_values_kernel<<<(unsigned)p.n_tiles, PARSE_THREADS, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
+// out[c][r] = in[r][c] through a 32 x 33 shared tile (both the reads and the writes coalesced); blockIdx.y strides over
+// the row tiles, so that any number of rows fits the grid
+__global__ void __launch_bounds__(256) transpose_u32_kernel(const uint32_t *__restrict__ in, uint64_t rows, uint64_t cols,
+                                                            uint32_t *__restrict__ out)
+{
+    __shared__ uint32_t t[32][33];
+    const uint64_t c0 = (uint64_t)blockIdx.x * 32u;
+    for (uint64_t r0 = (uint64_t)blockIdx.y * 32u; r0 < rows; r0 += (uint64_t)gridDim.y * 32u) {
+        for (uint32_t k = threadIdx.y; k < 32u; k += 8u)
+            if (r0 + k < rows && c0 + threadIdx.x < cols) t[k][threadIdx.x] = in[(r0 + k) * cols + c0 + threadIdx.x];
+        __syncthreads();
+        for (uint32_t k = threadIdx.y; k < 32u; k += 8u)
+            if (c0 + k < cols && r0 + threadIdx.x < rows) out[(c0 + k) * rows + r0 + threadIdx.x] = t[threadIdx.x][k];
+        __syncthreads();
+    }
+}
+
+cudaError_t launch_transpose_u32(cudaStream_t st, const uint32_t *in, uint64_t rows, uint64_t cols, uint32_t *out)
+{
+    if (rows == 0 || cols == 0) return cudaSuccess;
+    const dim3 grid((unsigned)((cols + 31) / 32), (unsigned)std::min<uint64_t>((rows + 31) / 32, 65535u));
+    transpose_u32_kernel<<<grid, dim3(32, 8), 0, st>>>(in, rows, cols, out);
+    return cudaGetLastError();
 }
 
 void launch_stats_pass1(cudaStream_t st, const StatsParams &p)

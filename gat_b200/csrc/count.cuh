@@ -156,7 +156,8 @@ struct StatsParams {
 //   out[s][p] = log((obs1[p] / (m1[s][col1[p]] + pc) + 1e-4) / (obs2[p] / (m2[s][col2[p]] + pc) + 1e-4)) + delta[p]
 // for pairs p0 <= p < p0 + n_pairs; out is [n_samples][n_pairs] float64, ready for the column statistics
 struct CompareParams {
-    const double *m1, *m2;          // [n_samples][n_cols1], [n_samples][n_cols2]
+    const void *m1, *m2;            // [n_samples][n_cols1], [n_samples][n_cols2]: uint32, or float64 where is_float
+    int is_float1, is_float2;
     uint32_t n_cols1, n_cols2;
     uint64_t n_samples;
     const int32_t *col1, *col2;     // [n_pairs] (already offset to the chunk)
@@ -171,6 +172,32 @@ void launch_compare_derive(cudaStream_t st, const CompareParams &p);
 // Pass 1 (text == NULL): col_len[a] = bytes of column a.  Pass 2: the bytes, column a at text + col_off[a].
 void launch_format_counts(cudaStream_t st, const uint32_t *counts, uint64_t n_samples, uint32_t n_cols,
                           unsigned long long *col_len, const unsigned long long *col_off, char *text);
+
+// counts table reader, the inverse of the formatter (count.cu, "counts table parsing"): the body of a table (the
+// bytes after the header line) -> uint32 [n_lines][n_values], then transposed to [n_values][n_lines]
+constexpr uint32_t PARSE_TILE = 4096;           // bytes per tile of the passes over the text
+constexpr unsigned long long PARSE_NONE = ~0ull;  // no offending byte / no counts field
+struct ParseParams {
+    const uint8_t *text;
+    uint64_t n;                     // bytes
+    uint64_t n_tiles;
+    // [n_tiles + 1] each: per tile '\n' / '\t' / ',' counts, then (cub exclusive sum) the counts before the tile
+    unsigned long long *tile_nl, *tile_tab, *tile_comma;
+    unsigned long long *bad;        // the offset of the first byte outside the grammar (atomicMin; PARSE_NONE: none)
+    uint64_t n_lines;               // '\n' of the text
+    // per line [n_lines]: offset of its '\n'; tabs / commas of the text before that '\n'; start of its counts field
+    // (PARSE_NONE until its third tab is seen) and the commas of the text before it
+    unsigned long long *line_end, *tabs_end, *commas_end, *counts_start, *comma0;
+    uint64_t n_values;              // values per line (the first line's)
+    uint32_t *values;               // [n_lines][n_values], or NULL: check the grammar only
+};
+size_t parse_scan_bytes(uint64_t n_tiles);
+// tile counts ('\r' is reported here), then their exclusive sums
+cudaError_t launch_parse_tiles(cudaStream_t st, const ParseParams &p, void *scan_tmp, size_t scan_bytes);
+cudaError_t launch_parse_marks(cudaStream_t st, const ParseParams &p);        // line ends, counts fields, 4th tabs
+cudaError_t launch_parse_lines(cudaStream_t st, const ParseParams &p);        // 3 tabs and n_values per line
+cudaError_t launch_parse_values(cudaStream_t st, const ParseParams &p);       // the numbers
+cudaError_t launch_transpose_u32(cudaStream_t st, const uint32_t *in, uint64_t rows, uint64_t cols, uint32_t *out);
 
 // K5 as HBM-bound streaming passes over a uint32 matrix (stats_stream.cu): TMA bulk copies of whole rows into a
 // shared-memory ring, thread = column

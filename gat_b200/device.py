@@ -195,22 +195,76 @@ class Context(object):
                                                _p(text), int(text.size)))
         return text[:int(off[-1])], off
 
+    def parse_counts(self, device_ptr, n_bytes, line_capacity, counts_ptr=None):
+        """the body of a counts table (device bytes after the header line) -> dict(n_rows, n_samples, plain, bad_offset,
+        lines uint64 [n_rows][2] = (start of the line, start of its counts field)); with counts_ptr (device, n_samples *
+        n_rows uint32) the [n_samples][n_rows] matrix too (gatb_parse_counts)"""
+        rows, samples, bad = ctypes.c_uint64(), ctypes.c_uint64(), ctypes.c_uint64()
+        plain = ctypes.c_int()
+        lines = np.zeros((max(int(line_capacity), 1), 2), dtype=np.uint64)
+        rc = self.lib.gatb_parse_counts(self.handle, ctypes.c_void_p(device_ptr), int(n_bytes), int(line_capacity),
+                                        ctypes.byref(rows), ctypes.byref(samples), ctypes.byref(plain), ctypes.byref(bad),
+                                        _p(lines), ctypes.c_void_p(counts_ptr) if counts_ptr else None)
+        if rc != _lib.ERR_CAPACITY:
+            self.check(rc)
+        return dict(n_rows=int(rows.value), n_samples=int(samples.value), plain=bool(plain.value),
+                    bad_offset=int(bad.value), lines=lines[:min(int(rows.value), int(line_capacity))])
+
     def compare_stats(self, m1, m2, col1, col2, obs1, obs2, delta, pseudo_count=1.0):
         """gat-compare's pairwise statistics (scripts/gat-compare.py:218-241, :300-323) for pairs
-        (column col1[q] of m1, column col2[q] of m2); m1, m2: [n_samples][n_cols] float64 sample matrices"""
-        m1 = np.ascontiguousarray(m1, dtype=np.float64)
-        m2 = m1 if m2 is None else np.ascontiguousarray(m2, dtype=np.float64)
-        if m1.shape[0] != m2.shape[0]:
+        (column col1[q] of m1, column col2[q] of m2).  m1, m2 (None: m1): [n_samples][n_cols] host float64 sample
+        matrices (gatb_compare_stats), or device matrices (gatb_compare_stats_device): a SampleMatrix whose samples
+        are still on the GPU, or (device pointer, n_samples, n_cols, is_float); a host matrix paired with a device one
+        is uploaded as float64"""
+        dev1 = _device_matrix(m1)
+        dev2 = dev1 if m2 is None else _device_matrix(m2)
+        staged = []
+        if (dev1 is None) != (dev2 is None):
+            # one table read on the GPU, the other by the host reader: the host matrix goes to the device as float64
+            # (what gatb_compare_stats would upload for it; uint32 -> double is exact, so the results do not change)
+            import torch
+            host = _host_samples(m1 if dev1 is None else m2)
+            staged.append(torch.from_numpy(np.ascontiguousarray(host, dtype=np.float64)).to(torch.device("cuda", self.device)))
+            torch.cuda.synchronize(self.device)
+            dev = (staged[0].data_ptr(), int(host.shape[0]), int(host.shape[1]), 1)
+            dev1, dev2 = (dev, dev2) if dev1 is None else (dev1, dev)
+        if dev1 is None:
+            m1 = np.ascontiguousarray(_host_samples(m1), dtype=np.float64)
+            m2 = m1 if m2 is None else np.ascontiguousarray(_host_samples(m2), dtype=np.float64)
+            (n1, k1), (n2, k2) = m1.shape, m2.shape
+        else:
+            (p1, n1, k1, f1), (p2, n2, k2, f2) = dev1, dev2
+        if n1 != n2:
             raise ValueError("sample matrices differ in the number of samples")
         c1 = np.ascontiguousarray(col1, dtype=np.int32)
         c2 = np.ascontiguousarray(col2, dtype=np.int32)
         arrs = [np.ascontiguousarray(x, dtype=np.float64) for x in (obs1, obs2, delta)]
         n = len(c1)
         outs = [np.zeros(n, dtype=np.float64) for _ in range(6)]
-        self.check(self.lib.gatb_compare_stats(self.handle, int(m1.shape[0]), _p(m1), int(m1.shape[1]), _p(m2),
-                                               int(m2.shape[1]), n, _p(c1), _p(c2), *[_p(a) for a in arrs],
-                                               float(pseudo_count), *[_p(o) for o in outs]))
+        if dev1 is None:
+            self.check(self.lib.gatb_compare_stats(self.handle, int(n1), _p(m1), int(k1), _p(m2), int(k2), n, _p(c1),
+                                                   _p(c2), *[_p(a) for a in arrs], float(pseudo_count),
+                                                   *[_p(o) for o in outs]))
+        else:
+            self.check(self.lib.gatb_compare_stats_device(self.handle, int(n1), ctypes.c_void_p(p1), int(f1), int(k1),
+                                                          ctypes.c_void_p(p2), int(f2), int(k2), n, _p(c1), _p(c2),
+                                                          *[_p(a) for a in arrs], float(pseudo_count),
+                                                          *[_p(o) for o in outs]))
         return dict(zip(["expected", "stddev", "lower95", "upper95", "fold", "pvalue"], outs))
+
+
+def _device_matrix(m):
+    """(device pointer, n_samples, n_cols, is_float) of a sample matrix on the GPU, else None (a host array, or a
+    SampleMatrix whose samples have already been copied to the host)"""
+    if isinstance(m, tuple):
+        return m
+    if getattr(m, "_tensor", None) is not None:
+        return m._tensor.data_ptr(), m.nsamples, m.ncolumns, 0 if m._as_uint32 else 1
+    return None
+
+
+def _host_samples(m):
+    return m.host() if hasattr(m, "host") else m
 
 
 class ColumnAccumulator(object):

@@ -20,6 +20,7 @@ import os
 
 import numpy as np
 
+from . import _lib
 from . import device as _dev
 from . import stats as Stats
 from .segmentlist import SegmentList
@@ -941,6 +942,65 @@ class SamplesNotKept(SampleMatrix):
                            "the statistics without the sample matrix); run with keep_samples=True to keep them")
 
     host = column = text = _refuse
+
+
+COUNTS_HEADER = b"track\tannotation\tobserved\tcounts\n"
+
+
+def readCountsTable(filename):
+    """a counts table (output_counts_pattern, gat/__init__.py:1091-1119) read on the GPU -> (rows, SampleMatrix):
+    rows[r] = (track, annotation, float(observed)) and column r of the uint32 [n_samples][n_rows] matrix, which stays
+    on the device.  None when the host reader has to decide: the header is not the plain one (the host reader raises
+    or reads it), the body is empty or not plain (gatb_parse_counts: float values, values >= 2^32, '\\r', a last line
+    without '\\n', empty lines, extra tabs, empty values or rows of different lengths), the text does not decode with
+    the codec of Python's text mode, or the text and the matrix do not fit in free device memory."""
+    import codecs
+    import gzip
+    import locale
+    import warnings
+    import torch
+    # the fields are decoded as text mode decodes them; only an ASCII-compatible codec leaves the digits, tabs and
+    # newlines of the body as the bytes the parser reads
+    encoding = locale.getpreferredencoding(False)
+    if codecs.lookup(encoding).name not in ("utf-8", "ascii"):
+        return None
+    with (gzip.open(filename, "rb") if filename.endswith(".gz") else open(filename, "rb")) as infile:
+        raw = infile.read()
+    if not raw.startswith(COUNTS_HEADER) or len(raw) == len(COUNTS_HEADER):
+        return None
+    body = np.frombuffer(raw, dtype=np.uint8, offset=len(COUNTS_HEADER))
+    ctx = getContext()
+    dev = torch.device("cuda", ctx.device)
+    n_lines = raw.count(b"\n", len(COUNTS_HEADER))
+    if body.size + 40 * n_lines > torch.cuda.mem_get_info(dev)[0]:
+        return None
+    # the checks of free memory come first; an allocation that still fails (the GPU is shared) takes the host path too
+    try:
+        with warnings.catch_warnings():             # (a read-only buffer: the tensor is only read, by the copy)
+            warnings.simplefilter("ignore")
+            text = torch.from_numpy(body).to(dev)
+        torch.cuda.synchronize(dev)
+        table = ctx.parse_counts(text.data_ptr(), body.size, n_lines)
+        if not table["plain"]:
+            return None
+        R, S = table["n_rows"], table["n_samples"]
+        # the matrix, and the row-major copy the parser transposes from
+        if 8 * R * S > torch.cuda.mem_get_info(dev)[0]:
+            return None
+        counts = torch.empty((S, R), dtype=torch.int32, device=dev)
+        ctx.parse_counts(text.data_ptr(), body.size, n_lines, counts_ptr=counts.data_ptr())
+    except torch.cuda.OutOfMemoryError:
+        return None
+    except _lib.GatB200Error as e:
+        if e.code == _lib.ERR_CUDA and "out of memory" in str(e):
+            return None
+        raise
+    del text
+    try:
+        fields = [body[a:b - 1].tobytes().decode(encoding).split("\t") for a, b in table["lines"].tolist()]
+    except UnicodeDecodeError:
+        return None
+    return [(track, annotation, float(observed)) for track, annotation, observed in fields], SampleMatrix(counts, True)
 
 
 class AnnotatorResult(object):

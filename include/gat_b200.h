@@ -369,6 +369,14 @@ int  gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const double *m1, int
                         const int32_t *col2, const double *obs1, const double *obs2, const double *delta,
                         double pseudo_count, double *expected, double *stddev, double *lower95,
                         double *upper95, double *fold, double *pvalue);
+/* gatb_compare_stats on DEVICE matrices: m1 / m2 [n_samples][n_cols] each uint32, or float64 where is_float (m2 may
+ * equal m1); all other arrays host, as above.  A uint32 converted to double is exact, so every output is bit-identical
+ * to gatb_compare_stats on the same values stored as float64. */
+int  gatb_compare_stats_device(gatb_ctx *ctx, uint64_t n_samples, const void *m1, int is_float1, int n_cols1,
+                               const void *m2, int is_float2, int n_cols2, uint64_t n_pairs, const int32_t *col1,
+                               const int32_t *col2, const double *obs1, const double *obs2, const double *delta,
+                               double pseudo_count, double *expected, double *stddev, double *lower95,
+                               double *upper95, double *fold, double *pvalue);
 
 /* ---- counts table: the text of --output-counts-pattern ------------------------------------------------
  * Replaces the Python loop of gat/__init__.py:1072-1086, which writes for every result
@@ -380,6 +388,25 @@ int  gatb_compare_stats(gatb_ctx *ctx, uint64_t n_samples, const double *m1, int
  * (col_off[n_cols] = bytes needed).  GATB_ERR_CAPACITY when capacity is too small (col_off is still filled). */
 int  gatb_format_counts(gatb_ctx *ctx, const uint32_t *counts, int counts_is_device, uint64_t n_samples,
                         int n_cols, uint64_t *col_off, char *text, uint64_t capacity);
+
+/* ---- counts table reader: --input-counts-file and gat-compare -------------------------------------------
+ * Replaces the Python loop of gat/__init__.py:1091-1119, which parses every number of a counts table with
+ *     numpy.array(list(map(float, counts.split(","))))
+ * text (device, n_bytes): the BODY of a table, the bytes after its header line.  Plain = every line is
+ *     field \t field \t field \t D(,D)* \n
+ * with D = 1 to 10 ASCII digits of value <= 2^32 - 1 (leading zeros allowed), the same number of D on every line,
+ * the last byte '\n' and no '\r' anywhere.  Line r is column r of the uint32 matrix counts[n_samples][n_rows] (the
+ * layout of gatb_column_stats).  Two calls, as gatb_format_counts:
+ *   counts == NULL: *n_rows, *n_samples, *plain and *bad_offset, the offset of the first byte outside the grammar
+ *       (UINT64_MAX when plain; for a line with fewer values than the first line, its '\n', for one with more, its first
+ *       extra comma), and for a
+ *       plain table lines[2 * r] = start of line r, lines[2 * r + 1] = start of its counts field (host, line_capacity
+ *       pairs; GATB_ERR_CAPACITY when there are more lines, the counts are still returned)
+ *   counts != NULL (device, n_samples * n_rows uint32, caller-allocated): the same, and the matrix; GATB_ERR_INVALID
+ *       when the text is not plain.
+ * An empty body is plain with no rows. */
+int  gatb_parse_counts(gatb_ctx *ctx, const char *text, uint64_t n_bytes, uint64_t line_capacity, uint64_t *n_rows,
+                       uint64_t *n_samples, int *plain, uint64_t *bad_offset, uint64_t *lines, uint32_t *counts);
 
 #ifdef __cplusplus
 }
