@@ -119,8 +119,9 @@ RunPlan = collections.namedtuple("RunPlan", "exchange transport matrix_free rows
 TrackSamples = collections.namedtuple("TrackSamples", "atracks planes gather")
 
 # the inputs of one run(): observed[counter_id] = {track: {annotation: count}}
+# (shard: None, or the (begin, end) sample range of a shard job)
 _Job = collections.namedtuple("_Job", "segments annotations workspace sampler counters observed reference num_samples "
-                                      "pseudo_count samples_pattern annos_cache")
+                                      "pseudo_count samples_pattern annos_cache shard")
 
 _STATS = ("expected", "stddev", "lower95", "upper95", "fold", "pvalue")
 
@@ -137,6 +138,21 @@ def run(segments, annotations, workspace, sampler, counters, workspace_generator
     same, but their samples cannot be asked for; None (default) does so only when the matrices would not fit in
     the free GPU memory and no counts table is written.
     """
+    return _onRunStream(_run, segments, annotations, workspace, sampler, counters, workspace_generator, **kwargs)
+
+
+def runShard(segments, annotations, workspace, sampler, counters, workspace_generator, sample_range, filename, **kwargs):
+    """one shard of a run: the global samples [begin, end) = sample_range of run(..., num_samples=...) with the same
+    arguments (kwargs of run()), written to `filename` as the exact integer state of every (track, counter) instead of
+    statistics (gat_b200/shards.py).  Shards of the same inputs and seed whose ranges tile [0, num_samples) merge, in
+    any order, into run()'s results bit for bit (mergeShards).  The run must be seeded (engine.seed): each shard
+    would otherwise draw a seed of its own.  On several ranks each rank samples its part of the range and rank 0
+    writes the file.  Returns None."""
+    _onRunStream(_run, segments, annotations, workspace, sampler, counters, workspace_generator,
+                 shard=(tuple(sample_range), filename), **kwargs)
+
+
+def _onRunStream(fn, *args, **kwargs):
     import torch
     # ONE CUDA stream for the whole run: the library's kernels, torch's tensor operations and the NCCL
     # collectives are all ordered on it (the library's own stream is non-blocking: it would not even wait for
@@ -147,14 +163,14 @@ def run(segments, annotations, workspace, sampler, counters, workspace_generator
     stream.wait_stream(torch.cuda.current_stream(dev))
     with torch.cuda.stream(stream):
         try:
-            return _run(segments, annotations, workspace, sampler, counters, workspace_generator, **kwargs)
+            return fn(*args, **kwargs)
         finally:
             torch.cuda.synchronize(dev)
             ctx.set_stream(None)
 
 
 def _planRun(num_samples, n_tracks, n_annotations, counter_names, counts_table, keep_samples, exchange, transport,
-             rank, world, free_bytes):
+             rank, world, free_bytes, sample_range=None, seeded=True):
     """how run() computes, from sizes alone (no I/O, no collective, no device query) -> RunPlan; every refusal of
     a bad argument is made here, alike on every rank and before the run's first collective.
 
@@ -167,8 +183,13 @@ def _planRun(num_samples, n_tracks, n_annotations, counter_names, counts_table, 
       collective per counter plane after the kernels.
     matrix_free: stream the samples through column accumulators instead of keeping the S x A matrices; exchange and
       transport do not apply then.  free_bytes (keep_samples=None only) differs between GPUs: run() makes them agree.
-    rows, columns: [begin, end) of this rank's global sample indices and of the annotation columns it holds"""
+    rows, columns: [begin, end) of this rank's global sample indices and of the annotation columns it holds.
+    sample_range: (begin, end) of a shard job (runShard): its rows are this rank's part of the range, always counted
+      by the matrix-free accumulators; seeded: a seed was set before the run (a shard must not draw its own)."""
     from . import parallel
+    if sample_range is not None:
+        return _planShard(num_samples, n_annotations, counter_names, counts_table, keep_samples, rank, world,
+                          sample_range, seeded)
     if exchange not in ("auto", "allgather", "columns"):
         raise ValueError("exchange must be auto, allgather or columns")
     if exchange == "auto":
@@ -189,12 +210,33 @@ def _planRun(num_samples, n_tracks, n_annotations, counter_names, counts_table, 
     return RunPlan(exchange, transport, matrix_free, parallel.shard_range(num_samples, rank, world), columns)
 
 
+def _planShard(num_samples, n_annotations, counter_names, counts_table, keep_samples, rank, world, sample_range,
+               seeded):
+    from . import parallel
+    begin, end = (int(x) for x in sample_range)
+    if counts_table:
+        raise ValueError("a shard job writes no counts table: output_counts_pattern needs every sample in one run")
+    if keep_samples:
+        raise ValueError("a shard job keeps no samples: keep_samples=True is refused")
+    if not 0 <= begin < end <= num_samples < (1 << 32):
+        raise ValueError("sample_range (%i, %i) must satisfy 0 <= begin < end <= num_samples (%i) < 2^32"
+                         % (begin, end, num_samples))
+    if "nucleotide-density" in counter_names:
+        raise NotImplementedError("nucleotide-density has no shard mode (float64 samples have no exact split)")
+    if not seeded:
+        raise ValueError("a shard job needs a seeded run (engine.seed, --random-seed): every shard must place the "
+                         "same samples")
+    b, e = parallel.shard_range(end - begin, rank, world)
+    return RunPlan("allgather", "nccl", True, (begin + b, begin + e), (0, n_annotations))
+
+
 def _columnRange(exchange, n_annotations, rank, world):
     from . import parallel
     return parallel.column_range(n_annotations, rank, world) if exchange == "columns" else (0, n_annotations)
 
 
-def _run(segments, annotations, workspace, sampler, counters, workspace_generator, **kwargs):
+def _run(segments, annotations, workspace, sampler, counters, workspace_generator, shard=None, **kwargs):
+    """run() -> results; runShard() (shard = (sample_range, filename)) -> None, the shard file written"""
     from . import parallel
     import torch
     num_samples = kwargs.get("num_samples", 10000)
@@ -225,18 +267,20 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
                                      annos_cache=annos_cache) for c in counters]
     mark("observed")
     job = _Job(segments, annotations, workspace, sampler, counters, observed, kwargs.get("reference", None),
-               num_samples, kwargs.get("pseudo_count", 1.0), kwargs.get("output_samples_pattern", None), annos_cache)
+               num_samples, kwargs.get("pseudo_count", 1.0), kwargs.get("output_samples_pattern", None), annos_cache,
+               None if shard is None else shard[0])
 
     free_bytes = torch.cuda.mem_get_info(ctx.device)[0] if keep_samples is None else 0
     n_annotations = len(list(annotations.tracks))
     plan = _planRun(num_samples, len(segments.tracks), n_annotations, [c.name for c in counters],
                     bool(output_counts_pattern), keep_samples,
                     kwargs.get("exchange", os.environ.get("GATB_EXCHANGE", "auto")),
-                    kwargs.get("transport", os.environ.get("GATB_TRANSPORT", "peer")), rank, world, free_bytes)
+                    kwargs.get("transport", os.environ.get("GATB_TRANSPORT", "peer")), rank, world, free_bytes,
+                    sample_range=job.shard, seeded=Engine._rng_state["seed"] is not None)
     # every rank must place with the SAME seed (the matrix is keyed by seed and global sample index): an
     # unseeded run draws its seed on rank 0 and broadcasts it
     parallel.share_seed()
-    if keep_samples is None and world > 1:
+    if keep_samples is None and world > 1 and shard is None:
         plan = plan._replace(matrix_free=any(matrixfree.allgather(plan.matrix_free, world)))
 
     # (torch's legacy default stream has handle 0 = "the library's own stream" at the C ABI: pass cudaStreamLegacy)
@@ -251,6 +295,14 @@ def _run(segments, annotations, workspace, sampler, counters, workspace_generato
     for a in annos_cache.values():
         a.close()
     mark("overlap columns")
+    if shard is not None:
+        if rank == 0:
+            from . import shards
+            shards.writeShard(shard[1], job, sampled, sizes)
+        mark("shard file")
+        if seconds is not None and rank == 0:
+            sys.stderr.write("# gat_b200.runShard phases: " + ", ".join("%s %.3fs" % p for p in seconds.items()) + "\n")
+        return None
 
     # statistics per (counter, track): one batched column-stats call over all annotations
     results = []
@@ -286,7 +338,7 @@ def _peerMatrix(plan, n_counters, num_samples):
 def _matrixFreeSlab(n_counters, n_annotations, plan):
     """the one device buffer every slab of the matrix-free mode is counted into -> (int32 tensor, rows per slab)"""
     import torch
-    matrixfree.info.update(reruns=0, arena_bytes=0, chunk_rows=0)
+    matrixfree.info.update(reruns=0, arena_bytes=0, chunk_rows=0, pass2_seconds=0.0)
     n_local = plan.rows[1] - plan.rows[0]
     chunk = max(1, min(max(n_local, 1), matrixfree.SLAB_BYTES // (4 * n_counters * max(n_annotations, 1))))
     return torch.zeros(n_counters * chunk * max(n_annotations, 1), dtype=torch.int32, device=getContext().device), chunk
@@ -383,7 +435,8 @@ def _exchange(out_u, out_f, peer, plan, num_samples):
 
 def _streamTrack(ntrack, track, smp, annos, names, atracks, job, plan, slab):
     """the matrix-free mode: this rank's samples in slabs of one reused device buffer, counted into column
-    accumulators and overwritten -> [statistics dict per counter], complete (summed over the ranks)"""
+    accumulators and overwritten -> [statistics dict per counter], complete (summed over the ranks); in a shard job
+    [integer state per counter] of the shard's rows (matrixfree.shard_states)"""
     from . import parallel
     buf, chunk = slab
     begin, end = plan.rows
@@ -397,6 +450,9 @@ def _streamTrack(ntrack, track, smp, annos, names, atracks, job, plan, slab):
 
     rank, world = parallel.rank_world()
     planes = [_observed(job, counter_id, track, atracks) for counter_id in range(len(names))]
+    if job.shard is not None:
+        return matrixfree.shard_states(getContext(), produce, planes, job.num_samples, end - begin, len(atracks), chunk,
+                                       rank=rank, world=world)
     return matrixfree.stream_statistics(getContext(), produce, planes, job.num_samples, end - begin, len(atracks), chunk,
                                         pseudo_count=job.pseudo_count, rank=rank, world=world)
 
@@ -542,3 +598,4 @@ def _fromCountsHost(filename):
 
 
 from .cli import buildParser  # noqa: E402  (flags of gat.buildParser, gat/__init__.py:54-429)
+from .shards import mergeShards  # noqa: E402

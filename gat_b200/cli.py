@@ -5,6 +5,10 @@
         [--isochore-file=i.bed] [--counter=nucleotide-overlap] [--num-samples=1000] [--sampler=annotator]
 
 Multi-GPU: launch with `python -m torch.distributed.run --nproc-per-node N -m gat_b200.cli ...`.
+
+A run in several jobs: `--random-seed=S --sample-range=BEGIN:END --output-shard=FILE` samples only the global samples
+[BEGIN, END) of the run and writes their exact state to FILE instead of a table; `python -m gat_b200.shards FILE...`
+merges the shards of ranges that tile [0, --num-samples) into the run's table (gat_b200/shards.py).
 """
 import optparse
 import random
@@ -142,8 +146,9 @@ def buildParser(usage=None):
     return parser
 
 
-def fromSegments(options, log=None):
-    """load, prepare and run (scripts/gat-run.py:77-220)"""
+def fromSegments(options, log=None, shard=None):
+    """load, prepare and run (scripts/gat-run.py:77-220); shard = ((begin, end), filename): write the shard of that
+    sample range instead (gat_b200.runShard) -> None"""
     import gat_b200
     from . import io as IO
     from . import engine as Engine
@@ -171,12 +176,15 @@ def fromSegments(options, log=None):
     t0 = time.time()
     if log:
         log("sampling started")
-    results = gat_b200.run(segments, annotations, workspace, sampler, counters,
-                           workspace_generator=Engine.UnconditionalWorkspace(),
-                           num_samples=options.num_samples,
-                           output_counts_pattern=options.output_counts_pattern,
-                           output_samples_pattern=options.output_samples_pattern,
-                           reference=options.reference, pseudo_count=options.pseudo_count)
+    kwargs = dict(num_samples=options.num_samples, output_counts_pattern=options.output_counts_pattern,
+                  output_samples_pattern=options.output_samples_pattern, reference=options.reference,
+                  pseudo_count=options.pseudo_count)
+    if shard is not None:
+        results = gat_b200.runShard(segments, annotations, workspace, sampler, counters,
+                                    Engine.UnconditionalWorkspace(), shard[0], shard[1], **kwargs)
+    else:
+        results = gat_b200.run(segments, annotations, workspace, sampler, counters,
+                               workspace_generator=Engine.UnconditionalWorkspace(), **kwargs)
     if log:
         log("sampling completed in %.2f seconds" % (time.time() - t0))
     return results
@@ -192,7 +200,13 @@ def main(argv=None):
     parser = buildParser(usage=__doc__)
     parser.add_option("-v", "--verbose", dest="loglevel", type="int", default=1, help="log level")
     parser.add_option("-S", "--stdout", dest="stdout_file", type="string", default=None, help="output file")
+    parser.add_option("--sample-range", dest="sample_range", type="string", default=None,
+                      help="BEGIN:END -- sample only the global samples [BEGIN, END) of the run and write them to "
+                           "--output-shard (needs --random-seed); merge the shards with python -m gat_b200.shards")
+    parser.add_option("--output-shard", dest="output_shard", type="string", default=None,
+                      help="shard file written by a --sample-range job")
     options, _ = parser.parse_args(argv[1:])
+    shard = _shardOption(options)
     parallel.init_from_env()
     import os
     if os.environ.get("GATB_TRANSPORT", "peer") == "nccl":
@@ -219,6 +233,12 @@ def main(argv=None):
         raise NotImplementedError("--null is read by the reference from a results table; pass `reference` to run()")
     options.reference = None
 
+    if shard is not None:
+        fromSegments(options, log, shard)
+        if options.stdout_file:
+            options.stdout.close()
+        parallel.finalize()
+        return 0
     if options.input_filename_counts:
         results = gat_b200.fromCounts(options.input_filename_counts)
     else:
@@ -234,6 +254,23 @@ def main(argv=None):
         options.stdout.close()
     parallel.finalize()
     return 0
+
+
+def _shardOption(options):
+    """--sample-range / --output-shard -> None or ((begin, end), filename)"""
+    if options.sample_range is None and options.output_shard is None:
+        return None
+    if options.sample_range is None or options.output_shard is None:
+        raise ValueError("--sample-range and --output-shard go together")
+    if options.random_seed is None:
+        raise ValueError("--sample-range needs --random-seed: every shard of a run must place the same samples")
+    if options.input_filename_counts:
+        raise ValueError("--sample-range samples the run: it cannot start from --input-counts-file")
+    try:
+        begin, end = (int(x) for x in options.sample_range.split(":"))
+    except ValueError:
+        raise ValueError("--sample-range must be BEGIN:END, got %r" % options.sample_range)
+    return (begin, end), options.output_shard
 
 
 if __name__ == "__main__":

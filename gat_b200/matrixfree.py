@@ -9,6 +9,8 @@ rank falls outside its window is counted again over [min, max] of the column: ev
 (seed, track, unit, global sample index), so the second pass sees the same values.  The results are the
 matrix path's, bit for bit; the device memory is one slab plus the windows, whatever S is.
 """
+import time
+
 import numpy as np
 
 from . import device
@@ -17,8 +19,9 @@ SLAB_BYTES = 512 << 20          # one slab of [counters][rows][columns] uint32
 ARENA_FRACTION = 0.25           # histogram windows of one track may take this share of the free device memory
 PILOT_WINDOW = None             # (tests) every pilot window this many bins wide, to force the second pass
 
-# what the last matrix-free run did (per process): second passes, largest arena of one track, rows per slab
-info = dict(reruns=0, arena_bytes=0, chunk_rows=0)
+# what the last matrix-free run did (per process): second sampling passes, largest arena of one track, rows per slab,
+# seconds of the shard jobs' histogram passes
+info = dict(reruns=0, arena_bytes=0, chunk_rows=0, pass2_seconds=0.0)
 
 
 def use_matrix_free(keep_samples, counts_table, density, matrix_bytes, free_bytes):
@@ -68,6 +71,18 @@ def _merge_ranks(accs, world, rank, sums):
                 a.merge(s, sums=sums)
 
 
+def _slabs(produce, start, n_local, chunk):
+    for r0 in range(start, n_local, chunk):
+        n = min(chunk, n_local - r0)
+        yield n, produce(r0, n)
+
+
+def _count(accs, n, ptr, n_cols, sums, hist):
+    """slab [planes][n][n_cols] at ptr into the accumulators of the planes"""
+    for i, a in enumerate(accs):
+        a.add(ptr + 4 * i * n * n_cols, n, n_cols, sums=sums, hist=hist)
+
+
 def _set_windows(accs, lo, hi, budget_bytes, what):
     width = [np.where(h >= l, h - l + 1, 0).astype(np.uint64) for l, h in zip(lo, hi)]
     arena = 4 * int(sum(int(w.sum()) for w in width))
@@ -102,11 +117,6 @@ def _stream(ctx, accs, produce, n_local, n_cols, chunk, pseudo_count, budget_byt
     chunk = max(1, min(chunk, n_local)) if n_local else 1
     info["chunk_rows"] = chunk
 
-    def slabs(start):
-        for r0 in range(start, n_local, chunk):
-            n = min(chunk, n_local - r0)
-            yield n, produce(r0, n)
-
     # pilot: the first slab of this rank; every rank takes the union of all ranks' windows
     lo = [np.full(n_cols, np.iinfo(np.int64).max, dtype=np.int64) for _ in range(P)]
     hi = [np.full(n_cols, -1, dtype=np.int64) for _ in range(P)]
@@ -125,14 +135,10 @@ def _stream(ctx, accs, produce, n_local, n_cols, chunk, pseudo_count, budget_byt
             hi[i] = np.maximum(hi[i], other[1][i])
     _set_windows(accs, lo, hi, budget_bytes, "pilot")
 
-    def count(n, ptr, sums):
-        for i, a in enumerate(accs):
-            a.add(ptr + 4 * i * n * n_cols, n, n_cols, sums=sums, hist=True)
-
     if n0:
-        count(n0, ptr0, True)
-    for n, ptr in slabs(n0):
-        count(n, ptr, True)
+        _count(accs, n0, ptr0, n_cols, True, True)
+    for n, ptr in _slabs(produce, n0, n_local, chunk):
+        _count(accs, n, ptr, n_cols, True, True)
     _merge_ranks(accs, world, rank, sums=True)
     results = [a.finish(pseudo_count) for a in accs]
     if not any(m.any() for _, m in results):
@@ -146,8 +152,8 @@ def _stream(ctx, accs, produce, n_local, n_cols, chunk, pseudo_count, budget_byt
         lo2.append(np.where(m, minmax[0], 0))
         hi2.append(np.where(m, minmax[1], -1))
     _set_windows(accs, lo2, hi2, budget_bytes, "second-pass")
-    for n, ptr in slabs(0):
-        count(n, ptr, False)
+    for n, ptr in _slabs(produce, 0, n_local, chunk):
+        _count(accs, n, ptr, n_cols, False, True)
     _merge_ranks(accs, world, rank, sums=False)
     out = []
     for a, (st, m) in zip(accs, results):
@@ -158,3 +164,109 @@ def _stream(ctx, accs, produce, n_local, n_cols, chunk, pseudo_count, budget_byt
             st[k] = np.where(m, st2[k], st[k])
         out.append(st)
     return out
+
+
+# ------------------------------------------------------------------------------------------------ shards
+# A shard job (gat_b200.runShard) counts a range of the global samples and keeps the exact integers instead of the
+# statistics: the sums of the range and the histogram of every column over the column's whole [min, max] in the
+# range.  Integers add across any split of the samples, and a histogram over [min, max] holds every rank, so shards
+# of the same run merge into its statistics bit for bit, without sampling again and without agreeing on windows.
+
+def shard_states(ctx, produce, planes, n_samples, n_local, n_cols, chunk, budget_bytes=None, rank=0, world=1):
+    """the integer state of this shard's rows of all ranks, for len(planes) uint32 counter planes whose rows are
+    produced in slabs (produce, planes, chunk as in stream_statistics).  Pass 1 counts the sums; pass 2 counts the
+    histograms over the [min, max] of every column, from the slab still in the buffer when the rank's rows fit in
+    one slab, else sampled again.  -> [dict(rows, moments [5][A], minmax [2][A], col_ptr int64 [A+1], value uint32,
+    count uint64) per plane]: the gatb_colacc_state layout, the histogram as sparse CSR per column (sparse_histogram)."""
+    if budget_bytes is None:
+        import torch
+        budget_bytes = int(ARENA_FRACTION * torch.cuda.mem_get_info(ctx.device)[0])
+    accs = [device.ColumnAccumulator(ctx, n_cols, n_samples, obs, ref) for obs, ref in planes]
+    try:
+        chunk = max(1, min(chunk, n_local)) if n_local else 1
+        info["chunk_rows"] = chunk
+        ptr = None
+        for n, ptr in _slabs(produce, 0, n_local, chunk):
+            _count(accs, n, ptr, n_cols, True, False)
+        _merge_ranks(accs, world, rank, sums=True)
+        states = [a.state() for a in accs]
+        t0 = time.perf_counter()
+        lo = [st["minmax"][0].astype(np.int64) for st in states]
+        hi = [st["minmax"][1].astype(np.int64) for st in states]
+        _set_windows(accs, lo, hi, budget_bytes, "shard")
+        if n_local and n_local <= chunk:
+            _count(accs, n_local, ptr, n_cols, False, True)
+        elif n_local:
+            info["reruns"] += 1
+            for n, p in _slabs(produce, 0, n_local, chunk):
+                _count(accs, n, p, n_cols, False, True)
+        _merge_ranks(accs, world, rank, sums=False)
+        out = []
+        for a, st, l in zip(accs, states, lo):
+            bins = a.state()
+            if bins["outside"].any():
+                raise RuntimeError("shard: a value fell outside the [min, max] window of its column")
+            col_ptr, value, count = sparse_histogram(bins["bins"], l, st["minmax"][1].astype(np.int64) - l + 1)
+            out.append(dict(rows=st["rows"], moments=st["moments"], minmax=st["minmax"], col_ptr=col_ptr, value=value,
+                            count=count))
+        info["pass2_seconds"] += time.perf_counter() - t0
+        return out
+    finally:
+        for a in accs:
+            a.close()
+
+
+def sparse_histogram(bins, lo, width):
+    """dense unit-width bins of the windows [lo[a], lo[a] + width[a]) of every column, one after the other ->
+    (col_ptr int64 [A+1], value uint32, count uint64): the non-zero bins of column a are entries col_ptr[a] ..
+    col_ptr[a+1] - 1, in increasing value"""
+    width = np.asarray(width, dtype=np.int64)
+    off = np.concatenate([[0], np.cumsum(width)])
+    bins = np.asarray(bins)[:int(off[-1])]
+    nz = np.flatnonzero(bins)
+    col = np.searchsorted(off, nz, side="right") - 1
+    col_ptr = np.searchsorted(col, np.arange(len(width) + 1), side="left").astype(np.int64)
+    value = (np.asarray(lo, dtype=np.int64)[col] + (nz - off[col])).astype(np.uint32)
+    return col_ptr, value, bins[nz].astype(np.uint64)
+
+
+def rebase_histogram(col_ptr, value, count, lo, width):
+    """a sparse histogram (sparse_histogram) -> the dense uint32 bins of the windows [lo[a], lo[a] + width[a]), which
+    must hold its values"""
+    lo = np.asarray(lo, dtype=np.int64)
+    width = np.asarray(width, dtype=np.int64)
+    off = np.concatenate([[0], np.cumsum(width)])
+    col = np.repeat(np.arange(len(width)), np.diff(np.asarray(col_ptr, dtype=np.int64)))
+    pos = np.asarray(value, dtype=np.int64) - lo[col]
+    if len(pos) and ((pos < 0) | (pos >= width[col])).any():
+        raise ValueError("histogram values outside the windows they are rebased into")
+    bins = np.zeros(max(int(off[-1]), 1), dtype=np.uint32)
+    bins[off[col] + pos] = np.asarray(count, dtype=np.uint64)
+    return bins
+
+
+def merge_shard_states(ctx, n_samples, observed, ref_fold, states, pseudo_count=1.0, budget_bytes=None):
+    """the statistics of one counter plane from the shard_states of shards whose rows together are all n_samples
+    samples -> statistics dict as Context.column_stats returns it.  One accumulator with the windows [min, max] of
+    the union of the shards; every shard's histogram rebased into them and its integers added (gatb_colacc_merge:
+    the 128-bit sum of squares with its carry)."""
+    A = len(observed)
+    if budget_bytes is None:
+        import torch
+        budget_bytes = int(ARENA_FRACTION * torch.cuda.mem_get_info(ctx.device)[0])
+    acc = device.ColumnAccumulator(ctx, A, n_samples, observed, ref_fold)
+    try:
+        lo = np.min([st["minmax"][0] for st in states], axis=0).astype(np.int64)
+        hi = np.max([st["minmax"][1] for st in states], axis=0).astype(np.int64)
+        _set_windows([acc], [lo], [hi], budget_bytes, "merge")
+        outside = np.zeros((2, A), dtype=np.uint64)
+        for st in states:
+            acc.merge(dict(rows=int(st["rows"]), moments=np.ascontiguousarray(st["moments"], dtype=np.uint64),
+                           minmax=np.ascontiguousarray(st["minmax"], dtype=np.uint32), outside=outside,
+                           bins=rebase_histogram(st["col_ptr"], st["value"], st["count"], lo, hi - lo + 1)))
+        stats, missed = acc.finish(pseudo_count)
+        if missed.any():
+            raise RuntimeError("shard merge: a CI rank missed the [min, max] window of its column")
+        return stats
+    finally:
+        acc.close()
