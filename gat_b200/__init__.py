@@ -598,4 +598,4 @@ def _fromCountsHost(filename):
 
 
 from .cli import buildParser  # noqa: E402  (flags of gat.buildParser, gat/__init__.py:54-429)
-from .shards import mergeShards  # noqa: E402
+from .shards import combineShards, mergeShardPrefix, mergeShards  # noqa: E402

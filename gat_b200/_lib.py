@@ -29,7 +29,7 @@ SYMBOLS = [
     "gatb_annotations_create_from_lists",
     "gatb_set_output_routes", "gatb_set_route_mode", "gatb_peer_alloc", "gatb_peer_free", "gatb_peer_open", "gatb_peer_close",
     "gatb_colacc_create", "gatb_colacc_set_windows", "gatb_colacc_add", "gatb_colacc_state", "gatb_colacc_merge",
-    "gatb_colacc_finish", "gatb_colacc_destroy",
+    "gatb_colacc_finish", "gatb_colacc_destroy", "gatb_colacc_export", "gatb_colacc_add_sparse",
 ]
 
 COLACC_SUMS, COLACC_HIST = 1, 2
@@ -182,6 +182,10 @@ def bind(L):
     L.gatb_colacc_merge.argtypes = [vp, u64, vp, vp, vp, vp]
     L.gatb_colacc_finish.restype = i32
     L.gatb_colacc_finish.argtypes = [vp, dbl, vp, vp, vp, vp, vp, vp, vp]
+    L.gatb_colacc_export.restype = i32
+    L.gatb_colacc_export.argtypes = [vp, vp, vp, vp, u64]
+    L.gatb_colacc_add_sparse.restype = i32
+    L.gatb_colacc_add_sparse.argtypes = [vp, vp, vp, vp]
     L.gatb_colacc_destroy.restype = None
     L.gatb_colacc_destroy.argtypes = [vp]
     return L

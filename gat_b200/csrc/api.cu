@@ -1941,9 +1941,11 @@ extern "C" int gatb_colacc_merge(gatb_colacc *c, uint64_t rows, const uint64_t *
     gatb_ctx *ctx = c->ctx;
     const size_t A = c->A;
     if (c->sums.rows + rows > c->l) return fail(ctx, GATB_ERR_INVALID, "colacc_merge: more rows than n_samples_total");
-    std::vector<uint64_t> o(2 * A);
-    std::vector<uint32_t> b(c->n_bins);
-    if (const int rc = gatb_colacc_state(c, nullptr, nullptr, nullptr, o.data(), b.data())) return rc;
+    // (only the parts given come down to the host: a merge of the sums alone does not move the arena)
+    std::vector<uint64_t> o(outside ? 2 * A : 0);
+    std::vector<uint32_t> b(bins ? c->n_bins : 0);
+    if (const int rc = gatb_colacc_state(c, nullptr, nullptr, nullptr, outside ? o.data() : nullptr,
+                                         bins ? b.data() : nullptr)) return rc;
     if (const int rc = c->sums.merge(rows, moments, minmax)) return rc;
     cudaStream_t st = ctx->stream;
     if (outside) {
@@ -1955,6 +1957,86 @@ extern "C" int gatb_colacc_merge(gatb_colacc *c, uint64_t rows, const uint64_t *
         CU(ctx, cudaMemcpyAsync(c->bins.p, b.data(), c->n_bins * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     }
     CU(ctx, cudaStreamSynchronize(st));
+    return GATB_OK;
+}
+
+static ColSparseParams sparse_params(gatb_colacc *c)
+{
+    ColSparseParams p;
+    memset(&p, 0, sizeof(p));
+    p.n_cols = c->A; p.lo = c->win.p; p.width = c->win.p + c->A; p.bin_off = c->bin_off.p; p.bins = c->bins.p;
+    return p;
+}
+
+// the windows' non-zero bins as CSR, compacted on the device: only the sparse arrays come to the host
+extern "C" int gatb_colacc_export(gatb_colacc *c, int64_t *col_ptr, uint32_t *value, uint64_t *count, uint64_t capacity)
+{
+    if (!c || !col_ptr || (!value) != (!count)) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const uint32_t A = c->A;
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    ColSparseParams p = sparse_params(c);
+    DevBuf<unsigned long long> d_nnz;
+    CU(ctx, d_nnz.alloc(A));
+    p.nnz = d_nnz.p;
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_export(st, p, false)); }
+    std::vector<unsigned long long> nnz(A);
+    CU(ctx, cudaMemcpyAsync(nnz.data(), d_nnz.p, A * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    col_ptr[0] = 0;
+    for (uint32_t a = 0; a < A; a++) col_ptr[a + 1] = col_ptr[a] + (int64_t)nnz[a];
+    const uint64_t n = (uint64_t)col_ptr[A];
+    if (!value || n == 0) return GATB_OK;
+    if (capacity < n)
+        return fail(ctx, GATB_ERR_CAPACITY, "colacc_export: " + std::to_string(n) + " non-zero bins, capacity " +
+                                                std::to_string(capacity));
+    DevBuf<long long> d_ptr;
+    DevBuf<uint32_t> d_value;
+    DevBuf<unsigned long long> d_count;
+    CU(ctx, d_ptr.upload((const long long *)col_ptr, (size_t)A + 1, st));
+    CU(ctx, d_value.alloc(n));
+    CU(ctx, d_count.alloc(n));
+    p.col_ptr = d_ptr.p; p.value = d_value.p; p.count = d_count.p;
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_export(st, p, true)); }
+    CU(ctx, cudaMemcpyAsync(value, d_value.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaMemcpyAsync(count, d_count.p, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    return GATB_OK;
+}
+
+extern "C" int gatb_colacc_add_sparse(gatb_colacc *c, const int64_t *col_ptr, const uint32_t *value, const uint64_t *count)
+{
+    if (!c || !col_ptr) return GATB_ERR_INVALID;
+    gatb_ctx *ctx = c->ctx;
+    const uint32_t A = c->A;
+    if (col_ptr[0] != 0) return fail(ctx, GATB_ERR_INVALID, "colacc_add_sparse: col_ptr[0] is not 0");
+    for (uint32_t a = 0; a < A; a++)
+        if (col_ptr[a + 1] < col_ptr[a]) return fail(ctx, GATB_ERR_INVALID, "colacc_add_sparse: col_ptr decreases");
+    const uint64_t n = (uint64_t)col_ptr[A];
+    if (n == 0) return GATB_OK;
+    if (!value || !count) return GATB_ERR_INVALID;
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_stream = ctx->stream;
+    cudaStream_t st = ctx->stream;
+    ColSparseParams p = sparse_params(c);
+    DevBuf<long long> d_ptr;
+    DevBuf<uint32_t> d_value, d_error;
+    DevBuf<unsigned long long> d_count;
+    CU(ctx, d_ptr.upload((const long long *)col_ptr, (size_t)A + 1, st));
+    CU(ctx, d_value.upload(value, n, st));
+    CU(ctx, d_count.upload((const unsigned long long *)count, n, st));
+    CU(ctx, d_error.alloc(1));
+    CU(ctx, cudaMemsetAsync(d_error.p, 0, sizeof(uint32_t), st));
+    p.col_ptr = d_ptr.p; p.value = d_value.p; p.count = d_count.p; p.n_entries = n; p.error = d_error.p;
+    uint32_t error = 0;
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_add_sparse(st, p, false)); }
+    CU(ctx, cudaMemcpyAsync(&error, d_error.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(ctx, cudaStreamSynchronize(st));
+    if (error) return fail(ctx, GATB_ERR_RANGE, "colacc_add_sparse: a histogram value lies outside the window of its "
+                                                "column, or a count is 2^32 or more");
+    { ProfScope ps(ctx, PROF_OTHER); CU(ctx, launch_colacc_add_sparse(st, p, true)); }
     return GATB_OK;
 }
 

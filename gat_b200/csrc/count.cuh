@@ -251,6 +251,23 @@ struct ColHistParams {
 cudaError_t launch_colacc_hist(cudaStream_t st, const ColHistParams &p, int sm_count);
 cudaError_t launch_colacc_pick(cudaStream_t st, const ColHistParams &p);
 
+// The windows' histograms as sparse CSR (gatb_colacc_export / gatb_colacc_add_sparse): entries col_ptr[a] ..
+// col_ptr[a + 1] - 1 are the non-zero bins of column a in increasing value.
+struct ColSparseParams {
+    uint32_t n_cols;
+    const uint32_t *lo, *width;
+    const unsigned long long *bin_off;
+    uint32_t *bins;
+    unsigned long long *nnz;        // export, count pass: out [n_cols], the non-zero bins of every column
+    const long long *col_ptr;       // [n_cols + 1]
+    uint32_t *value;                // export: out; add_sparse: in
+    unsigned long long *count;
+    uint64_t n_entries;             // add_sparse: col_ptr[n_cols]
+    uint32_t *error;                // add_sparse check: set when a value lies outside its window or a count >= 2^32
+};
+cudaError_t launch_colacc_export(cudaStream_t st, const ColSparseParams &p, bool emit);
+cudaError_t launch_colacc_add_sparse(cudaStream_t st, const ColSparseParams &p, bool add);
+
 void launch_stats_pass1(cudaStream_t st, const StatsParams &p);
 void launch_stats_pass2(cudaStream_t st, const StatsParams &p);
 void launch_stats_select(cudaStream_t st, const StatsParams &p);

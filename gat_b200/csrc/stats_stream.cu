@@ -428,4 +428,94 @@ cudaError_t launch_colacc_pick(cudaStream_t st, const ColHistParams &p)
     return cudaGetLastError();
 }
 
+// Sparse export of the windows (a shard's histograms, gatb_colacc_export): one CTA per column walks its window in
+// tiles of CH_THREADS bins, coalesced.  The count pass sums the column's non-zero bins; after the host's scan of the
+// column totals (col_ptr) the emit pass writes them in increasing value, each non-zero bin's slot from the ballot of
+// its warp and the totals of the warps before it, so the order is the bins' order whatever the grid.
+template <bool EMIT>
+__global__ void __launch_bounds__(CH_THREADS) colacc_export_kernel(ColSparseParams p)
+{
+    __shared__ uint32_t warp_nz[CH_THREADS / 32];
+    const uint32_t a = blockIdx.x, tid = threadIdx.x, lane = tid & 31u, wid = tid >> 5;
+    const uint64_t w = p.width[a];
+    const uint32_t *bins = p.bins + p.bin_off[a];
+    if (!EMIT) {
+        uint32_t n = 0;                             // (a column has fewer than 2^32 bins)
+        for (uint64_t b = tid; b < w; b += CH_THREADS) n += bins[b] != 0u ? 1u : 0u;
+        n = __reduce_add_sync(GATB_FULL, n);
+        if (lane == 0) warp_nz[wid] = n;
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long s = 0;
+            for (uint32_t i = 0; i < CH_THREADS / 32; i++) s += warp_nz[i];
+            p.nnz[a] = s;
+        }
+        return;
+    }
+    const uint32_t lo = p.lo[a];
+    unsigned long long out = (unsigned long long)p.col_ptr[a];
+    for (uint64_t t0 = 0; t0 < w; t0 += CH_THREADS) {
+        const uint64_t b = t0 + tid;
+        const uint32_t v = b < w ? bins[b] : 0u;
+        const unsigned m = __ballot_sync(GATB_FULL, v != 0u);
+        if (lane == 0) warp_nz[wid] = (uint32_t)__popc(m);
+        __syncthreads();
+        uint32_t before = 0, total = 0;
+        for (uint32_t i = 0; i < CH_THREADS / 32; i++) {
+            const uint32_t c = warp_nz[i];
+            before += i < wid ? c : 0u;
+            total += c;
+        }
+        if (v) {
+            const unsigned long long slot = out + before + (uint32_t)__popc(m & ((1u << lane) - 1u));
+            p.value[slot] = lo + (uint32_t)b;
+            p.count[slot] = v;
+        }
+        out += total;
+        __syncthreads();                            // (warp_nz of the next tile)
+    }
+}
+
+// A sparse histogram added into the windows (gatb_colacc_add_sparse): one thread per entry, its column by binary
+// search in col_ptr, its bin value - lo[column].  The check pass (ADD false) only flags an entry outside its window,
+// so that a refused histogram leaves the bins untouched; the add pass adds the counts.  The bins are uint32 (a
+// column holds fewer than 2^32 samples), and the entries of one call are distinct bins, so the atomics only meet
+// when a caller repeats a value.
+template <bool ADD>
+__global__ void __launch_bounds__(CH_THREADS) colacc_add_sparse_kernel(ColSparseParams p)
+{
+    const uint64_t i = (uint64_t)blockIdx.x * CH_THREADS + threadIdx.x;
+    if (i >= p.n_entries) return;
+    uint32_t a = 0, hi = p.n_cols;                  // col_ptr[a] <= i < col_ptr[hi]
+    while (hi - a > 1u) {
+        const uint32_t mid = (a + hi) >> 1;
+        if ((unsigned long long)p.col_ptr[mid] <= i) a = mid; else hi = mid;
+    }
+    const uint32_t d = p.value[i] - p.lo[a];        // (a value below the window wraps to >= width)
+    const unsigned long long c = p.count[i];
+    if (!ADD) {
+        if (d >= p.width[a] || c > 0xffffffffull) *p.error = 1u;
+        return;
+    }
+    if (c) atomicAdd(p.bins + p.bin_off[a] + d, (uint32_t)c);
+}
+
+cudaError_t launch_colacc_export(cudaStream_t st, const ColSparseParams &p, bool emit)
+{
+    if (p.n_cols == 0) return cudaSuccess;
+    if (emit) colacc_export_kernel<true><<<p.n_cols, CH_THREADS, 0, st>>>(p);
+    else colacc_export_kernel<false><<<p.n_cols, CH_THREADS, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_colacc_add_sparse(cudaStream_t st, const ColSparseParams &p, bool add)
+{
+    if (p.n_entries == 0) return cudaSuccess;
+    const uint64_t nb = (p.n_entries + CH_THREADS - 1u) / CH_THREADS;
+    if (nb > 0x7fffffffull) return cudaErrorInvalidValue;
+    if (add) colacc_add_sparse_kernel<true><<<(unsigned)nb, CH_THREADS, 0, st>>>(p);
+    else colacc_add_sparse_kernel<false><<<(unsigned)nb, CH_THREADS, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
 }  // namespace gatb

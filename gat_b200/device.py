@@ -296,22 +296,56 @@ class ColumnAccumulator(object):
         self.ctx.check(self.ctx.lib.gatb_colacc_add(self.handle, ctypes.c_void_p(device_ptr), int(n_rows),
                                                     int(row_stride or self.n_cols), what))
 
-    def state(self):
-        """-> dict of the integer state (rows, moments [5][A], minmax [2][A], outside [2][A], bins)"""
+    def state(self, bins=True):
+        """-> dict of the integer state (rows, moments [5][A], minmax [2][A], outside [2][A], bins; bins=False: without
+        the dense bins, which stay on the device)"""
         A = self.n_cols
         rows = np.zeros(1, dtype=np.uint64)
         st = dict(moments=np.zeros((5, A), dtype=np.uint64), minmax=np.zeros((2, A), dtype=np.uint32),
-                  outside=np.zeros((2, A), dtype=np.uint64), bins=np.zeros(max(self.n_bins, 1), dtype=np.uint32))
+                  outside=np.zeros((2, A), dtype=np.uint64))
+        if bins:
+            st["bins"] = np.zeros(max(self.n_bins, 1), dtype=np.uint32)
         self.ctx.check(self.ctx.lib.gatb_colacc_state(self.handle, _p(rows), _p(st["moments"]), _p(st["minmax"]),
-                                                      _p(st["outside"]), _p(st["bins"])))
+                                                      _p(st["outside"]), _p(st.get("bins"))))
         st["rows"] = int(rows[0])
         return st
 
     def merge(self, st, sums=True):
-        """add another accumulator's state (sums=False: only its histograms) into this one"""
+        """add another accumulator's state (sums=False: only its histograms) into this one; a part missing from st
+        (outside, bins) is not added"""
         self.ctx.check(self.ctx.lib.gatb_colacc_merge(
             self.handle, st["rows"] if sums else 0, _p(st["moments"]) if sums else None,
-            _p(st["minmax"]) if sums else None, _p(st["outside"]), _p(st["bins"])))
+            _p(st["minmax"]) if sums else None, _p(st.get("outside")), _p(st.get("bins"))))
+
+    def export(self):
+        """the windows' histograms as sparse CSR, compacted on the device -> (col_ptr int64 [A+1], value uint32,
+        count uint64): the non-zero bins of column a are entries col_ptr[a] .. col_ptr[a+1] - 1, in increasing value
+        (the layout of matrixfree.sparse_histogram)"""
+        col_ptr = np.zeros(self.n_cols + 1, dtype=np.int64)
+        self.ctx.check(self.ctx.lib.gatb_colacc_export(self.handle, _p(col_ptr), None, None, 0))
+        n = int(col_ptr[-1])
+        value = np.zeros(max(n, 1), dtype=np.uint32)
+        count = np.zeros(max(n, 1), dtype=np.uint64)
+        self.ctx.check(self.ctx.lib.gatb_colacc_export(self.handle, _p(col_ptr), _p(value), _p(count), n))
+        return col_ptr, value[:n], count[:n]
+
+    def add_sparse(self, col_ptr, value, count):
+        """add a sparse histogram (export's layout) into the windows' bins; ValueError, with the bins unchanged, when
+        a value lies outside the window of its column (as matrixfree.rebase_histogram)"""
+        col_ptr = np.ascontiguousarray(col_ptr, dtype=np.int64)
+        if col_ptr.shape != (self.n_cols + 1,):
+            raise ValueError("sparse histogram of %i columns added into an accumulator of %i"
+                             % (len(col_ptr) - 1, self.n_cols))
+        n = int(col_ptr[-1])
+        value = np.ascontiguousarray(value, dtype=np.uint32)
+        count = np.ascontiguousarray(count, dtype=np.uint64)
+        if len(value) != n or len(count) != n:
+            raise ValueError("sparse histogram: col_ptr ends at %i, with %i values and %i counts"
+                             % (n, len(value), len(count)))
+        rc = self.ctx.lib.gatb_colacc_add_sparse(self.handle, _p(col_ptr), _p(value), _p(count))
+        if rc == _lib.ERR_RANGE:
+            raise ValueError("histogram values outside the windows they are added into")
+        self.ctx.check(rc)
 
     def finish(self, pseudo_count=1.0):
         """-> (statistics dict as Context.column_stats returns it, missed bool [A])"""

@@ -177,7 +177,8 @@ def shard_states(ctx, produce, planes, n_samples, n_local, n_cols, chunk, budget
     produced in slabs (produce, planes, chunk as in stream_statistics).  Pass 1 counts the sums; pass 2 counts the
     histograms over the [min, max] of every column, from the slab still in the buffer when the rank's rows fit in
     one slab, else sampled again.  -> [dict(rows, moments [5][A], minmax [2][A], col_ptr int64 [A+1], value uint32,
-    count uint64) per plane]: the gatb_colacc_state layout, the histogram as sparse CSR per column (sparse_histogram)."""
+    count uint64) per plane]: the gatb_colacc_state layout, the histogram as sparse CSR per column, compacted on the
+    device (ColumnAccumulator.export; the layout of sparse_histogram)."""
     if budget_bytes is None:
         import torch
         budget_bytes = int(ARENA_FRACTION * torch.cuda.mem_get_info(ctx.device)[0])
@@ -202,11 +203,10 @@ def shard_states(ctx, produce, planes, n_samples, n_local, n_cols, chunk, budget
                 _count(accs, n, p, n_cols, False, True)
         _merge_ranks(accs, world, rank, sums=False)
         out = []
-        for a, st, l in zip(accs, states, lo):
-            bins = a.state()
-            if bins["outside"].any():
+        for a, st in zip(accs, states):
+            if a.state(bins=False)["outside"].any():
                 raise RuntimeError("shard: a value fell outside the [min, max] window of its column")
-            col_ptr, value, count = sparse_histogram(bins["bins"], l, st["minmax"][1].astype(np.int64) - l + 1)
+            col_ptr, value, count = a.export()
             out.append(dict(rows=st["rows"], moments=st["moments"], minmax=st["minmax"], col_ptr=col_ptr, value=value,
                             count=count))
         info["pass2_seconds"] += time.perf_counter() - t0
@@ -217,7 +217,7 @@ def shard_states(ctx, produce, planes, n_samples, n_local, n_cols, chunk, budget
 
 
 def sparse_histogram(bins, lo, width):
-    """dense unit-width bins of the windows [lo[a], lo[a] + width[a]) of every column, one after the other ->
+    """(the numpy statement of ColumnAccumulator.export) dense unit-width bins of the windows [lo[a], lo[a] + width[a]) of every column, one after the other ->
     (col_ptr int64 [A+1], value uint32, count uint64): the non-zero bins of column a are entries col_ptr[a] ..
     col_ptr[a+1] - 1, in increasing value"""
     width = np.asarray(width, dtype=np.int64)
@@ -231,8 +231,8 @@ def sparse_histogram(bins, lo, width):
 
 
 def rebase_histogram(col_ptr, value, count, lo, width):
-    """a sparse histogram (sparse_histogram) -> the dense uint32 bins of the windows [lo[a], lo[a] + width[a]), which
-    must hold its values"""
+    """(the numpy statement of ColumnAccumulator.add_sparse into cleared bins) a sparse histogram (sparse_histogram)
+    -> the dense uint32 bins of the windows [lo[a], lo[a] + width[a]), which must hold its values"""
     lo = np.asarray(lo, dtype=np.int64)
     width = np.asarray(width, dtype=np.int64)
     off = np.concatenate([[0], np.cumsum(width)])
@@ -245,11 +245,10 @@ def rebase_histogram(col_ptr, value, count, lo, width):
     return bins
 
 
-def merge_shard_states(ctx, n_samples, observed, ref_fold, states, pseudo_count=1.0, budget_bytes=None):
-    """the statistics of one counter plane from the shard_states of shards whose rows together are all n_samples
-    samples -> statistics dict as Context.column_stats returns it.  One accumulator with the windows [min, max] of
-    the union of the shards; every shard's histogram rebased into them and its integers added (gatb_colacc_merge:
-    the 128-bit sum of squares with its carry)."""
+def _union(ctx, n_samples, observed, ref_fold, states, budget_bytes):
+    """one accumulator holding the union of shard_states: the windows [min, max] of the union, every shard's
+    integers added (gatb_colacc_merge: the 128-bit sum of squares with its carry) and its sparse histogram added on
+    the device (ColumnAccumulator.add_sparse).  The caller closes it."""
     A = len(observed)
     if budget_bytes is None:
         import torch
@@ -259,14 +258,38 @@ def merge_shard_states(ctx, n_samples, observed, ref_fold, states, pseudo_count=
         lo = np.min([st["minmax"][0] for st in states], axis=0).astype(np.int64)
         hi = np.max([st["minmax"][1] for st in states], axis=0).astype(np.int64)
         _set_windows([acc], [lo], [hi], budget_bytes, "merge")
-        outside = np.zeros((2, A), dtype=np.uint64)
         for st in states:
             acc.merge(dict(rows=int(st["rows"]), moments=np.ascontiguousarray(st["moments"], dtype=np.uint64),
-                           minmax=np.ascontiguousarray(st["minmax"], dtype=np.uint32), outside=outside,
-                           bins=rebase_histogram(st["col_ptr"], st["value"], st["count"], lo, hi - lo + 1)))
+                           minmax=np.ascontiguousarray(st["minmax"], dtype=np.uint32)))
+            acc.add_sparse(st["col_ptr"], st["value"], st["count"])
+        return acc
+    except BaseException:
+        acc.close()
+        raise
+
+
+def merge_shard_states(ctx, n_samples, observed, ref_fold, states, pseudo_count=1.0, budget_bytes=None):
+    """the statistics of one counter plane from the shard_states of shards whose rows together are all n_samples
+    samples -> statistics dict as Context.column_stats returns it"""
+    acc = _union(ctx, n_samples, observed, ref_fold, states, budget_bytes)
+    try:
         stats, missed = acc.finish(pseudo_count)
         if missed.any():
             raise RuntimeError("shard merge: a CI rank missed the [min, max] window of its column")
         return stats
+    finally:
+        acc.close()
+
+
+def combine_shard_states(ctx, n_samples, observed, ref_fold, states, budget_bytes=None):
+    """the shard_states of shards whose rows are consecutive ranges of one run -> the shard_states of their union
+    range: summed integers, union [min, max], and the histogram over the union's [min, max] exported from the device
+    (the state a shard job over the union range would have counted)"""
+    acc = _union(ctx, n_samples, observed, ref_fold, states, budget_bytes)
+    try:
+        st = acc.state(bins=False)
+        col_ptr, value, count = acc.export()
+        return dict(rows=st["rows"], moments=st["moments"], minmax=st["minmax"], col_ptr=col_ptr, value=value,
+                    count=count)
     finally:
         acc.close()

@@ -10,6 +10,14 @@ with the exact integer state of every (segment track, counter): the sums of matr
 histogram of every column over its [min, max] in the shard, as sparse CSR.  Every sample is a function of (seed,
 track, unit, global sample index), so shards of the same inputs and seed whose ranges tile [0, num_samples), in any
 order, merge (mergeShards) into the statistics of run() over all samples, bit for bit; the merge samples nothing.
+
+    python -m gat_b200.shards --combine=OUT part*.npz       # one shard file for the shards' contiguous range
+    python -m gat_b200.shards [output flags] --prefix part*.npz
+
+Shards whose ranges form one contiguous [b, e) combine (combineShards) into the shard file a job over [b, e) would
+write, so finished shards can be folded together as they arrive.  Shards that tile [0, k) hold exactly the samples of
+run(..., num_samples=k): mergeShardPrefix reads the results of the first k samples from the shards that have
+finished, up to the first missing range.
 """
 import hashlib
 import sys
@@ -128,9 +136,9 @@ def _same(x, y):
         bool(np.all((x == y) | ((x != x) & (y != y)) if x.dtype.kind == "f" else x == y))
 
 
-def readShards(filenames):
-    """-> [Shard], checked to be shards of one run whose ranges tile [0, num_samples) (in any order); ValueError
-    naming the files otherwise"""
+def _readRun(filenames):
+    """-> [Shard], checked to be shards of one run (their ranges are not looked at); ValueError naming the files
+    otherwise"""
     if not filenames:
         raise ValueError("no shard files given")
     shards = [Shard(f) for f in filenames]
@@ -145,7 +153,31 @@ def readShards(filenames):
                 not all(_same(first.arrays[k], s.arrays[k]) for k in row_fields):
             raise ValueError("%s and %s are not shards of the same run: their observed counts, reference folds or "
                              "size columns differ" % (first.filename, s.filename))
-    order = sorted(shards, key=lambda s: (s.begin, s.end))
+    return shards
+
+
+def _inRange(order):
+    """order: shards sorted by range; ValueError for a range that is empty or reaches outside [0, num_samples)"""
+    if not 0 <= order[0].begin:
+        raise ValueError("%s: sample range starts below 0" % order[0].filename)
+    for s in order:
+        if s.end <= s.begin:
+            raise ValueError("%s: empty sample range [%i, %i)" % (s.filename, s.begin, s.end))
+        if s.end > s.num_samples:
+            raise ValueError("%s: sample range [%i, %i) ends past num_samples = %i" % (s.filename, s.begin, s.end,
+                                                                                       s.num_samples))
+
+
+def _byRange(shards):
+    return sorted(shards, key=lambda s: (s.begin, s.end))
+
+
+def readShards(filenames):
+    """-> [Shard], checked to be shards of one run whose ranges tile [0, num_samples) (in any order); ValueError
+    naming the files otherwise"""
+    shards = _readRun(filenames)
+    first = shards[0]
+    order = _byRange(shards)
     if not 0 <= order[0].begin:
         raise ValueError("%s: sample range starts below 0" % order[0].filename)
     at, prev = 0, None
@@ -171,9 +203,80 @@ def mergeShards(filenames):
     return _merge(readShards(filenames), Engine.getContext())
 
 
-def _merge(shards, ctx, budget_bytes=None):
+def _contiguous(order):
+    """order: shards sorted by range, each range inside [0, num_samples); ValueError naming the files when two
+    overlap or when samples between two are in none"""
+    at, prev = order[0].begin, None
+    for s in order:
+        if prev is not None and s.begin < at:
+            raise ValueError("%s and %s overlap: samples [%i, %i)" % (prev.filename, s.filename, s.begin,
+                                                                      min(at, s.end)))
+        if prev is not None and s.begin > at:
+            raise ValueError("samples [%i, %i) are in no shard (a gap between %s and %s)"
+                             % (at, s.begin, prev.filename, s.filename))
+        at, prev = s.end, s
+    return order[0].begin, at
+
+
+def combineShards(filenames, output):
+    """the shard files of one run whose ranges are disjoint and together one contiguous range [b, e), in any order ->
+    one shard file `output` for [b, e): the state a shard job over [b, e) writes (summed integers, union [min, max],
+    the union histogram, exported from the device).  It is an ordinary shard: mergeShards, combineShards and
+    mergeShardPrefix take it, so that shards can be merged as they arrive, or as a tree."""
+    shards = _readRun(filenames)
+    order = _byRange(shards)
+    _inRange(order)
+    b, e = _contiguous(order)
+    first = shards[0]
+    a = first.arrays
+    out = dict((k, v) for k, v in a.items() if not k.startswith("state_"))
+    out["sample_range"] = np.array([b, e], dtype=np.int64)
+    ctx = Engine.getContext()
+    row_c, row_t = a["row_counter"], a["row_track"]
+    for r0, r1 in _blocks(row_c, row_t):
+        ci, ti = int(row_c[r0]), int(row_t[r0])
+        ref = a["row_ref_fold"][r0:r1] if bool(a["has_reference"]) else None
+        st = matrixfree.combine_shard_states(ctx, first.num_samples, a["row_observed"][r0:r1], ref,
+                                             [s.state(ti, ci) for s in shards])
+        for k in STATE:
+            out["state_%i_%i_%s" % (ti, ci, k)] = np.asarray(st[k])
+    _save(output, out)
+
+
+def mergeShardPrefix(filenames):
+    """the results of run(..., num_samples=k) from shard files of a run of num_samples >= k samples -> (k,
+    [AnnotatorResultExtended] in run()'s order).  k is the end of the longest run of the shards that tiles [0, k)
+    from 0: a campaign whose shard jobs have not all finished can be read up to its first missing range.  Shards
+    past that gap are not used; their names are written to stderr.  ValueError naming the files when two ranges
+    overlap or no shard starts at 0."""
+    shards = _readRun(filenames)
+    order = _byRange(shards)
+    _inRange(order)
+    at, prev = 0, None
+    for s in order:
+        if prev is not None and s.begin < at:
+            raise ValueError("%s and %s overlap: samples [%i, %i)" % (prev.filename, s.filename, s.begin,
+                                                                      min(at, s.end)))
+        at, prev = max(at, s.end), s
+    if order[0].begin != 0:
+        raise ValueError("samples [0, %i) are in no shard (a gap before %s)" % (order[0].begin, order[0].filename))
+    k, used = 0, []
+    for s in order:
+        if s.begin != k:
+            break
+        used.append(s)
+        k = s.end
+    unused = order[len(used):]
+    if unused:
+        sys.stderr.write("# gat_b200.shards: samples [%i, %i) are in no shard; not used: %s\n"
+                         % (k, unused[0].begin, " ".join(s.filename for s in unused)))
+    return k, _merge(used, Engine.getContext(), num_samples=k)
+
+
+def _merge(shards, ctx, budget_bytes=None, num_samples=None):
+    """the results of the shards, whose rows together are the run's first num_samples (default: all) samples"""
     first = shards[0].arrays
-    S = int(first["num_samples"])
+    S = int(first["num_samples"]) if num_samples is None else int(num_samples)
     pseudo_count = float(first["pseudo_count"])
     counters, tracks, atracks = shards[0].counters, shards[0].tracks, shards[0].annotations
     row_c, row_t, row_a = first["row_counter"], first["row_track"], first["row_annotation"]
@@ -218,14 +321,31 @@ def main(argv=None):
     parser.set_defaults(**dict((k, cli._DEFAULTS[k]) for k in wanted))
     parser.add_option("-v", "--verbose", dest="loglevel", type="int", default=1, help="log level")
     parser.add_option("-S", "--stdout", dest="stdout_file", type="string", default=None, help="output file")
+    parser.add_option("--combine", dest="combine", type="string", default=None,
+                      help="write the shards, whose ranges must form one contiguous range, as one shard file COMBINE "
+                      "instead of printing a table")
+    parser.add_option("--prefix", dest="prefix", action="store_true", default=False,
+                      help="print the table of the run of the first k samples, k the end of the shards' ranges that "
+                      "tile [0, k) from 0, instead of requiring them to tile all samples")
     options, filenames = parser.parse_args(argv[1:])
     if not filenames:
         parser.error("no shard files given")
+    if options.combine and options.prefix:
+        parser.error("--combine and --prefix exclude each other")
+    if options.combine:
+        combineShards(filenames, options.combine)
+        return 0
     if "%s" not in options.output_tables_pattern:
         raise ValueError("output_tables_pattern should contain at least one '%s'")
     options.stdout = open(options.stdout_file, "w") if options.stdout_file else sys.stdout
     description_header, descriptions, description_width = IO.readDescriptions(options)
-    results = mergeShards(filenames)
+    if options.prefix:
+        k, results = mergeShardPrefix(filenames)
+        with np.load(filenames[0], allow_pickle=False) as z:
+            n = int(z["num_samples"])
+        sys.stderr.write("# gat_b200.shards: samples [0, %i) of %i\n" % (k, n))
+    else:
+        results = mergeShards(filenames)
     if options.pvalue_method != "empirical":
         Engine.updatePValues(results, options.pvalue_method)
     IO.outputResults(results, options, Engine.AnnotatorResultExtended.headers, description_header, description_width,

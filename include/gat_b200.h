@@ -42,7 +42,7 @@ extern "C" {
 #define GATB_ERR_CAPACITY   -3   /* a placement unit overflowed its segment buffer                    */
 #define GATB_ERR_TOO_LARGE  -4   /* segment too large for nbuckets*bucket_size (ValueError in         */
                                  /* SegmentList.getLengthDistribution, gat/SegmentList.pyx:1170-1182) */
-#define GATB_ERR_RANGE      -5   /* coordinate >= 2^31 or total overlap >= 2^32                       */
+#define GATB_ERR_RANGE      -5   /* coordinate >= 2^31 or total overlap >= 2^32; a histogram value outside its window */
 
 /* counters (gat/Engine.pyx:1412-1472; names are the --counter choices, gat/__init__.py:214-223) */
 #define GATB_NUCLEOTIDE_OVERLAP    0   /* CounterNucleotideOverlap       :1417-1425 */
@@ -348,6 +348,16 @@ int  gatb_colacc_state(gatb_colacc *acc, uint64_t *rows, uint64_t *moments, uint
  * this one: the sum of squares with its carry, min / max, counts. */
 int  gatb_colacc_merge(gatb_colacc *acc, uint64_t rows, const uint64_t *moments, const uint32_t *minmax,
                        const uint64_t *outside, const uint32_t *bins);
+/* the windows' histograms as sparse CSR, compacted on the device (a per-column count of the non-zero bins, a scan, an
+ * emit pass): col_ptr[n_cols + 1] (host) receives the offsets, and entries col_ptr[a] .. col_ptr[a + 1] - 1 of value /
+ * count (host, `capacity` entries) the non-zero bins of column a in increasing value.  Two calls, as
+ * gatb_format_counts: value == count == NULL asks for col_ptr only (col_ptr[n_cols] = entries needed);
+ * GATB_ERR_CAPACITY when capacity is too small (col_ptr is still filled). */
+int  gatb_colacc_export(gatb_colacc *acc, int64_t *col_ptr, uint32_t *value, uint64_t *count, uint64_t capacity);
+/* adds a sparse histogram (gatb_colacc_export layout, host arrays, col_ptr[n_cols] entries) into the windows' bins:
+ * count[i] at value[i] of its column.  GATB_ERR_RANGE, with the bins untouched, when a value lies outside its
+ * column's window or a count is 2^32 or more.  Enqueued on the context's stream after the check. */
+int  gatb_colacc_add_sparse(gatb_colacc *acc, const int64_t *col_ptr, const uint32_t *value, const uint64_t *count);
 /* the statistics of gatb_column_stats (host outputs of n_cols doubles, any may be NULL) once the sums hold
  * n_samples_total rows and every histogram n_samples_total values (GATB_ERR_INVALID otherwise).  missed[n_cols]
  * (host, may be NULL): 1 where a CI rank fell outside the column's window -- lower95 / upper95 are NaN there,
