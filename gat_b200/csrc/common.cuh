@@ -358,8 +358,9 @@ __device__ __forceinline__ bool warp_bucket_sort(uint64_t *buf, uint32_t n, uint
         tmp[atomicAdd(&cnt[sort_bucket(pl, seg_start(key))], 1u)] = key;
     }
     __syncwarp();                                   // now cnt[b] = end of bucket b = start of bucket b + 1
-    // rank inside the bucket; two keys per lane and pass, so that their dependent loads (key -> bucket bounds
-    // -> bucket mates) overlap
+    // rank inside the bucket; two keys per lane and pass, and four bucket mates of each per turn of the inner loop,
+    // so that eight independent loads are in flight at once instead of two (a bucket holds a few keys, and each
+    // turn waits for its loads)
     for (uint32_t j0 = lane; j0 < n; j0 += 64) {
         const uint32_t j1 = j0 + 32u;
         const bool has1 = j1 < n;
@@ -369,14 +370,18 @@ __device__ __forceinline__ bool warp_bucket_sort(uint64_t *buf, uint32_t n, uint
         const uint32_t first1 = has1 ? (b1 ? cnt[b1 - 1u] : 0u) : 0u, last1 = has1 ? cnt[b1] : 0u;
         const uint32_t m0 = last0 - first0, m1 = last1 - first1;
         uint32_t r0 = 0, r1 = 0;
-        for (uint32_t t = 0; t < max(m0, m1); t++) {
-            if (t < m0) {
-                const uint64_t other = tmp[first0 + t];
-                r0 += (other < key0 || (other == key0 && first0 + t < j0)) ? 1u : 0u;
+        for (uint32_t t = 0; t < max(m0, m1); t += 4) {
+            const uint32_t p0 = first0 + t, p1 = first1 + t;
+            uint64_t x0[4], x1[4];      // (a slot past the bucket reads as +inf: never below a key, and past its own slot)
+#pragma unroll
+            for (uint32_t u = 0; u < 4; u++) {
+                x0[u] = t + u < m0 ? tmp[p0 + u] : GATB_KEY_INF;
+                x1[u] = t + u < m1 ? tmp[p1 + u] : GATB_KEY_INF;
             }
-            if (t < m1) {
-                const uint64_t other = tmp[first1 + t];
-                r1 += (other < key1 || (other == key1 && first1 + t < j1)) ? 1u : 0u;
+#pragma unroll
+            for (uint32_t u = 0; u < 4; u++) {
+                r0 += (x0[u] < key0 || (x0[u] == key0 && p0 + u < j0)) ? 1u : 0u;
+                r1 += (x1[u] < key1 || (x1[u] == key1 && p1 + u < j1)) ? 1u : 0u;
             }
         }
         buf[first0 + r0] = key0;
