@@ -818,6 +818,7 @@ struct gatb_sampler {
     gatb_ctx *ctx = nullptr;
     uint32_t n_units = 0, n_contigs = 0;
     bool has_iso = false;
+    bool one_piece = false;             // every unit's workspace is one piece (place_kernel<true>)
     int kind = 0;                       // 0 SamplerAnnotator, 1 SamplerSegments, 2 SamplerShift
     double shift_radius = 2.0;          // SamplerShift(radius, extension), gat/Engine.pyx:1021-1026
     int32_t shift_extension = 0;
@@ -956,6 +957,7 @@ extern "C" int gatb_sampler_create(gatb_ctx *ctx, int n_units, const int32_t *un
             ws_tab_total += 2 + (WS_NB + 1);        // words: two multipliers + 2 * (WS_NB + 1) 16-bit entries
         }
     }
+    s->one_piece = std::all_of(s->h_units.begin(), s->h_units.end(), [](const UnitDesc &d) { return d.ws_n == 1; });
     const double t_host = since();
     DevBuf<uint32_t> &d_seg_start = s->seg_start, &d_seg_end = s->seg_end;
     DevBuf<uint64_t> d_scratch, d_scratch_off;
@@ -1124,8 +1126,8 @@ static int place_batch(gatb_sampler *s, uint64_t seed, uint32_t track, uint64_t 
         p.buf = pb.placed.p; p.sample_stride = s->placed_stride;
         p.out_n = pb.placed_n.p; p.out_n_stride = s->n_contigs; p.out_by_contig = 1;
     }
-    p.status = pb.status.p; p.unit_over = s->unit_over.p; p.n_units = s->n_units; p.n_samples = B; p.sample_begin = sample_begin;
-    p.seed = seed; p.track = track; p.sampler_kind = s->kind;
+    p.status = pb.status.p; p.unit_over = s->unit_over.p; p.n_units = s->n_units; p.one_piece = s->one_piece ? 1 : 0; p.n_samples = B; p.sample_begin = sample_begin;
+    p.keys = philox_keys(seed); p.track = track; p.sampler_kind = s->kind;
     p.seg_start = s->seg_start.p; p.seg_end = s->seg_end.p;
     p.shift_half_radius = s->shift_radius / 2; p.shift_extension = s->shift_extension;
     { ProfScope ps(ctx, PROF_PLACE, st); launch_place(st, p); }

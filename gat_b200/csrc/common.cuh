@@ -29,8 +29,24 @@ __host__ __device__ __forceinline__ uint32_t next_pow2(uint32_t x)
 // unit, sample), key = 64-bit seed.  Must stay bit-identical to oracle/gat_oracle.c:go_philox4x32_10.
 struct Philox4 { uint32_t x, y, z, w; };
 
+// The ten round keys of a seed, k[0][r] = k0 + r * 0x9E3779B9 and k[1][r] = k1 + r * 0xBB67AE85.  A kernel that takes
+// them as a launch parameter reads them from the constant bank (into uniform registers, operands of the rounds' XORs)
+// instead of rebuilding them at every inlined call.
+struct PhiloxKeys { uint32_t k[2][10]; };
+
+__host__ __device__ inline PhiloxKeys philox_keys(uint64_t seed)
+{
+    PhiloxKeys rk;
+    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+    for (int r = 0; r < 10; r++) {
+        rk.k[0][r] = k0; rk.k[1][r] = k1;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    return rk;
+}
+
 __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
-                                                          uint32_t k0, uint32_t k1)
+                                                          const PhiloxKeys &rk)
 {
 #pragma unroll
     for (int r = 0; r < 10; r++) {
@@ -41,9 +57,8 @@ __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t 
         uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
         uint32_t hi0 = (uint32_t)(p0 >> 32), lo0 = (uint32_t)p0, hi1 = (uint32_t)(p1 >> 32), lo1 = (uint32_t)p1;
 #endif
-        uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
+        uint32_t n0 = hi1 ^ c1 ^ rk.k[0][r], n2 = hi0 ^ c3 ^ rk.k[1][r];
         c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
     }
     Philox4 o; o.x = c0; o.y = c1; o.z = c2; o.w = c3;
     return o;

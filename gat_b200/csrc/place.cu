@@ -35,10 +35,10 @@ __device__ __forceinline__ uint32_t ws_pick(const WsView &w, uint32_t r)
 
 __device__ __forceinline__ TurnDraw draw_turn(const UnitDesc &d, const WsView &ws, const uint32_t *tab,
                                               uint32_t turn, uint32_t c1base, uint32_t unit, uint32_t sample,
-                                              uint32_t k0, uint32_t k1)
+                                              const PhiloxKeys &rk)
 {
-    Philox4 b0 = philox4x32_10(turn, 0u | c1base, unit, sample, k0, k1);
-    Philox4 b1 = philox4x32_10(turn, 1u | c1base, unit, sample, k0, k1);
+    Philox4 b0 = philox4x32_10(turn, 0u | c1base, unit, sample, rk);
+    Philox4 b1 = philox4x32_10(turn, 1u | c1base, unit, sample, rk);
     TurnDraw t;
     // HistogramSampler.sample (gat/Engine.pyx:413-435): r = randint(1,total) ranks the sorted lengths
     uint32_t r = 1;
@@ -219,6 +219,10 @@ __device__ __forceinline__ uint32_t warp_drop_empty(uint64_t *buf, uint32_t n, c
 #ifndef GATB_PLACE_MINBLOCKS
 #define GATB_PLACE_MINBLOCKS 8      // 64 registers: occupancy beats the few spilled values (measured)
 #endif
+// ONE_PIECE: every unit's workspace is one piece (contig workspaces, PlaceParams.one_piece).  With the piece count a
+// constant the compiler drops the piece draw, its search, the predecessor clamp and the multi-piece branches of the
+// coverage helpers from every turn.
+template <bool ONE_PIECE>
 __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceParams p)
 {
     __shared__ uint32_t sort_cnt[4][GATB_SORT_NB];         // counting-sort buckets, one set per warp
@@ -232,11 +236,10 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
     uint64_t *buf = p.buf + (uint64_t)sl * p.sample_stride + d.buf_off;
     WsView ws;
     ws.start = p.ws_start + d.ws_off; ws.end = p.ws_end + d.ws_off; ws.cuminc = p.ws_cuminc + d.ws_off;
-    ws.n = d.ws_n;
-    ws.tabw = d.ws_tab_off != 0xffffffffu ? p.ws_tab + d.ws_tab_off : nullptr;
+    ws.n = ONE_PIECE ? 1u : d.ws_n;
+    ws.tabw = !ONE_PIECE && d.ws_tab_off != 0xffffffffu ? p.ws_tab + d.ws_tab_off : nullptr;
     const uint32_t *tab = p.len_tab + d.tab_off;
     const uint32_t sample = (uint32_t)(p.sample_begin + sl);
-    const uint32_t k0 = (uint32_t)p.seed, k1 = (uint32_t)(p.seed >> 32);
     const uint32_t c1base = p.track << 8;
 
     // every placement starts in [first workspace start - longest length, last workspace end): the range of
@@ -267,7 +270,7 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
         // SamplerSegments.sample (gat/Engine.pyx:719-735): exactly len(segments) placements, every one
         // kept, returned in draw order (unsorted, unmerged); fromIsochores' merge(0) normalizes them later
         for (uint32_t t = lane; t < d.seg_n; t += 32) {
-            const TurnDraw td = draw_turn(d, ws, tab, t, c1base, unit, sample, k0, k1);
+            const TurnDraw td = draw_turn(d, ws, tab, t, c1base, unit, sample, p.keys);
             buf[t] = pack_seg(td.start, td.end);
         }
         nu = d.seg_n;
@@ -283,7 +286,7 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
             uint32_t f = 0;
             int32_t incl = 0;
             if (!certain) {
-                t = draw_turn(d, ws, tab, t0 + lane, c1base, unit, sample, k0, k1);
+                t = draw_turn(d, ws, tab, t0 + lane, c1base, unit, sample, p.keys);
                 // no turn can trigger while what is left after ALL 32 still exceeds the longest of their lengths
                 // (two warp reductions instead of the prefix scan: the usual case until the unit is nearly full)
                 const int32_t all = __reduce_add_sync(GATB_FULL, t.ov);
@@ -336,8 +339,8 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
             if (true_remaining == remaining) fails++; else true_remaining = remaining;
 
             if (true_remaining < 0) {           // overshoot (gat/Engine.pyx:608-625)
-                Philox4 b2 = philox4x32_10(t0, 2u | c1base, unit, sample, k0, k1);
-                Philox4 b3 = philox4x32_10(t0, 3u | c1base, unit, sample, k0, k1);
+                Philox4 b2 = philox4x32_10(t0, 2u | c1base, unit, sample, p.keys);
+                Philox4 b3 = philox4x32_10(t0, 3u | c1base, unit, sample, p.keys);
                 uint32_t removed, orphaned;
                 warp_trim(buf, nu, (uint32_t)(-true_remaining), ulen, b2, b3, ws, &removed, &trim_emptied, &orphaned);
                 cov -= removed; orphans += orphaned;
@@ -349,7 +352,7 @@ __global__ void __launch_bounds__(128, GATB_PLACE_MINBLOCKS) place_kernel(PlaceP
             }
             if (true_remaining > 0) {           // gat/Engine.pyx:632-634
                 if (certain) {                  // the draw that was put off (every lane computes turn t0)
-                    const TurnDraw t1 = draw_turn(d, ws, tab, t0, c1base, unit, sample, k0, k1);
+                    const TurnDraw t1 = draw_turn(d, ws, tab, t0, c1base, unit, sample, p.keys);
                     sf = t1.start; ef = t1.end; ovf = t1.ov;
                 }
                 if (lane == 0) buf[nu + np] = pack_seg(sf, ef);
@@ -478,7 +481,6 @@ __global__ void __launch_bounds__(128) shift_kernel(PlaceParams p)
     ws.n = d.ws_n;
     ws.tabw = d.ws_tab_off != 0xffffffffu ? p.ws_tab + d.ws_tab_off : nullptr;
     const uint32_t sample = (uint32_t)(p.sample_begin + sl);
-    const uint32_t k0 = (uint32_t)p.seed, k1 = (uint32_t)(p.seed >> 32);
     const uint32_t c1 = p.track << 8;       // Philox block 0 of turn x: words 0,1 = position, words 2,3 = direction
     uint32_t *counter = &emitted[threadIdx.x >> 5];
     if (lane == 0) *counter = 0u;
@@ -518,7 +520,7 @@ __global__ void __launch_bounds__(128) shift_kernel(PlaceParams p)
         if (L.k == 0) continue;
         uint32_t total = 0;
         for (uint32_t j = 0; j < L.k; j++) total += L.e(j) - L.s(j);
-        const Philox4 r = philox4x32_10(x, c1, unit, sample, k0, k1);
+        const Philox4 r = philox4x32_10(x, c1, unit, sample, p.keys);
         uint32_t pos = bounded_u32(r.x, r.y, total);                  // getRandomPosition (gat/SegmentList.pyx:902-915)
         int32_t start = 0, end;
         for (uint32_t j = 0; j < L.k; j++) {
@@ -566,7 +568,8 @@ void launch_place(cudaStream_t st, const PlaceParams &p)
     const int warps_per_block = 4;
     uint64_t blocks = (items + warps_per_block - 1) / warps_per_block;
     if (p.sampler_kind == 2) shift_kernel<<<(unsigned)blocks, warps_per_block * 32, 0, st>>>(p);
-    else place_kernel<<<(unsigned)blocks, warps_per_block * 32, 0, st>>>(p);
+    else if (p.one_piece) place_kernel<true><<<(unsigned)blocks, warps_per_block * 32, 0, st>>>(p);
+    else place_kernel<false><<<(unsigned)blocks, warps_per_block * 32, 0, st>>>(p);
 }
 
 // ---------------------------------------------------------------------------------------------------

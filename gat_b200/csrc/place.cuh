@@ -46,9 +46,10 @@ struct PlaceParams {
     uint32_t *unit_over;         // [n_units]: set when any sample of the unit overflowed its buffer (the caller
                                  // grows those units and runs the call again)
     uint32_t n_units;
+    int one_piece;               // 1: every unit's workspace is one piece (place_kernel<true>)
     uint32_t n_samples;          // samples in this launch
     uint64_t sample_begin;       // global index of the first sample
-    uint64_t seed;
+    PhiloxKeys keys;             // round keys of the 64-bit seed (philox_keys)
     uint32_t track;
     int sampler_kind;            // 0: SamplerAnnotator (gat/Engine.pyx:445-646), 1: SamplerSegments (:653-737),
                                  // 2: SamplerShift (:998-1111, shift_kernel)
